@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
                     [--workload wide|mnist] [--batch-per-gpu B] [--global-batch G]
+                    [--dump-outputs DIR]
 
 Workload at N=1 (default): BASELINE.json configs[3] -- 4 x Dense(4096) with 3 ReLU, D_in = C =
 4096, batch 8192, fp32 storage, fp32-accurate split tensor-core GEMMs, fused global-softmax CE,
@@ -28,6 +29,14 @@ Extra objects in the same JSON line (every one measured in this run):
                    loss equals ln(B_global * C) to the tolerance random init allows
   mnist          : (N=1) BASELINE.json configs[0], the examples/mnist MLP at batch 128: the
                    unmodified five-line loop (eager) and Model.train_step (recorded step)
+
+--dump-outputs DIR (B200 arm, rank 0) writes what the last timed step handed its caller as
+DIR/<name>.npy (float32, or float64 where the output is float64): `loss`, `prediction` (eager steps
+only; a recorded step returns the loss alone) and every parameter after the update as
+`layer<i>_<key>`.  An output of more than DUMP_SAMPLE elements is stored as its values at a fixed
+seeded sample of DUMP_SAMPLE flat indices (sorted), the same sample on every run; the wide MLP's
+dump is about 20 MB.  The inputs and the initial weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 
 --impl reference times the CPU implementation alone (all host threads, also under torchrun), on
 the same config/metric/unit; each of its steps is a bounded sample of the workload: a train step
@@ -60,6 +69,7 @@ WIDE = dict(name="wide_mlp_4x4096", widths=[4096, 4096, 4096, 4096], d_in=4096, 
 MNIST = dict(name="mnist_mlp_784-200-100-70-30-10", widths=[200, 100, 70, 30, 10], d_in=784, batch=128)
 REF_SAMPLE_BATCH = 1024     # rows per CPU-reference step on the wide MLP (fixed; see module docstring)
 STRONG_GLOBAL_BATCH = 65536  # BASELINE.json configs[4]
+DUMP_SAMPLE = 1 << 20        # --dump-outputs: elements kept of a larger output (4 MB in float32)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -305,16 +315,21 @@ class Stepper(object):
         self.model.defer_loop = bool(defer_loop)
         self.loss_layer = SoftmaxCrossEntropyLoss()
         self.use_graph = use_graph
+        self.keep_outputs = False    # keep the last step's (loss, prediction) for --dump-outputs
+        self.outputs = None
 
     def __call__(self, x_t, y_t):
         if self.use_graph:   # the same five calls, recorded once per batch shape and replayed
-            return self.model.train_step(x_t, y_t)
-        m = self.model
-        m.zero_grad()
-        pred = m.forward(x_t)
-        loss = self.loss_layer.loss(pred, y_t)
-        loss.backward()
-        m.step()
+            loss, pred = self.model.train_step(x_t, y_t), None
+        else:
+            m = self.model
+            m.zero_grad()
+            pred = m.forward(x_t)
+            loss = self.loss_layer.loss(pred, y_t)
+            loss.backward()
+            m.step()
+        if self.keep_outputs:
+            self.outputs = (loss, pred)
         return loss
 
     def param_checksum(self):
@@ -324,6 +339,27 @@ class Stepper(object):
             return None
         host = be.to_numpy(a["p"])
         return float(np.sum(host.astype(np.float64))), float(np.sum(np.abs(host).astype(np.float64)))
+
+
+def dump_outputs(stepper, out_dir):
+    """--dump-outputs: the last step's loss, prediction and updated parameters as out_dir/<name>.npy
+    (see the module docstring); returns the names written"""
+    loss, pred = stepper.outputs
+    arrays = {"loss": loss.values}
+    if pred is not None:
+        arrays["prediction"] = pred.values
+    for i, layer in enumerate(stepper.net.get_parameters()):
+        for key, p in layer.items():
+            if p is not None:
+                arrays["layer%d_%s" % (i, key)] = p.values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float64 if np.asarray(a).dtype == np.float64 else np.float32)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(arrays)
 
 
 LAST_TIMED_REGION = {}   # host-side facts about the most recent timed loop (diagnostics)
@@ -481,6 +517,7 @@ def run_b200_arm(args, cfg):
     y_dev = [be.from_numpy(one_hot_host(y, C)) for y in ys]
     use_graph = args.graph == "on" or (args.graph == "auto" and args.workload == "mnist")
     stepper = Stepper(cfg, use_graph)
+    stepper.keep_outputs = bool(args.dump_outputs) and rank == 0
 
     # ---- step-0 loss: with zero biases and Xavier weights the logits are O(1) and the global
     # softmax is near uniform over B_global*C entries, so loss_0 = ln(B_global*C) up to the logit spread
@@ -507,6 +544,9 @@ def run_b200_arm(args, cfg):
     s_last = sampler.mark() + 1
     clocks = sampler.stop(s_first, s_last)
     timed_region = dict(LAST_TIMED_REGION)
+    if stepper.keep_outputs:              # before the e2e steps below move the parameters on
+        dump_outputs(stepper, args.dump_outputs)
+        stepper.keep_outputs, stepper.outputs = False, None
 
     # ---- replicas agree (driver-visible correctness at N>1) ------------------------------------
     if world > 1:
@@ -666,10 +706,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the strong-scaling / all-reduce / mnist side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's loss, prediction and updated parameters to "
+                         "DIR/<name>.npy (large outputs as a fixed seeded sample)")
     args = ap.parse_args()
     args.steps_given = args.steps is not None
     if args.steps is None:
         args.steps = 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     cfg = dict(WIDE if args.workload == "wide" else MNIST)
     if args.impl == "reference":

@@ -312,6 +312,48 @@ def test_save_load_roundtrip(tmp_path):
     assert np.array_equal(model2.forward(x).values, y0)
 
 
+def test_bench_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs on the MNIST workload, eager steps: the loss is the JSON line's
+    final_loss, and loss, prediction and every parameter equal those of the same seeded steps run
+    here (step 0 and warm-up, then exactly --steps timed steps: one step more or less moves every
+    parameter by about Adam's lr)"""
+    import json
+    import subprocess
+    import sys
+    import bench
+    import core._backend as be
+    from core.tensor import Tensor
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    steps, warmup = 3, 4
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "mnist", "--graph", "off",
+                          "--steps", str(steps), "--warmup", str(warmup), "--no-extras", "--no-cpu-baseline",
+                          "--dump-outputs", str(tmp_path / "bench")],
+                         capture_output=True, text=True, timeout=600, cwd=root)
+    assert out.returncode == 0, out.stderr[-3000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps and line["warmup"] == warmup
+
+    cfg = dict(bench.MNIST)
+    B, C = cfg["batch"], cfg["widths"][-1]
+    xs, ys = bench.synthetic_shard(cfg, B, 0)
+    x_dev = [be.from_numpy(x) for x in xs]
+    y_dev = [be.from_numpy(bench.one_hot_host(y, C)) for y in ys]
+    stepper = bench.Stepper(cfg, use_graph=False)
+    stepper.keep_outputs = True
+    for i in list(range(warmup)) + list(range(steps)):
+        stepper(Tensor(x_dev[i % 2]), Tensor(y_dev[i % 2]))
+    names = bench.dump_outputs(stepper, str(tmp_path / "here"))
+    assert names == ["layer%d_%s" % (i, k) for i in (0, 2, 4, 6, 8) for k in ("b", "w")] + ["loss", "prediction"]
+    assert sorted(f[:-len(".npy")] for f in os.listdir(str(tmp_path / "bench"))) == names
+    for n in names:
+        got = np.load(str(tmp_path / "bench" / (n + ".npy")))
+        want = np.load(str(tmp_path / "here" / (n + ".npy")))
+        assert got.dtype == np.float32 and got.shape == want.shape, n
+        assert op_cases.rel_err(got, want) <= 1e-6, n
+    assert float(np.load(str(tmp_path / "bench" / "loss.npy"))) == line["final_loss"]
+    assert np.load(str(tmp_path / "bench" / "prediction.npy")).shape == (B, C)
+
+
 def test_prefetch_iterator_delivers_the_right_rows():
     """utils.data_iterator.PrefetchIterator: host data set -> device batches over the copy stream
     (pinned in place without shuffling, staged with shuffling); every batch must hold exactly the

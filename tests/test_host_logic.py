@@ -273,6 +273,39 @@ def test_reference_arm_runs_on_cpu_and_reports_its_sample():
     assert "128 of its 128 rows" in line["cpu_baseline"]["sample"]
 
 
+def test_bench_dump_outputs_writes_float_arrays_and_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs on stand-in tensors: one float32/float64 .npy per output, outputs
+    larger than DUMP_SAMPLE cut to the same sorted sample on every run, and the wide MLP's dump
+    (loss, prediction, 4 weights, 4 biases) stays under 64 MB"""
+    import types
+    sys.path.insert(0, ROOT)
+    import bench
+
+    def t(a):
+        return types.SimpleNamespace(values=a)
+    rng = np.random.RandomState(0)
+    pred = np.arange(bench.DUMP_SAMPLE + 12, dtype=np.float32).reshape(-1, 4)   # value = flat index
+    w, b = rng.standard_normal((6, 3)).astype(np.float32), np.arange(3.0)
+    net = types.SimpleNamespace(get_parameters=lambda: [{"w": t(w), "b": t(b)}, {}])
+    stepper = types.SimpleNamespace(outputs=(t(np.float32(2.5)), t(pred)), net=net)
+    names = bench.dump_outputs(stepper, str(tmp_path / "a"))
+    assert names == ["layer0_b", "layer0_w", "loss", "prediction"]
+    assert bench.dump_outputs(stepper, str(tmp_path / "b")) == names
+    got = {n: np.load(str(tmp_path / "a" / (n + ".npy"))) for n in names}
+    for n in names:
+        assert np.array_equal(got[n], np.load(str(tmp_path / "b" / (n + ".npy")))), n
+    assert got["loss"].dtype == np.float32 and float(got["loss"]) == 2.5
+    assert got["layer0_b"].dtype == np.float64 and np.array_equal(got["layer0_b"], b)
+    assert np.array_equal(got["layer0_w"], w)
+    sample = got["prediction"]
+    assert sample.dtype == np.float32 and sample.shape == (bench.DUMP_SAMPLE,)
+    assert np.all(np.diff(sample) > 0) and 0 <= sample[0] and sample[-1] < pred.size   # sorted distinct indices
+    assert (1 + 4) * bench.DUMP_SAMPLE * 4 + 4 * 4096 * 4 + 4 <= 64 << 20
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps must be at least 1" in out.stderr
+
+
 def test_numa_binding_helpers():
     sys.path.insert(0, ROOT)
     import core._dist as dist
