@@ -120,6 +120,10 @@ _SIGNATURES = {
     "tnn_relu_fwd": [_c_int, _c_vp, _c_vp, _c_i64],
     "tnn_relu_bwd": [_c_int, _c_vp, _c_vp, _c_vp, _c_i64],
     "tnn_colsum": [_c_int, _c_vp, _c_vp, _c_i64, _c_i64],
+    "tnn_im2col": [_c_int, _c_vp, _c_vp] + [_c_i64] * 12,
+    "tnn_col2im": [_c_int, _c_vp, _c_vp] + [_c_i64] * 12,
+    "tnn_maxpool_fwd": [_c_int, _c_vp, _c_vp, _c_vp] + [_c_i64] * 12,
+    "tnn_maxpool_bwd": [_c_int, _c_vp, _c_vp, _c_vp] + [_c_i64] * 12,
     "tnn_ce_stats": [_c_int, _c_vp, _c_i64, _c_i64, _c_vp],
     "tnn_ce_merge_stats": [_c_int, _c_vp, _c_vp, _c_int],
     "tnn_ce_loss": [_c_int, _c_vp, _c_int, _c_vp, _c_i64, _c_i64, _c_vp, _c_dbl, _c_vp, _c_vp, _c_vp],
@@ -1157,6 +1161,47 @@ def relu_bwd(g, x):
     out = empty(x.shape, x.dtype)
     if x.size and _lib.tnn_relu_bwd(_DT_CODE[x.dtype], out.ptr, g.ptr, x.ptr, x.size):
         _raise("tnn_relu_bwd")
+    return out
+
+
+# NHWC window passes (csrc/conv.cu).  `geom` = (KH, KW, SH, SW, PH0, PW0, OH, OW): window, stride,
+# padding before the first row / column and output extent, as core.layers.window_geometry gives them.
+def im2col(x, geom):
+    """(N, H, W, C) -> col (N*OH*OW, KH*KW*C), zeros where a window reaches into the padding"""
+    N, H, W, C = x.shape
+    KH, KW, _, _, _, _, OH, OW = geom
+    out = empty((N * OH * OW, KH * KW * C), x.dtype)
+    if out.size and _lib.tnn_im2col(_DT_CODE[x.dtype], out.ptr, x.ptr, N, H, W, C, *geom):
+        _raise("tnn_im2col")
+    return out
+
+
+def col2im(dcol, x_shape, geom):
+    """adjoint of im2col: dx of shape x_shape, each element the sum of the dcol entries that read it"""
+    N, H, W, C = x_shape
+    out = empty(x_shape, dcol.dtype)
+    if out.size and _lib.tnn_col2im(_DT_CODE[dcol.dtype], out.ptr, dcol.ptr, N, H, W, C, *geom):
+        _raise("tnn_col2im")
+    return out
+
+
+def maxpool_fwd(x, geom):
+    """(y, arg): the window maxima (N, OH, OW, C) and, as int32, each one's offset in its window"""
+    N, H, W, C = x.shape
+    OH, OW = geom[6], geom[7]
+    y = empty((N, OH, OW, C), x.dtype)
+    arg = empty((N, OH, OW, C), np.int32)
+    if y.size and _lib.tnn_maxpool_fwd(_DT_CODE[x.dtype], y.ptr, arg.ptr, x.ptr, N, H, W, C, *geom):
+        _raise("tnn_maxpool_fwd")
+    return y, arg
+
+
+def maxpool_bwd(g, arg, x_shape, geom):
+    """dx of shape x_shape: each element sums the gradients of the windows that selected it"""
+    N, H, W, C = x_shape
+    out = empty(x_shape, g.dtype)
+    if out.size and _lib.tnn_maxpool_bwd(_DT_CODE[g.dtype], out.ptr, g.ptr, arg.ptr, N, H, W, C, *geom):
+        _raise("tnn_maxpool_bwd")
     return out
 
 

@@ -1,10 +1,13 @@
 """Layers (interface of the reference's core/layers.py: Layer, Dense, Activation, Sigmoid, Tanh,
-ReLU; `params` dicts, `inputs` bookkeeping, lazy Dense initialisation).
+ReLU; `params` dicts, `inputs` bookkeeping, lazy Dense initialisation), plus the NHWC image layers
+Conv2D, MaxPool2D and Flatten of the tinynn family.
 
 Dense is one fused GEMM(+bias) node; together with a following ReLU it is one launch (see
 core/nn.py).  Activations are compositions of the op library, which routes `clip(x, 0.0)` to the
-fused ReLU kernels.
+fused ReLU kernels.  Conv2D is im2col + that same Dense node.
 """
+import numpy as np
+
 import core.ops as ops
 from core.initializer import XavierUniformInit
 from core.initializer import ZerosInit
@@ -68,6 +71,128 @@ class Dense(Layer):
         pre_activation, activated = ops.dense_relu_(inputs, w, b)
         relu_layer.inputs = pre_activation
         return activated
+
+
+def _pair(v, what):
+    """an int or a pair of ints -> (rows, columns), both >= 1"""
+    pair = (v, v) if isinstance(v, (int, np.integer)) else tuple(v)
+    if len(pair) != 2 or not all(isinstance(p, (int, np.integer)) and p >= 1 for p in pair):
+        raise ValueError("%s must be a positive int or a pair of them, got %r" % (what, v))
+    return int(pair[0]), int(pair[1])
+
+
+def _check_padding(padding):
+    if padding not in ("SAME", "VALID"):
+        raise ValueError("padding must be 'SAME' or 'VALID', got %r" % (padding,))
+    return padding
+
+
+def window_geometry(in_hw, window_hw, stride_hw, padding):
+    """Output extent and leading padding of a sliding window over an (H, W) image, per dimension:
+
+      "VALID": no padding, O = (I - K) // S + 1; a ValueError if I < K.
+      "SAME":  K - 1 padded positions in total, (K - 1) // 2 before the first row / column and the rest
+               after it (an even window pads one more after than before), O = ceil(I / S).
+
+    Returns ((OH, OW), (PH0, PW0)).  Used by Conv2D and MaxPool2D."""
+    _check_padding(padding)
+    out, before = [], []
+    for i, k, s in zip(in_hw, window_hw, stride_hw):
+        if padding == "VALID":
+            if i < k:
+                raise ValueError("VALID padding: input extent %d is smaller than the window %d" % (i, k))
+            out.append((i - k) // s + 1)
+            before.append(0)
+        else:
+            out.append(-(-i // s))
+            before.append((k - 1) // 2)
+    return tuple(out), tuple(before)
+
+
+def _check_nhwc(layer, inputs, channels=None):
+    shape = tuple(inputs.shape)
+    if len(shape) != 4 or (channels is not None and shape[3] != channels):
+        want = "(N, H, W, %d)" % channels if channels is not None else "(N, H, W, C)"
+        raise ValueError("%s: input of shape %s does not match %s" % (layer, shape, want))
+    return shape
+
+
+class Conv2D(Layer):
+    """2-D convolution over NHWC float32 / float64 inputs:
+
+        y[n, oh, ow, o] = b[o] + sum_{kh, kw, c} xpad[n, oh*SH + kh, ow*SW + kw, c] * w[kh, kw, c, o]
+
+    kernel = (KH, KW, C_in, C_out); params["w"] has that shape and params["b"] is (1, C_out), as for
+    Dense; both are drawn at construction, w then b, by calling the initialisers with those shapes.
+    stride is an int or an (SH, SW) pair.  padding is "SAME" or "VALID" (see window_geometry: SAME
+    pads K - 1 positions per dimension, (K - 1) // 2 of them before, and gives ceil(I / S) outputs).
+    An input that is not 4-D or whose channel count is not C_in is a ValueError.
+
+    The layer is a composition of existing nodes: im2col_ lays the windows out as rows of a
+    (N*OH*OW, KH*KW*C_in) matrix, which is multiplied by w viewed as (KH*KW*C_in, C_out) through the
+    Dense node (bias in the GEMM epilogue, the usual tensor-core / SIMT routing), and the product is
+    viewed as (N, OH, OW, C_out).  The col matrix lives until backward, as a Dense input does."""
+
+    def __init__(self, kernel, stride=(1, 1), padding="SAME", w_init=XavierUniformInit(), b_init=ZerosInit()):
+        Layer.__init__(self, "Conv2D")
+        kernel = tuple(kernel)
+        if len(kernel) != 4 or not all(isinstance(k, (int, np.integer)) and k >= 1 for k in kernel):
+            raise ValueError("kernel must be (KH, KW, C_in, C_out) positive ints, got %r" % (kernel,))
+        self.kernel = tuple(int(k) for k in kernel)
+        self.stride = _pair(stride, "stride")
+        self.padding = _check_padding(padding)
+        self.initializers = {"w": w_init, "b": b_init}
+        shapes = {"w": list(self.kernel), "b": [1, self.kernel[3]]}
+        for key in ("w", "b"):
+            tensor = self.initializers[key](shape=shapes[key])
+            tensor.zero_grad()
+            self.params[key] = tensor
+        self.inputs = None
+
+    def forward(self, inputs):
+        KH, KW, C, O = self.kernel
+        N, H, W, _ = _check_nhwc("Conv2D", inputs, C)
+        out_hw, pads = window_geometry((H, W), (KH, KW), self.stride, self.padding)
+        self.inputs = inputs
+        col = ops.im2col_(inputs, KH, KW, self.stride, pads, out_hw)
+        w2 = ops.reshape_(self.params["w"], (KH * KW * C, O))
+        z = ops.dense_(col, w2, self.params["b"])
+        return ops.reshape_(z, (N, out_hw[0], out_hw[1], O))
+
+
+class MaxPool2D(Layer):
+    """Window maxima over NHWC inputs.  stride=None means stride = pool_size; padding as Conv2D's
+    (window_geometry), and padded positions are never selected (SAME leaves at least one real element
+    in every window).  The selected element is the first maximum in row-major window order -- np.argmax
+    over the flattened window -- or the first NaN, which makes the output NaN, as np.max does.  Each
+    output's gradient goes wholly to its selected input; where windows overlap (stride < pool_size)
+    the contributions are summed.  (Unlike the reference's max_, tied elements do not all receive it.)"""
+
+    def __init__(self, pool_size=(2, 2), stride=None, padding="VALID"):
+        Layer.__init__(self, "MaxPool2D")
+        self.pool_size = _pair(pool_size, "pool_size")
+        self.stride = self.pool_size if stride is None else _pair(stride, "stride")
+        self.padding = _check_padding(padding)
+        self.inputs = None
+
+    def forward(self, inputs):
+        N, H, W, C = _check_nhwc("MaxPool2D", inputs)
+        out_hw, pads = window_geometry((H, W), self.pool_size, self.stride, self.padding)
+        self.inputs = inputs
+        return ops.maxpool2d_(inputs, self.pool_size, self.stride, pads, out_hw)
+
+
+class Flatten(Layer):
+    """(N, ...) -> (N, prod(...)), a view (no kernel)"""
+
+    def __init__(self):
+        Layer.__init__(self, "Flatten")
+        self.inputs = None
+
+    def forward(self, inputs):
+        self.inputs = inputs
+        shape = tuple(inputs.shape)
+        return ops.reshape_(inputs, (shape[0], int(np.prod(shape[1:], dtype=np.int64))))
 
 
 class Activation(Layer):

@@ -6,7 +6,8 @@ to /root/reference/core/ops.py.
 A grad_fn receives the incoming gradient as a device array and returns a device array; the
 un-broadcast reduction the reference inlines twelve times (ops.py:41-46 ...) is one backend call.
 Three fused nodes are added for the training path (dense_, relu_, softmax_ce_); they are what
-core/layers.py and core/losses.py use.
+core/layers.py and core/losses.py use.  Two more serve the NHWC image layers: im2col_ (Conv2D's
+window matrix) and maxpool2d_.
 """
 import builtins as _bi
 
@@ -583,6 +584,38 @@ def dense_relu_(ts_x, ts_w, ts_b):
     ts_a = build_unary_ops_tensor(ts_z, relu_grad, av)
     ts_a._relu_pre = zv
     return ts_z, ts_a
+
+
+def im2col_(ts, KH, KW, stride, pads, out_hw):
+    """NHWC x (N, H, W, C) -> col (N*OH*OW, KH*KW*C): row (n, oh, ow) holds the window of output pixel
+    (oh, ow), columns in (kh, kw, c) order, zeros where the window reaches into the padding.  `pads` is
+    the padding before the first row and column.  Backward is the adjoint (tnn_col2im, a gather)."""
+    x = ts._data
+    geom = (KH, KW, stride[0], stride[1], pads[0], pads[1], out_hw[0], out_hw[1])
+    values = be.im2col(x, geom)
+
+    def grad_fn(grad):
+        if grad.dtype != x.dtype:
+            grad = be.astype(grad, x.dtype)
+        return be.col2im(grad, x.shape, geom)
+
+    return build_unary_ops_tensor(ts, grad_fn, values)
+
+
+def maxpool2d_(ts, pool, stride, pads, out_hw):
+    """NHWC window maxima; the selected element of each window (the first maximum in row-major window
+    order, or the first NaN) is kept as an int32 offset for backward, which hands each output's
+    gradient wholly to it (summed where windows overlap)."""
+    x = ts._data
+    geom = (pool[0], pool[1], stride[0], stride[1], pads[0], pads[1], out_hw[0], out_hw[1])
+    values, arg = be.maxpool_fwd(x, geom)
+
+    def grad_fn(grad):
+        if grad.dtype != x.dtype:
+            grad = be.astype(grad, x.dtype)
+        return be.maxpool_bwd(grad, arg, x.shape, geom)
+
+    return build_unary_ops_tensor(ts, grad_fn, values)
 
 
 def softmax_ce_(ts_logits, ts_labels):

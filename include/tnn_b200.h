@@ -309,6 +309,33 @@ int tnn_relu_bwd(int dtype, void* dx, const void* g, const void* x, int64_t n);
 /* column sum of a (R, C) gradient = bias gradient (ops.py:49-55 on the (1,N) bias) */
 int tnn_colsum(int dtype, void* out, const void* g, int64_t R, int64_t C);
 
+/* ---- convolution / pooling passes, NHWC (new: no reference counterpart) ---------------------
+ * Conv2D is im2col + the GEMM route above (core/layers.py); MaxPool2D is one pass each way.
+ * x is (N, H, W, C) contiguous; the window is (KH, KW) (pooling: (PH, PW)), the stride (SH, SW),
+ * PH0 / PW0 the padding before the first row / column, (OH, OW) the output extent.  One launch
+ * each, no atomics (the backward passes gather in a fixed order: bit-reproducible), no host sync.
+ * tnn_im2col: col[(n,oh,ow), (kh,kw,c)] = x[n, oh*SH+kh-PH0, ow*SW+kw-PW0, c], 0 in the padding;
+ *   col is (N*OH*OW, KH*KW*C) row-major, so col @ w.reshape(KH*KW*C, C_out) is the convolution.
+ * tnn_col2im: its adjoint, dx (N, H, W, C) WRITTEN (not accumulated): each element sums the dcol
+ *   entries that read it, in ascending (kh, kw) order. */
+int tnn_im2col(int dtype, void* col, const void* x, int64_t N, int64_t H, int64_t W, int64_t C,
+               int64_t KH, int64_t KW, int64_t SH, int64_t SW, int64_t PH0, int64_t PW0,
+               int64_t OH, int64_t OW);
+int tnn_col2im(int dtype, void* dx, const void* dcol, int64_t N, int64_t H, int64_t W, int64_t C,
+               int64_t KH, int64_t KW, int64_t SH, int64_t SW, int64_t PH0, int64_t PW0,
+               int64_t OH, int64_t OW);
+/* tnn_maxpool_fwd: y (N, OH, OW, C) = max over the real (unpadded) elements of each window, and
+ *   arg (same shape, int32) = the selected element's offset INSIDE its window, kh*PW + kw: the first
+ *   maximum in row-major window order, or the first NaN (np.max / np.argmax of the window).
+ * tnn_maxpool_bwd: dx (N, H, W, C) WRITTEN: each element sums dy over the windows that cover it and
+ *   whose arg points at it (overlapping windows included). */
+int tnn_maxpool_fwd(int dtype, void* y, int32_t* arg, const void* x, int64_t N, int64_t H, int64_t W,
+                    int64_t C, int64_t PH, int64_t PW, int64_t SH, int64_t SW, int64_t PH0, int64_t PW0,
+                    int64_t OH, int64_t OW);
+int tnn_maxpool_bwd(int dtype, void* dx, const void* dy, const int32_t* arg, int64_t N, int64_t H,
+                    int64_t W, int64_t C, int64_t PH, int64_t PW, int64_t SH, int64_t SW, int64_t PH0,
+                    int64_t PW0, int64_t OH, int64_t OW);
+
 /* SoftmaxCrossEntropyLoss.loss (losses.py:24-32) with its batch-GLOBAL max and normaliser.
  * Stage 1: local max + local sum exp(z - local max) -> stats_dev[0..1] (device, dtype of z).
  * (data parallel: all-gather stats across ranks, merge on host or with tnn_ce_merge_stats)
