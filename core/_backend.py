@@ -124,6 +124,11 @@ _SIGNATURES = {
     "tnn_col2im": [_c_int, _c_vp, _c_vp] + [_c_i64] * 12,
     "tnn_maxpool_fwd": [_c_int, _c_vp, _c_vp, _c_vp] + [_c_i64] * 12,
     "tnn_maxpool_bwd": [_c_int, _c_vp, _c_vp, _c_vp] + [_c_i64] * 12,
+    "tnn_bn_stats": [_c_int, _c_vp, _c_i64, _c_i64, _c_dbl, _c_dbl, _c_vp, _c_vp, _c_vp, _c_vp],
+    "tnn_bn_merge": [_c_int, _c_vp, _c_int, _c_i64, _c_dbl, _c_dbl, _c_vp, _c_vp, _c_vp],
+    "tnn_bn_apply": [_c_int, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_dbl],
+    "tnn_bn_bwd_reduce": [_c_int, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_int, _c_vp, _c_int],
+    "tnn_bn_dx": [_c_int, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp],
     "tnn_ce_stats": [_c_int, _c_vp, _c_i64, _c_i64, _c_vp],
     "tnn_ce_merge_stats": [_c_int, _c_vp, _c_vp, _c_int],
     "tnn_ce_loss": [_c_int, _c_vp, _c_int, _c_vp, _c_i64, _c_i64, _c_vp, _c_dbl, _c_vp, _c_vp, _c_vp],
@@ -1203,6 +1208,65 @@ def maxpool_bwd(g, arg, x_shape, geom):
     if out.size and _lib.tnn_maxpool_bwd(_DT_CODE[g.dtype], out.ptr, g.ptr, arg.ptr, N, H, W, C, *geom):
         _raise("tnn_maxpool_bwd")
     return out
+
+
+# Batch normalisation passes (csrc/batchnorm.cu) on an (M, C) view.  `mr` is the (2C + 1,) float64
+# array of column means, r = 1/sqrt(var + eps) and the row count the statistics cover.
+def bn_stats(x, momentum, eps, running_mean, running_var, local=False):
+    """TRAIN statistics of x (M, C): mr, with the running statistics updated in place -- or, with
+    `local`, this rank's (M, mean[C], M2[C]) as a (1 + 2C,) float64 array and nothing updated"""
+    M, C = x.shape
+    out = empty((1 + 2 * C,) if local else (2 * C + 1,), F64)
+    mr, part = (None, out.ptr) if local else (out.ptr, None)
+    if _lib.tnn_bn_stats(_DT_CODE[x.dtype], x.ptr, M, C, float(momentum), float(eps), running_mean.ptr,
+                         running_var.ptr, mr, part):
+        _raise("tnn_bn_stats")
+    return out
+
+
+def bn_merge(gathered, world, C, momentum, eps, running_mean, running_var):
+    """`world` ranks' local statistics (bn_stats(local=True), gathered in rank order) -> mr, with the
+    running statistics updated in place"""
+    mr = empty((2 * C + 1,), F64)
+    if _lib.tnn_bn_merge(_DT_CODE[running_mean.dtype], gathered.ptr, world, C, float(momentum), float(eps),
+                         running_mean.ptr, running_var.ptr, mr.ptr):
+        _raise("tnn_bn_merge")
+    return mr
+
+
+def bn_apply(x, gamma, beta, mr=None, running=None, eps=0.0):
+    """(y, mr): y = (x - mean) * r * gamma + beta with the statistics of mr (TRAIN) or, given
+    running = (running_mean, running_var), of the running statistics (TEST; mr is then made here)"""
+    M, C = x.shape
+    y = empty((M, C), x.dtype)
+    if running is not None:
+        mr = empty((2 * C + 1,), F64)
+    rm, rv = (running[0].ptr, running[1].ptr) if running is not None else (None, None)
+    if _lib.tnn_bn_apply(_DT_CODE[x.dtype], y.ptr, x.ptr, M, C, gamma.ptr, beta.ptr, mr.ptr, rm, rv, float(eps)):
+        _raise("tnn_bn_apply")
+    return y, mr
+
+
+def bn_bwd_reduce(g, x, mr, dgamma, acc_gamma, dbeta, acc_beta):
+    """(sum dy, sum dy * xhat) per column as one (2C,) float64 array; dbeta / dgamma (C values each,
+    or None) receive the two halves, written or (acc_*) added"""
+    M, C = x.shape
+    sums = empty((2 * C,), F64)
+    if _lib.tnn_bn_bwd_reduce(_DT_CODE[x.dtype], g.ptr, x.ptr, M, C, mr.ptr, sums.ptr,
+                              dgamma.ptr if dgamma is not None else None, int(acc_gamma),
+                              dbeta.ptr if dbeta is not None else None, int(acc_beta)):
+        _raise("tnn_bn_bwd_reduce")
+    return sums
+
+
+def bn_dx(g, x, mr, gamma, sums=None):
+    """dx of the normalisation: with the batch statistics' terms when `sums` is given (TRAIN)"""
+    M, C = x.shape
+    dx = empty((M, C), x.dtype)
+    if _lib.tnn_bn_dx(_DT_CODE[x.dtype], dx.ptr, g.ptr, x.ptr, M, C, mr.ptr, gamma.ptr,
+                      sums.ptr if sums is not None else None):
+        _raise("tnn_bn_dx")
+    return dx
 
 
 def ce_stats(z):

@@ -7,6 +7,8 @@ compute stream, driven through libtnn_b200.so:
     global batch size, so no averaging)
   * merge_ce_stats -- all-gather of the (max, sum-exp) pair so SoftmaxCrossEntropyLoss keeps the
     reference's batch-global normaliser under row sharding.
+  * bn_global_stats / an all-reduce of 2C sums -- BatchNormalization's TRAIN statistics and their
+    backward sums span the global batch (core/ops.py batchnorm_).
 """
 import ctypes
 import os
@@ -177,6 +179,36 @@ def merge_ce_stats(stats):
     if be._lib.tnn_allgather(be._DT_CODE[stats.dtype], gathered.ptr, stats.ptr, 2):
         be._raise("tnn_allgather")
     return be.ce_merge_stats(gathered, _world)
+
+
+def bn_global_stats(x, momentum, eps, running_mean, running_var):
+    """BatchNormalization's TRAIN statistics over the GLOBAL batch: each rank's (count, mean, M2) per
+    column, 1 + 2C float64 values, are all-gathered over NCCL and merged in rank order on the device,
+    so every rank gets the same mean, r and running statistics"""
+    C = x.shape[1]
+    part = be.bn_stats(x, momentum, eps, running_mean, running_var, local=True)
+    if _world == 1:
+        gathered = part
+    else:
+        gathered = be.empty((_world * (1 + 2 * C),), be.F64)
+        if be._lib.tnn_allgather(be._DT_CODE[be.F64], gathered.ptr, part.ptr, 1 + 2 * C):
+            be._raise("tnn_allgather")
+    return be.bn_merge(gathered, _world, C, momentum, eps, running_mean, running_var)
+
+
+def merge_bn_stats_host(parts):
+    """[(n_r, mean_r[C], M2_r[C])] in rank order -> (n, mean[C], M2[C]) with Chan's pairwise update,
+    the order and formulas of tnn_bn_merge (host mirror, used by the CPU tests of the scheme)"""
+    n, mean, m2 = 0.0, 0.0, 0.0
+    for nb, mb, m2b in parts:
+        if nb == 0:
+            continue
+        tot = n + nb
+        delta = np.asarray(mb, np.float64) - mean
+        mean = mean + delta * (nb / tot)
+        m2 = m2 + np.asarray(m2b, np.float64) + delta * delta * (n * nb / tot)
+        n = tot
+    return n, mean, m2
 
 
 def barrier():

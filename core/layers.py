@@ -9,16 +9,21 @@ fused ReLU kernels.  Conv2D is im2col + that same Dense node.
 import numpy as np
 
 import core.ops as ops
+from core.initializer import ConstantInit
 from core.initializer import XavierUniformInit
 from core.initializer import ZerosInit
+from core.tensor import Tensor
 
 
 class Layer(object):
-    """Base class: a name, a dict of parameter tensors and the TRAIN/TEST flag."""
+    """Base class: a name, a dict of parameter tensors, a dict of state tensors that are not
+    parameters (`buffers`: saved and loaded with the parameters, never optimised) and the
+    TRAIN/TEST flag."""
 
     def __init__(self, name):
         self.name = name
         self.params = {}
+        self.buffers = {}
         self.grads = {}
         self.is_training = True
 
@@ -180,6 +185,68 @@ class MaxPool2D(Layer):
         out_hw, pads = window_geometry((H, W), self.pool_size, self.stride, self.padding)
         self.inputs = inputs
         return ops.maxpool2d_(inputs, self.pool_size, self.stride, pads, out_hw)
+
+
+class BatchNormalization(Layer):
+    """Batch normalisation over every axis but the last: a (N, C) Dense output or an (N, H, W, C)
+    NHWC Conv2D output is normalised per channel over its N (or N*H*W) rows M,
+
+        y = (x - mean) * gamma / sqrt(var + epsilon) + beta
+
+    params["gamma"] and params["beta"] are (1, C), drawn at construction in that order through the
+    initialisers.  layer.buffers holds the running statistics, running_mean (starts at 0) and
+    running_var (starts at 1): (1, C) device tensors of the parameters' dtype without gradients, not
+    parameters (the optimiser does not see them), saved and loaded with them by Model.save / load.
+
+    TRAIN phase: mean and the biased variance of the batch (of the global batch under data
+    parallelism), and running = (1 - momentum) * running + momentum * batch value with the unbiased
+    variance (* M / (M - 1)) -- the torch conventions.  The phase decides, not the grad mode: a
+    forward under no_grad() in TRAIN also updates them.  M < 2 is a ValueError there.
+    TEST phase: the running statistics, unchanged; gradients still flow.  An empty batch is allowed.
+
+    The input must be 2-D or 4-D with a last axis of num_features and share gamma's dtype (float32
+    or float64); anything else is a ValueError.  momentum and epsilon are fixed at construction."""
+
+    def __init__(self, num_features, momentum=0.1, epsilon=1e-5, gamma_init=ConstantInit(1.0),
+                 beta_init=ZerosInit()):
+        Layer.__init__(self, "BatchNormalization")
+        if not isinstance(num_features, (int, np.integer)) or num_features < 1:
+            raise ValueError("num_features must be a positive int, got %r" % (num_features,))
+        self.num_features = int(num_features)
+        self.momentum = float(momentum)
+        self.epsilon = float(epsilon)
+        self.initializers = {"gamma": gamma_init, "beta": beta_init}
+        for key in ("gamma", "beta"):
+            tensor = self.initializers[key](shape=[1, self.num_features])
+            tensor.zero_grad()
+            self.params[key] = tensor
+        dt = self.params["gamma"].dtype
+        self.buffers = {"running_mean": Tensor(np.zeros((1, self.num_features), dt), dtype=dt),
+                        "running_var": Tensor(np.ones((1, self.num_features), dt), dtype=dt)}
+        self.inputs = None
+
+    def _check(self, inputs):
+        shape = tuple(inputs.shape)
+        if len(shape) not in (2, 4) or shape[-1] != self.num_features:
+            raise ValueError("BatchNormalization: input of shape %s does not match (N, %d) or (N, H, W, %d)"
+                             % (shape, self.num_features, self.num_features))
+        dt = self.params["gamma"].dtype
+        if inputs.dtype != dt or self.params["beta"].dtype != dt:
+            raise ValueError("BatchNormalization: input dtype %s and gamma / beta dtype %s / %s differ"
+                             % (inputs.dtype, dt, self.params["beta"].dtype))
+        rows = int(np.prod(shape[:-1], dtype=np.int64))
+        if self.is_training and rows < 2:
+            raise ValueError("BatchNormalization: TRAIN phase needs at least 2 values per channel, got %d "
+                             "(input of shape %s)" % (rows, shape))
+
+    def forward(self, inputs):
+        self._check(inputs)
+        dt = self.params["gamma"].dtype
+        for buf in self.buffers.values():
+            if buf.dtype != dt:          # gamma / beta were replaced by tensors of another dtype
+                buf.values = np.asarray(buf.values, dt)
+        self.inputs = inputs
+        return ops.batchnorm_(inputs, self.params["gamma"], self.params["beta"], self, self.is_training)
 
 
 class Flatten(Layer):

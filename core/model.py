@@ -96,8 +96,13 @@ class Model(object):
 
     # ------------------------------------------------------------------ checkpoint (values only)
     def save(self, path):
-        state = [{k: v.values for k, v in layer.items() if v is not None}
-                 for layer in self.net.get_parameters()]
+        """one dict per layer: its parameters' values, then its buffers' (BatchNormalization's
+        running statistics) under their own names"""
+        state = []
+        for layer, params in zip(self.net.layers, self.net.get_parameters()):
+            entry = {k: v.values for k, v in params.items() if v is not None}
+            entry.update((k, v.values) for k, v in getattr(layer, "buffers", {}).items())
+            state.append(entry)
         with open(path, "wb") as f:
             pickle.dump(state, f, -1)
         print("Model saved in %s." % path)
@@ -117,6 +122,15 @@ class Model(object):
                              % (len(state), len(params)))
         for layer, saved in zip(self.net.layers, state):
             for k, arr in saved.items():
+                buf = getattr(layer, "buffers", {}).get(k)
+                if buf is not None:
+                    # copied into the existing device array: a recorded step that names it stays valid
+                    if tuple(buf.shape) != tuple(arr.shape):
+                        raise ValueError("Incompatible architecture. %s in loaded model and %s in "
+                                         "defined model." % (arr.shape, buf.shape))
+                    be.upload_into(buf._data, arr)
+                    buf._touch()
+                    continue
                 cur = layer.params.get(k)
                 if cur is not None and tuple(cur.shape) != tuple(arr.shape):
                     raise ValueError("Incompatible architecture. %s in loaded model and %s in "
@@ -546,6 +560,9 @@ class _CapturedStep(object):
         for p in self.plist:
             p._touch()
             p._drop_grad()   # as after the eager step(): `param += step` leaves grad = None (tensor.py:35-38)
+        for layer in self.layers:
+            for buf in getattr(layer, "buffers", {}).values():
+                buf._touch()     # updated in place by the replay (running statistics)
         # the loss buffer is rewritten by the next replay: hand out a copy
         return Tensor(be.clone(self.loss))
 

@@ -7,7 +7,7 @@ A grad_fn receives the incoming gradient as a device array and returns a device 
 un-broadcast reduction the reference inlines twelve times (ops.py:41-46 ...) is one backend call.
 Three fused nodes are added for the training path (dense_, relu_, softmax_ce_); they are what
 core/layers.py and core/losses.py use.  Two more serve the NHWC image layers: im2col_ (Conv2D's
-window matrix) and maxpool2d_.
+window matrix) and maxpool2d_; batchnorm_ is BatchNormalization.
 """
 import builtins as _bi
 
@@ -616,6 +616,99 @@ def maxpool2d_(ts, pool, stride, pads, out_hw):
         return be.maxpool_bwd(grad, arg, x.shape, geom)
 
     return build_unary_ops_tensor(ts, grad_fn, values)
+
+
+def batchnorm_(ts_x, ts_gamma, ts_beta, layer_state, training):
+    """Batch normalisation of x (..., C) over every axis but the last, viewed as (M, C):
+
+        y = (x - mean) * gamma / sqrt(var + eps) + beta
+
+    `layer_state` carries `buffers` (running_mean, running_var: (1, C) tensors without gradients),
+    `momentum` and `epsilon` -- the BatchNormalization layer.  TRAIN (`training`): mean and the biased
+    variance of this batch (of the global batch under data parallelism), and the running statistics
+    are updated in place, running = (1 - momentum) * running + momentum * batch value with the
+    unbiased variance.  TEST: the running statistics, left unchanged.  Two launches forward (TRAIN;
+    one in TEST), two backward.
+
+    The node depends on x, gamma and beta and keeps x and mr -- the per-column mean, r = 1/sqrt(var +
+    eps) and row count -- for backward, which recomputes xhat = (x - mean) * r from them: dbeta =
+    sum dy, dgamma = sum dy * xhat (one reduction whose fold writes them straight into the arena slots
+    through _fused_bwd), dx = gamma * r * (dy - sum dy / M - xhat * sum(dy * xhat) / M), or gamma * r * dy
+    in TEST.  Under data parallelism the two sums are all-reduced before dx, and the slots receive this
+    rank's partials: Model.step's gradient all-reduce completes them."""
+    import core._dist as dist
+    x = ts_x._data
+    shape = x.shape
+    C = shape[-1]
+    M = x.size // C
+    x2 = x.view((M, C))
+    gamma, beta = ts_gamma._data, ts_beta._data
+    rm, rv = layer_state.buffers["running_mean"], layer_state.buffers["running_var"]
+    eps = layer_state.epsilon
+    world = dist.world_size()
+    if training:
+        if world > 1:
+            mr = dist.bn_global_stats(x2, layer_state.momentum, eps, rm._data, rv._data)
+        else:
+            mr = be.bn_stats(x2, layer_state.momentum, eps, rm._data, rv._data)
+        rm._touch()
+        rv._touch()
+        values, _ = be.bn_apply(x2, gamma, beta, mr=mr)
+    else:
+        values, mr = be.bn_apply(x2, gamma, beta, running=(rm._data, rv._data), eps=eps)
+    values = values.view(shape)
+    cache = {}
+
+    def _as_x(grad):
+        if grad.dtype != x.dtype:
+            grad = be.astype(grad, x.dtype)
+        return grad.view((M, C))
+
+    def _sums(grad, dgamma=None, acc_gamma=False, dbeta=None, acc_beta=False):
+        sums = be.bn_bwd_reduce(_as_x(grad), x2, mr, dgamma, acc_gamma, dbeta, acc_beta)
+        if training and world > 1:
+            dist.allreduce_sum(sums)     # after the local partials went to dgamma / dbeta
+        return sums
+
+    def _dx(grad, sums):
+        return be.bn_dx(_as_x(grad), x2, mr, gamma, sums if training else None).view(shape)
+
+    def _param_grads(grad):
+        """(dgamma, dbeta, sums) from one reduction shared by the per-input functions below"""
+        if cache.get("grad") is not grad:
+            dg, db = be.empty((1, C), x.dtype), be.empty((1, C), x.dtype)
+            cache.update(grad=grad, dg=dg, db=db, sums=_sums(grad, dg, False, db, False))
+        return cache
+
+    def grad_fn_x(grad):
+        return _dx(grad, _param_grads(grad)["sums"] if training else None)
+
+    def grad_fn_gamma(grad):
+        return _param_grads(grad)["dg"]
+
+    def grad_fn_beta(grad):
+        return _param_grads(grad)["db"]
+
+    def fused_bwd(grad, direct):
+        """dgamma and dbeta written (or added) into their arena slots by the reduction's fold"""
+        if ts_gamma is ts_beta or id(ts_gamma) not in direct or id(ts_beta) not in direct:
+            return None
+        (g_slot, g_acc), (b_slot, b_acc) = direct[id(ts_gamma)], direct[id(ts_beta)]
+        sums = _sums(grad, g_slot, g_acc, b_slot, b_acc)
+        out = {id(ts_gamma): WRITTEN_IN_PLACE, id(ts_beta): WRITTEN_IN_PLACE}
+        if ts_x.requires_grad:
+            out[id(ts_x)] = _dx(grad, sums)
+        return out
+
+    dependency = []
+    requires_grad = (ts_x.requires_grad or ts_gamma.requires_grad or ts_beta.requires_grad) and _GRAD_ENABLED
+    for t, fn in ((ts_x, grad_fn_x), (ts_gamma, grad_fn_gamma), (ts_beta, grad_fn_beta)):
+        if t.requires_grad and requires_grad:
+            dependency.append(dict(tensor=t, grad_fn=fn))
+    node = ts_x.__class__(values, requires_grad, dependency)
+    if requires_grad and ts_gamma.requires_grad and ts_beta.requires_grad:
+        node._fused_bwd = fused_bwd
+    return node
 
 
 def softmax_ce_(ts_logits, ts_labels):

@@ -336,6 +336,35 @@ int tnn_maxpool_bwd(int dtype, void* dx, const void* dy, const int32_t* arg, int
                     int64_t W, int64_t C, int64_t PH, int64_t PW, int64_t SH, int64_t SW, int64_t PH0,
                     int64_t PW0, int64_t OH, int64_t OW);
 
+/* ---- batch normalisation over the rows of an (M, C) matrix (new: no reference counterpart) --
+ * BatchNormalization in core/layers.py; x, y, dy, dx are (M, C) contiguous in `dtype`, gamma, beta
+ * and the running statistics are C values of the same dtype.  mr is 2C + 1 float64 values: the
+ * column means, r = 1/sqrt(var + eps) and the row count M the statistics were taken over (global
+ * under data parallelism).  Statistics and sums are float64; no atomics on values, no host sync.
+ * tnn_bn_stats: TRAIN statistics (biased variance) of x.  part == NULL: writes mr and updates the
+ *   running statistics in place, running = (1 - momentum) * running + momentum * batch value, the
+ *   variance unbiased (* M / (M - 1)); M >= 2.  part != NULL: writes the local (M, mean[C], M2[C])
+ *   to part (1 + 2C float64) instead and touches nothing else.
+ * tnn_bn_merge: `world` such parts (gathered in rank order) -> mr and the running update as above,
+ *   merged in rank order (every rank computes the same bits). */
+int tnn_bn_stats(int dtype, const void* x, int64_t M, int64_t C, double momentum, double eps, void* running_mean,
+                 void* running_var, double* mr, double* part);
+int tnn_bn_merge(int dtype, const double* gathered, int world, int64_t C, double momentum, double eps,
+                 void* running_mean, void* running_var, double* mr);
+/* tnn_bn_apply: y = (x - mean) * r * gamma + beta.  running_mean == NULL: mean and r from mr (TRAIN);
+ *   otherwise from the running statistics (TEST), and they are written to mr for backward. */
+int tnn_bn_apply(int dtype, void* y, const void* x, int64_t M, int64_t C, const void* gamma, const void* beta,
+                 double* mr, const void* running_mean, const void* running_var, double eps);
+/* tnn_bn_bwd_reduce: sums = (sum_rows dy, sum_rows dy * xhat), 2C float64, xhat = (x - mean) * r
+ *   recomputed from mr; dbeta = the first C, dgamma = the second, each WRITTEN or (acc_* != 0) added
+ *   to what it holds; a NULL dgamma / dbeta is skipped.
+ * tnn_bn_dx: dx = gamma * r * (dy - sums[c] / M - xhat * sums[C + c] / M), M = mr[2C] (TRAIN), or
+ *   dx = gamma * r * dy when sums == NULL (TEST: the statistics are constants). */
+int tnn_bn_bwd_reduce(int dtype, const void* dy, const void* x, int64_t M, int64_t C, const double* mr,
+                      double* sums, void* dgamma, int acc_gamma, void* dbeta, int acc_beta);
+int tnn_bn_dx(int dtype, void* dx, const void* dy, const void* x, int64_t M, int64_t C, const double* mr,
+              const void* gamma, const double* sums);
+
 /* SoftmaxCrossEntropyLoss.loss (losses.py:24-32) with its batch-GLOBAL max and normaliser.
  * Stage 1: local max + local sum exp(z - local max) -> stats_dev[0..1] (device, dtype of z).
  * (data parallel: all-gather stats across ranks, merge on host or with tnn_ce_merge_stats)

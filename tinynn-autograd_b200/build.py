@@ -18,7 +18,8 @@ OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libtnn_b200.so")
 
 SOURCES = ["runtime.cu", "elementwise.cu", "reduce.cu", "layout.cu", "gemm_simt.cu",
-           "gemm_tc.cu", "gemm_f16.cu", "fused.cu", "mlp_fused.cu", "comm.cu", "conv.cu"]
+           "gemm_tc.cu", "gemm_f16.cu", "fused.cu", "mlp_fused.cu", "comm.cu", "conv.cu",
+           "batchnorm.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "math.cuh"), os.path.join(CSRC, "tc_ptx.cuh"),
            os.path.join(ROOT, "include", "tnn_b200.h")]
 

@@ -36,6 +36,10 @@ void set_error(const std::string& msg);
 int fail(const char* file, int line, const std::string& msg);
 // reduction scratch on the compute stream (valid until the next call that asks for scratch)
 int get_scratch(size_t nbytes, void** out);
+// arrival counters of the split column reductions (reduce.cu, batchnorm.cu): MAX_COL_COUNTERS of them,
+// allocated on first use, each zero between launches
+constexpr int64_t MAX_COL_COUNTERS = 1 << 16;
+int col_fold_counters(unsigned int** out);
 
 // bracket a launch with events when profiling of `family` is on
 void prof_begin(int family);
@@ -139,6 +143,25 @@ struct Vec4<double> {
 };
 
 __host__ __device__ inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// A column reduction whose rows are split across nsplit CTAs: each CTA has written its partial, and
+// the LAST one to arrive for the column block (its counter `cnt`) folds them -- in split order, so
+// the result does not depend on which CTA that is.  Called by every thread of the CTA; true in the
+// last one, whose later reads see every partial.  That CTA rearms the counter for the next launch.
+__device__ __forceinline__ bool col_fold_last_arrival(unsigned int* cnt, unsigned int nsplit) {
+  __shared__ bool is_last;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0 && threadIdx.y == 0) {
+    const unsigned int prev = atomicAdd(cnt, 1u);
+    is_last = prev == nsplit - 1;
+    if (is_last) *cnt = 0u;
+  }
+  __syncthreads();
+  if (!is_last) return false;
+  __threadfence();
+  return true;
+}
 
 // grid for a grid-stride elementwise kernel: enough CTAs to fill the chip a few times over,
 // in multiples of the SM count

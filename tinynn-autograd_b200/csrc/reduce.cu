@@ -145,7 +145,6 @@ __global__ void __launch_bounds__(256)
 reduce_col_kernel(T* out, T* stage, const T* x, int64_t red, int64_t inner, int nsplit,
                   unsigned int* counters) {
   __shared__ T sm[8][32 * VEC + 1];
-  __shared__ bool is_last;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int64_t ncol = inner / VEC;
   const int64_t col = (int64_t)blockIdx.x * 32 + tx;
@@ -174,17 +173,7 @@ reduce_col_kernel(T* out, T* stage, const T* x, int64_t red, int64_t inner, int 
   }
   if (nsplit == 1) return;
   // ---- last CTA of this column block folds the partials ----
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned int* cnt = counters + o * gridDim.x + blockIdx.x;
-    const unsigned int prev = atomicAdd(cnt, 1u);
-    is_last = prev == (unsigned int)nsplit - 1;
-    if (is_last) *cnt = 0u;                      // rearmed for the next launch
-  }
-  __syncthreads();
-  if (!is_last) return;
-  __threadfence();
+  if (!col_fold_last_arrival(counters + o * gridDim.x + blockIdx.x, (unsigned int)nsplit)) return;
 #pragma unroll
   for (int k = 0; k < VEC; ++k) acc[k] = red_identity<RED, T>();
   if (col < ncol)
@@ -205,7 +194,15 @@ reduce_col_kernel(T* out, T* stage, const T* x, int64_t red, int64_t inner, int 
 }
 
 static unsigned int* g_col_counters = nullptr;     // one per (outer, column block), zero between launches
-constexpr int64_t MAX_COL_COUNTERS = 1 << 16;
+
+int col_fold_counters(unsigned int** out) {
+  if (!g_col_counters) {
+    TNN_CUDA(cudaMalloc(&g_col_counters, MAX_COL_COUNTERS * sizeof(unsigned int)));
+    TNN_CUDA(cudaMemsetAsync(g_col_counters, 0, MAX_COL_COUNTERS * sizeof(unsigned int), ctx().stream));
+  }
+  *out = g_col_counters;
+  return 0;
+}
 
 template <int RED, typename T>
 static int reduce_impl(T* out, const T* x, int64_t outer, int64_t red, int64_t inner) {
@@ -285,15 +282,13 @@ static int reduce_impl(T* out, const T* x, int64_t outer, int64_t red, int64_t i
     if (gx * outer > MAX_COL_COUNTERS) nsplit = 1;
     else if (get_scratch((size_t)(outer * nsplit * inner) * sizeof(T), &scratch)) return 1;
   }
-  if (nsplit > 1 && !g_col_counters) {
-    TNN_CUDA(cudaMalloc(&g_col_counters, MAX_COL_COUNTERS * sizeof(unsigned int)));
-    TNN_CUDA(cudaMemsetAsync(g_col_counters, 0, MAX_COL_COUNTERS * sizeof(unsigned int), st));
-  }
+  unsigned int* counters = nullptr;
+  if (nsplit > 1 && col_fold_counters(&counters)) return 1;
   dim3 grid((unsigned)gx, (unsigned)(outer * nsplit));
   if (vec)
-    reduce_col_kernel<RED, T, VW><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, g_col_counters);
+    reduce_col_kernel<RED, T, VW><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, counters);
   else
-    reduce_col_kernel<RED, T, 1><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, g_col_counters);
+    reduce_col_kernel<RED, T, 1><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, counters);
   TNN_POST_LAUNCH();
   return 0;
 }
