@@ -129,6 +129,8 @@ _SIGNATURES = {
     "tnn_bn_apply": [_c_int, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_dbl],
     "tnn_bn_bwd_reduce": [_c_int, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_int, _c_vp, _c_int],
     "tnn_bn_dx": [_c_int, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp],
+    "tnn_pointwise_loss": [_c_int, _c_int, _c_vp, _c_vp, _c_i64, _c_dbl, _c_dbl, _c_vp, _c_vp],
+    "tnn_pointwise_loss_bwd": [_c_int, _c_int, _c_vp, _c_vp, _c_vp, _c_i64, _c_dbl, _c_dbl, _c_vp],
     "tnn_ce_stats": [_c_int, _c_vp, _c_i64, _c_i64, _c_vp],
     "tnn_ce_merge_stats": [_c_int, _c_vp, _c_vp, _c_int],
     "tnn_ce_loss": [_c_int, _c_vp, _c_int, _c_vp, _c_i64, _c_i64, _c_vp, _c_dbl, _c_vp, _c_vp, _c_vp],
@@ -1267,6 +1269,34 @@ def bn_dx(g, x, mr, gamma, sums=None):
                       sums.ptr if sums is not None else None):
         _raise("tnn_bn_dx")
     return dx
+
+
+# Pointwise losses (csrc/loss.cu): MSE, MAE, Huber, sigmoid cross-entropy; the kind codes of
+# include/tnn_b200.h
+LOSS_MSE, LOSS_MAE, LOSS_HUBER, LOSS_SIGMOID_CE = range(4)
+
+
+def pointwise_loss(p, t, kind, m_global, delta=1.0, want_dp=False):
+    """(loss, dp): L = (1/m_global) sum l(p, t) over every element, one launch; with want_dp the same
+    pass also writes dL/dp for the upstream gradient 1 (else dp is None): what pointwise_loss_bwd
+    computes from backward()'s default seed, bit for bit"""
+    loss = empty((), p.dtype)
+    dp = empty(p.shape, p.dtype) if want_dp else None
+    if _lib.tnn_pointwise_loss(_DT_CODE[p.dtype], int(kind), p.ptr, t.ptr, p.size, float(m_global),
+                               float(delta), loss.ptr, dp.ptr if want_dp else None):
+        _raise("tnn_pointwise_loss")
+    return loss, dp
+
+
+def pointwise_loss_bwd(p, t, kind, m_global, delta, g):
+    """dL/dp for the upstream gradient g (a scalar device array)"""
+    dp = empty(p.shape, p.dtype)
+    if g.dtype != p.dtype:
+        g = astype(g, p.dtype)
+    if _lib.tnn_pointwise_loss_bwd(_DT_CODE[p.dtype], int(kind), dp.ptr, p.ptr, t.ptr, p.size, float(m_global),
+                                   float(delta), g.ptr):
+        _raise("tnn_pointwise_loss_bwd")
+    return dp
 
 
 def ce_stats(z):

@@ -11,9 +11,18 @@ and the initial loss of an untrained classifier is about log(m * C), not log(C).
 (ops.softmax_ce_) computes this with three streaming passes forward and one backward; under data
 parallelism the max / sum pair is merged across ranks so the normaliser still spans the global
 batch.
+
+Four elementwise losses have no reference counterpart (new): MSELoss, MAELoss, HuberLoss and
+SigmoidCrossEntropyLoss.  Each is L = (1/m) sum over every element of l(p, t), m = the prediction's
+row count (of the global batch under data parallelism): the per-sample convention of
+MSEEvaluator / MAEEvaluator, sum over each row, mean over rows.  They run as one fused node
+(ops.pointwise_loss_): one launch for the loss and, with backward()'s default seed, its gradient.
 """
+import math
+
 import numpy as np
 
+import core._backend as be
 import core.ops as ops
 from core.tensor import Tensor, as_tensor
 
@@ -60,3 +69,96 @@ class SoftmaxCrossEntropyLoss(BaseLoss):
         picked = ops.sum_(ops.mul_(probs, as_tensor(labels)), axis=1)   # q_i = sum_j p_ij y_ij
         total = ops.sum_(ops.neg_(ops.log_(picked)), axis=None)
         return total / batch
+
+
+class _PointwiseLoss(BaseLoss):
+    """L = (1/m) sum_all l(predicted, actual), m = predicted.shape[0]; dL/dpredicted only.
+
+    Prediction and target have the same shape (any rank >= 1, no broadcasting) and the same dtype,
+    float32 or float64; the target must not require a gradient.  NaN and +-inf propagate as in numpy;
+    target values are not range-checked (that would need a read back to the host)."""
+
+    _kind = None
+    _delta = 1.0         # read by the Huber kind only
+
+    def _config(self):
+        """the fixed configuration a recorded step depends on beyond the class (Model._step_key)"""
+        return ()
+
+    def loss(self, predicted, actual):
+        self._check(predicted, actual)
+        if type(predicted) is not Tensor and isinstance(predicted, Tensor):
+            # a prediction Model.forward postponed (core/_deferred.py): the loss is postponed with it
+            import core._deferred as deferred
+            if type(predicted) is deferred.LazyTensor:
+                lazy = deferred.defer_loss(self, predicted, actual)
+                if lazy is not None:
+                    return lazy
+        return ops.pointwise_loss_(as_tensor(predicted), as_tensor(actual), self._kind, self._delta)
+
+    @staticmethod
+    def _describe(x):
+        """(shape, dtype on the device, requires_grad) without touching the device"""
+        if isinstance(x, np.ndarray) or not (hasattr(x, "shape") and hasattr(x, "dtype")):
+            arr = np.asarray(x)
+            try:
+                return arr.shape, be.device_dtype(arr.dtype), False
+            except TypeError as exc:
+                raise ValueError(str(exc))
+        return tuple(x.shape), np.dtype(x.dtype), bool(getattr(x, "requires_grad", False))
+
+    def _check(self, predicted, actual):
+        name = type(self).__name__
+        p_shape, p_dtype, _ = self._describe(predicted)
+        t_shape, t_dtype, t_grad = self._describe(actual)
+        if p_shape != t_shape:
+            raise ValueError("%s: prediction %s and target %s must have the same shape (no broadcasting)"
+                             % (name, p_shape, t_shape))
+        if len(p_shape) < 1:
+            raise ValueError("%s: the prediction needs at least one axis (the batch rows)" % name)
+        if p_shape[0] < 1:
+            raise ValueError("%s: the batch has no rows" % name)
+        if p_dtype not in (be.F32, be.F64) or t_dtype != p_dtype:
+            raise ValueError("%s: prediction (%s) and target (%s) must both be float32 or both float64"
+                             % (name, p_dtype, t_dtype))
+        if t_grad:
+            raise ValueError("%s: the target requires a gradient; the loss differentiates the "
+                             "prediction only" % name)
+
+
+class MSELoss(_PointwiseLoss):
+    """l = (p - t)^2; for a 2-D prediction L equals MSEEvaluator's "mse" (new)"""
+    _kind = be.LOSS_MSE
+
+
+class MAELoss(_PointwiseLoss):
+    """l = |p - t|, gradient sign(p - t) with 0 at p = t (new)"""
+    _kind = be.LOSS_MAE
+
+
+class HuberLoss(_PointwiseLoss):
+    """l = (p - t)^2 / 2 where |p - t| < delta, else delta * (|p - t| - delta / 2) (new).  delta is
+    fixed at construction: it is part of what a recorded training step computes."""
+    _kind = be.LOSS_HUBER
+
+    def __init__(self, delta=1.0):
+        if isinstance(delta, (bool, np.bool_)) or not isinstance(delta, (int, float, np.integer, np.floating)):
+            raise ValueError("HuberLoss: delta must be a number, got %r" % (delta,))
+        delta = float(delta)
+        if not (math.isfinite(delta) and delta > 0.0):
+            raise ValueError("HuberLoss: delta must be finite and > 0, got %r" % delta)
+        self._delta = delta
+
+    @property
+    def delta(self):
+        return self._delta
+
+    def _config(self):
+        return (self._delta,)
+
+
+class SigmoidCrossEntropyLoss(_PointwiseLoss):
+    """Binary cross-entropy of logits z against targets t in [0, 1] (soft targets allowed), one
+    independent sigmoid per element -- multi-label classification (new):
+    l = max(z, 0) - z t + log1p(exp(-|z|)), gradient sigmoid(z) - t."""
+    _kind = be.LOSS_SIGMOID_CE

@@ -299,9 +299,13 @@ class Model(object):
         # (loss objects of one class without state are interchangeable: run.py:72-73 builds two)
         # the layer list is part of the key: swapping an activation leaves every parameter where it
         # was, but a recording of the old network must not be replayed for the new one
-        return (kind, x.shape, x.dtype.str, y.shape, y.dtype.str, dist.world_size(), id(self.optimizer),
-                type(loss_obj), id(getattr(loss_obj, "_weight", None)), self._phase,
-                tuple((id(layer), type(layer)) for layer in self.net.layers))
+        key = (kind, x.shape, x.dtype.str, y.shape, y.dtype.str, dist.world_size(), id(self.optimizer),
+               type(loss_obj), id(getattr(loss_obj, "_weight", None)), self._phase,
+               tuple((id(layer), type(layer)) for layer in self.net.layers))
+        # a loss with a fixed configuration (HuberLoss's delta) is interchangeable only with one
+        # configured alike: a recording bakes the configuration into its kernels' arguments
+        config = getattr(loss_obj, "_config", None)
+        return key + (config(),) if config is not None else key
 
     def _step_generic(self):
         """the reference's three stages verbatim (model.py:45-61), on device arrays"""

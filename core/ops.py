@@ -7,7 +7,8 @@ A grad_fn receives the incoming gradient as a device array and returns a device 
 un-broadcast reduction the reference inlines twelve times (ops.py:41-46 ...) is one backend call.
 Three fused nodes are added for the training path (dense_, relu_, softmax_ce_); they are what
 core/layers.py and core/losses.py use.  Two more serve the NHWC image layers: im2col_ (Conv2D's
-window matrix) and maxpool2d_; batchnorm_ is BatchNormalization.
+window matrix) and maxpool2d_; batchnorm_ is BatchNormalization, and pointwise_loss_ the MSE, MAE,
+Huber and sigmoid cross-entropy losses.
 """
 import builtins as _bi
 
@@ -743,6 +744,33 @@ def softmax_ce_(ts_logits, ts_labels):
         return be.ce_bwd(z, y, stats, q, m_global, grad)
 
     return build_unary_ops_tensor(ts_logits, grad_fn, loss)
+
+
+def pointwise_loss_(ts_pred, ts_target, kind, delta=1.0):
+    """MSELoss / MAELoss / HuberLoss / SigmoidCrossEntropyLoss (core/losses.py) as one node:
+    L = (1/m) sum over every element of l(p, t), m = pred.shape[0] rows of the global batch, `kind` one
+    of be.LOSS_*.  The forward launch also writes dL/dp for backward()'s default seed, so the loss's
+    forward and backward together are one launch; any other upstream gradient takes a second one.
+    The gradient flows to the prediction only (the caller refuses a target that requires one).
+
+    Under data parallelism m is the global batch (equal shards, the cross-entropy's convention), so
+    1/m_global is inside dL/dp and Model.step's SUM all-reduce of the gradients completes them; the
+    returned loss is the all-reduced global value."""
+    import core._dist as dist
+    p, t = ts_pred._data, ts_target._data
+    world = dist.world_size()
+    m_global = p.shape[0] * world
+    loss, dp_seed1 = be.pointwise_loss(p, t, kind, m_global, delta,
+                                       want_dp=ts_pred.requires_grad and _GRAD_ENABLED)
+    if world > 1:
+        dist.allreduce_sum(loss)
+
+    def grad_fn(grad):
+        if dp_seed1 is not None and be.is_ones_scalar(grad):
+            return dp_seed1              # bit-identical to pointwise_loss_bwd with g = 1, no launch
+        return be.pointwise_loss_bwd(p, t, kind, m_global, delta, grad)
+
+    return build_unary_ops_tensor(ts_pred, grad_fn, loss)
 
 
 # ------------------------------------------------------------------------------ coercing wrappers

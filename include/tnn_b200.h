@@ -365,6 +365,30 @@ int tnn_bn_bwd_reduce(int dtype, const void* dy, const void* x, int64_t M, int64
 int tnn_bn_dx(int dtype, void* dx, const void* dy, const void* x, int64_t M, int64_t C, const double* mr,
               const void* gamma, const double* sums);
 
+/* ---- pointwise losses (new: no reference counterpart) ------------------------------------------
+ * MSELoss, MAELoss, HuberLoss and SigmoidCrossEntropyLoss in core/losses.py:
+ *   L = (1/m_global) * sum over the n elements of l(p, t),  e = p - t,  `kind`:
+ *   TNN_LOSS_MSE         l = e^2                                            dl/dp = 2e
+ *   TNN_LOSS_MAE         l = |e|                                            dl/dp = sign(e), 0 at e = 0
+ *   TNN_LOSS_HUBER       l = e^2/2 if |e| < delta, else delta(|e| - delta/2)   dl/dp = e, else delta sign(e)
+ *   TNN_LOSS_SIGMOID_CE  p are logits z, t targets in [0, 1]:
+ *                        l = max(z, 0) - z t + log1p(exp(-|z|))             dl/dz = sigmoid(z) - t
+ * p, t and dp are n contiguous values of `dtype` (TNN_F32 / TNN_F64); n may be 0.  m_global >= 1 is
+ * the row count of the global batch (data parallel: local rows * world).  delta (Huber only) is
+ * finite and > 0.  Terms, derivatives and sums are float64, each result rounded once to dtype; the
+ * sum is folded in a fixed order (no atomics on values, no host sync), so the bits do not change
+ * from run to run.
+ * tnn_pointwise_loss: loss_dev[0] = L, one launch.  dp (optional, else NULL) receives dL/dp for the
+ *   upstream gradient 1 (the seed of loss.backward()) in the same pass, bit-identical to
+ *   tnn_pointwise_loss_bwd with g = 1.
+ * tnn_pointwise_loss_bwd: dp = dl/dp * (g / m_global), g = g_dev[0] (dtype, on the device); the seeded
+ *   output is dl/dp * (1 / m_global). */
+enum { TNN_LOSS_MSE = 0, TNN_LOSS_MAE = 1, TNN_LOSS_HUBER = 2, TNN_LOSS_SIGMOID_CE = 3 };
+int tnn_pointwise_loss(int dtype, int kind, const void* p, const void* t, int64_t n, double m_global,
+                       double delta, void* loss_dev, void* dp);
+int tnn_pointwise_loss_bwd(int dtype, int kind, void* dp, const void* p, const void* t, int64_t n,
+                           double m_global, double delta, const void* g_dev);
+
 /* SoftmaxCrossEntropyLoss.loss (losses.py:24-32) with its batch-GLOBAL max and normaliser.
  * Stage 1: local max + local sum exp(z - local max) -> stats_dev[0..1] (device, dtype of z).
  * (data parallel: all-gather stats across ranks, merge on host or with tnn_ce_merge_stats)

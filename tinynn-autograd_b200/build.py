@@ -19,7 +19,7 @@ LIB = os.path.join(HERE, "libtnn_b200.so")
 
 SOURCES = ["runtime.cu", "elementwise.cu", "reduce.cu", "layout.cu", "gemm_simt.cu",
            "gemm_tc.cu", "gemm_f16.cu", "fused.cu", "mlp_fused.cu", "comm.cu", "conv.cu",
-           "batchnorm.cu"]
+           "batchnorm.cu", "loss.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "math.cuh"), os.path.join(CSRC, "tc_ptx.cuh"),
            os.path.join(ROOT, "include", "tnn_b200.h")]
 
@@ -29,7 +29,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-Xcompiler", "-fPIC", "-diag-suppress", "550", "-split-compile", "0"]
 # bit-faithful elementwise arithmetic (numpy does not contract a*b+c): no FMA contraction outside
 # the GEMMs
-NO_FMAD = {"elementwise.cu", "fused.cu", "reduce.cu"}
+NO_FMAD = {"elementwise.cu", "fused.cu", "reduce.cu", "loss.cu"}
 
 
 def _nvcc():
