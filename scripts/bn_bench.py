@@ -5,18 +5,15 @@ card's name and power limit (read in the same run).
 
 1. kernel bandwidth of the four passes of csrc/batchnorm.cu -- statistics (with the running update),
    apply, backward reduction, dx (TRAIN) -- on a 256 x 32 x 32 x 64 NHWC input (an (262144, 64)
-   problem) and on (8192, 4096), float32, timed with sweep_ops.timed_rotating (rotating buffer sets
+   problem) and on (8192, 4096), float32, timed with bench_common.timed_rotating (rotating buffer sets
    that together exceed twice the L2, recorded into one graph and replayed).  Algorithmic bytes: every
    (M, C) operand read once, every (M, C) output written once (the C-sized vectors are left out).
    The yardstick is a device-to-device copy of one (M, C) buffer measured the same way in the same run.
 2. the MNIST-sized CNN of tests/test_gpu_batchnorm.py at batch 128 through Model.train_step (recorded,
    replayed), ms per step, beside the same CNN without its two BatchNormalization layers, alternating
    the two models twice."""
-import json
 import os
-import subprocess
 import sys
-import time
 
 import numpy as np
 
@@ -26,21 +23,7 @@ sys.path.insert(0, os.path.join(ROOT, "scripts"))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 import core._backend as be  # noqa: E402
-from sweep_ops import timed_rotating  # noqa: E402
-
-CARD = {}
-
-
-def emit(**row):
-    row.update(CARD)
-    print(json.dumps(row), flush=True)
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    name, power, clock = [s.strip() for s in q.stdout.splitlines()[0].split(",")]
-    return dict(gpu=name, power_limit=power, max_sm_clock=clock)
+from bench_common import CARD, alternate, card, emit, timed_rotating  # noqa: E402
 
 
 def kernel_bandwidth(l2, M, C, label):
@@ -114,16 +97,9 @@ def mnist_cnn(steps=200, rounds=2):
 
     models = {"with_batchnorm": build(True), "without_batchnorm": build(False)}
     out = {k: [] for k in models}
-    for _ in range(rounds):
-        for name, model in models.items():
-            be.sync()
-            t0 = time.perf_counter()
-            for _ in range(steps):
-                model.train_step(xb, yb)
-            be.sync()
-            ms = (time.perf_counter() - t0) * 1e3 / steps
-            out[name].append(ms)
-            emit(section="mnist_cnn", model=name, mode="train_step", batch=B, ms_per_step=ms, steps=steps)
+    for name, ms in alternate(models, steps, rounds, lambda m: m.train_step(xb, yb)):
+        out[name].append(ms)
+        emit(section="mnist_cnn", model=name, mode="train_step", batch=B, ms_per_step=ms, steps=steps)
     emit(section="mnist_cnn", ms_with_batchnorm=min(out["with_batchnorm"]),
          ms_without_batchnorm=min(out["without_batchnorm"]),
          added_ms=min(out["with_batchnorm"]) - min(out["without_batchnorm"]))

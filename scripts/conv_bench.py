@@ -3,7 +3,7 @@
     python scripts/conv_bench.py > profiles/<run>_conv_bench.jsonl
 
 1. kernel bandwidth of the four passes of csrc/conv.cu on a 256 x 32 x 32 x 64 float32 input (3 x 3
-   SAME im2col / col2im: a 604 MB col buffer; 2 x 2 / s2 pooling), timed with sweep_ops.timed_rotating
+   SAME im2col / col2im: a 604 MB col buffer; 2 x 2 / s2 pooling), timed with bench_common.timed_rotating
    (rotating buffer sets that together exceed twice the L2, recorded into one graph).  Algorithmic
    bytes: every input read once, every output written once.  The copy bandwidth they are compared
    with is a device-to-device copy of the col buffer measured the same way in the same run.
@@ -13,11 +13,8 @@
 3. the small MNIST CNN of tests/test_gpu_conv.py at batch 128: Model.train_step (recorded, replayed)
    against the five eager lines, ms per step and samples/s.
 The card's name and power limit are read in the same run (first line)."""
-import json
 import os
-import subprocess
 import sys
-import time
 
 import numpy as np
 
@@ -26,19 +23,8 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
 
 import core._backend as be  # noqa: E402
+from bench_common import alternate, card, emit, timed_rotating  # noqa: E402
 from core.layers import window_geometry  # noqa: E402
-from sweep_ops import timed_rotating  # noqa: E402
-
-
-def emit(**row):
-    print(json.dumps(row), flush=True)
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    name, power, clock = [s.strip() for s in q.stdout.splitlines()[0].split(",")]
-    return dict(gpu=name, power_limit=power, max_sm_clock=clock)
 
 
 def kernel_bandwidth(l2):
@@ -155,31 +141,26 @@ def mnist_cnn(steps=200):
     B = 128
     x, _, onehot = ref_fp32.learnable_mnist(B, seed=0)
     xb, yb = Tensor(x.reshape(B, 28, 28, 1)), Tensor(onehot)
-    out = {}
-    for mode in ("train_step", "eager"):
+
+    def eager(model):
+        model.zero_grad()
+        loss = model.loss.loss(model.forward(xb), yb)
+        loss.backward()
+        model.step()
+
+    def build(step):
         np.random.seed(0)
         net = Net([Conv2D((5, 5, 1, 8), stride=2), ReLU(), MaxPool2D(), Conv2D((3, 3, 8, 16)), ReLU(), Flatten(),
                    Dense(10, num_in=784)])
         model = Model(net=net, loss=SoftmaxCrossEntropyLoss(), optimizer=Adam(lr=1e-3))
         model.defer_loop = False
-
-        def step():
-            if mode == "train_step":
-                return model.train_step(xb, yb)
-            model.zero_grad()
-            loss = model.loss.loss(model.forward(xb), yb)
-            loss.backward()
-            model.step()
-            return loss
-
         for _ in range(10):
-            step()
-        be.sync()
-        t0 = time.perf_counter()
-        for _ in range(steps):
-            step()
-        be.sync()
-        ms = (time.perf_counter() - t0) * 1e3 / steps
+            step(model)
+        return lambda: step(model)
+
+    runs = {"train_step": build(lambda m: m.train_step(xb, yb)), "eager": build(eager)}
+    out = {}
+    for mode, ms in alternate(runs, steps, 1, lambda run: run()):
         out[mode] = ms
         emit(section="mnist_cnn", mode=mode, batch=B, ms_per_step=ms, samples_per_s=B / (ms * 1e-3),
              steps=steps)

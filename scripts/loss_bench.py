@@ -4,18 +4,15 @@ and power limit (read in the same run).
     python scripts/loss_bench.py > profiles/loss_bench_b200.jsonl
 
 1. the fused pass of csrc/loss.cu -- the loss and the seeded dL/dp in one launch, float32 -- for each
-   loss on 2^24 and 2^26 elements, timed with sweep_ops.timed_rotating (rotating buffer sets that
+   loss on 2^24 and 2^26 elements, timed with bench_common.timed_rotating (rotating buffer sets that
    together exceed twice the L2, recorded into one graph and replayed).  Algorithmic bytes: p and t
    read once, dp written once (12 bytes an element).  The yardstick is a device-to-device copy of p
    (8 bytes an element) measured the same way in the same run.
 2. a regression MLP step through Model.train_step (recorded, replayed) with the fused MSELoss beside
    the same loss composed from ops (sub_, mul_, sum_, / m), alternating the two models twice: ms per
    step, and the kernels one eager step launches."""
-import json
 import os
-import subprocess
 import sys
-import time
 
 import numpy as np
 
@@ -24,22 +21,9 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
 
 import core._backend as be  # noqa: E402
-from sweep_ops import timed_rotating  # noqa: E402
+from bench_common import CARD, alternate, card, emit, timed_rotating  # noqa: E402
 
-CARD = {}
 KINDS = (("mse", be.LOSS_MSE), ("mae", be.LOSS_MAE), ("huber", be.LOSS_HUBER), ("sigmoid_ce", be.LOSS_SIGMOID_CE))
-
-
-def emit(**row):
-    row.update(CARD)
-    print(json.dumps(row), flush=True)
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    name, power, clock = [s.strip() for s in q.stdout.splitlines()[0].split(",")]
-    return dict(gpu=name, power_limit=power, max_sm_clock=clock)
 
 
 def kernel_bandwidth(l2, log2n):
@@ -111,17 +95,10 @@ def regression_mlp(steps=200, rounds=2):
 
     models = {"fused_mse": build(MSELoss()), "composed_mse": build(ComposedMSE())}
     out = {k: [] for k in models}
-    for _ in range(rounds):
-        for name, (model, launches) in models.items():
-            be.sync()
-            t0 = time.perf_counter()
-            for _ in range(steps):
-                model.train_step(xb, yb)
-            be.sync()
-            ms = (time.perf_counter() - t0) * 1e3 / steps
-            out[name].append(ms)
-            emit(section="regression_mlp", loss=name, mode="train_step", batch=B, dims=list(dims), ms_per_step=ms,
-                 launches_per_eager_step=launches, steps=steps)
+    for name, ms in alternate(models, steps, rounds, lambda m: m[0].train_step(xb, yb)):
+        out[name].append(ms)
+        emit(section="regression_mlp", loss=name, mode="train_step", batch=B, dims=list(dims), ms_per_step=ms,
+             launches_per_eager_step=models[name][1], steps=steps)
     emit(section="regression_mlp", ms_fused=min(out["fused_mse"]), ms_composed=min(out["composed_mse"]),
          launches_fused=models["fused_mse"][1], launches_composed=models["composed_mse"][1])
 

@@ -25,28 +25,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 import core._backend as be  # noqa: E402
-
-
-def timed_rotating(make_launch, n_sets, reps=5):
-    """make_launch(k) issues the op on buffer set k; returns ms per launch"""
-    for k in range(n_sets):           # eager warm-up (scratch growth, lazily allocated counters)
-        make_launch(k)
-    be.sync()
-    g = be.StepGraph()
-    with g.capture():
-        for k in range(n_sets):
-            make_launch(k)
-    g.replay()
-    be.sync()
-    best = 1e30
-    e0, e1 = be.Event(), be.Event()
-    for _ in range(reps):
-        e0.record()
-        g.replay()
-        e1.record()
-        best = min(best, e1.elapsed_ms_since(e0))
-    g.destroy()
-    return best / n_sets
+from bench_common import timed_rotating  # noqa: E402
 
 
 def main():

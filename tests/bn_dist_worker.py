@@ -4,26 +4,19 @@ statistics are those of the GLOBAL batch (losses, parameters and running statist
 single-process oracle on the full batch), that replicas hold bit-identical parameters and running
 statistics, and that the recorded step (the all-gather and all-reduces inside the graph) gives the
 eager loop's bits."""
-import os
-import sys
-
 import numpy as np
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "oracle"))
-
-import core._backend as be  # noqa: E402
-import core._dist as dist  # noqa: E402
-import ref_bn as RB  # noqa: E402
-import ref_conv as RC  # noqa: E402
-import ref_numpy as R  # noqa: E402
-from core.layers import BatchNormalization, Conv2D, Dense, Flatten, ReLU  # noqa: E402
-from core.losses import SoftmaxCrossEntropyLoss  # noqa: E402
-from core.model import Model  # noqa: E402
-from core.nn import Net  # noqa: E402
-from core.optimizer import SGD  # noqa: E402
-from core.tensor import Tensor  # noqa: E402
+from dist_common import assert_replay_matches, eager_steps, same_on_every_rank, state  # sets sys.path
+import core._dist as dist
+import ref_bn as RB
+import ref_conv as RC
+import ref_numpy as R
+from core.layers import BatchNormalization, Conv2D, Dense, Flatten, ReLU
+from core.losses import SoftmaxCrossEntropyLoss
+from core.model import Model
+from core.nn import Net
+from core.optimizer import SGD
+from core.tensor import Tensor
 
 B, H, W, CIN, C, K = 10, 6, 5, 2, 4, 3     # 10 images: shards of 5 per rank
 
@@ -33,18 +26,6 @@ def _model(seed):
     net = Net([Conv2D((3, 3, CIN, C)), BatchNormalization(C, momentum=0.2), ReLU(), Flatten(),
                Dense(K, num_in=H * W * C)])
     return net, Model(net=net, loss=SoftmaxCrossEntropyLoss(), optimizer=SGD(lr=0.3))
-
-
-def _state(net):
-    vals = [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-    return vals + [b.values.copy() for layer in net.layers for b in layer.buffers.values()]
-
-
-def _same_on_every_rank(arrays, world):
-    flat = np.concatenate([a.ravel() for a in arrays]).astype(np.float64)
-    mine = be.from_numpy(flat)
-    dist.allreduce_sum(mine)
-    return np.array_equal(mine.numpy(), flat * world)
 
 
 def main():
@@ -57,16 +38,10 @@ def main():
     xs, ys = Tensor(x[lo:hi]), Tensor(labels[lo:hi])
 
     net, model = _model(0)
-    start = _state(net)
-    eager = []
-    for _ in range(4):
-        model.zero_grad()
-        loss = model.loss.loss(model.forward(xs), ys)
-        loss.backward()
-        model.step()
-        eager.append(float(loss.values))
-    final = _state(net)
-    assert _same_on_every_rank(final, world), "replicas diverged"
+    start = state(net)
+    eager = eager_steps(model, xs, ys, 4)
+    final = state(net)
+    assert same_on_every_rank(final, world), "replicas diverged"
 
     # the single-process oracle on the full batch
     p = [R.RefTensor(v, True) for v in start[:6]]
@@ -95,12 +70,7 @@ def main():
         print("BN_DIST_EAGER_OK world=%d losses=%s" % (world, eager))
 
     # the recorded step, collectives inside the graph, gives the eager bits
-    net_g, model_g = _model(0)
-    replayed = [float(model_g.train_step(xs, ys).values) for _ in range(4)]
-    assert any(hasattr(v, "graph") for v in model_g._captured.values()), "step was not recorded"
-    assert replayed == eager, (replayed, eager)
-    for a, b in zip(_state(net_g), final):
-        assert np.array_equal(a, b)
+    assert_replay_matches(lambda: _model(0), xs, ys, eager, final)
     if rank == 0:
         print("BN_DIST_OK world=%d" % world)
     dist.destroy_process_group()

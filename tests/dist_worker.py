@@ -1,24 +1,17 @@
 """Worker for tests/test_gpu_dist.py (launched by torch.distributed.run, one rank per GPU):
 trains a small MLP data-parallel through the public API and checks, on rank 0, that losses and
 parameters equal the single-process oracle on the FULL batch (SURVEY 8e)."""
-import os
-import sys
-
 import numpy as np
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "oracle"))
-
-import core._backend as be  # noqa: E402
-import core._dist as dist  # noqa: E402
-import ref_numpy as R  # noqa: E402
-from core.layers import Dense, ReLU  # noqa: E402
-from core.losses import SoftmaxCrossEntropyLoss  # noqa: E402
-from core.model import Model  # noqa: E402
-from core.nn import Net  # noqa: E402
-from core.optimizer import SGD  # noqa: E402
-from core.tensor import Tensor  # noqa: E402
+from dist_common import assert_replay_matches, eager_steps, same_on_every_rank, state  # sets sys.path
+import core._dist as dist
+import ref_numpy as R
+from core.layers import Dense, ReLU
+from core.losses import SoftmaxCrossEntropyLoss
+from core.model import Model
+from core.nn import Net
+from core.optimizer import SGD
+from core.tensor import Tensor
 
 
 def main():
@@ -33,21 +26,11 @@ def main():
     np.random.seed(0)
     net = Net([Dense(24), ReLU(), Dense(C)])
     model = Model(net=net, loss=SoftmaxCrossEntropyLoss(), optimizer=SGD(lr=0.5))
-    loss_layer = SoftmaxCrossEntropyLoss()
-    losses = []
-    for _ in range(4):
-        model.zero_grad()
-        loss = loss_layer.loss(model.forward(Tensor(x[lo:hi])), Tensor(labels[lo:hi]))
-        loss.backward()
-        model.step()
-        losses.append(float(loss.values))
-    params = [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
+    xs, ys = Tensor(x[lo:hi]), Tensor(labels[lo:hi])
+    losses = eager_steps(model, xs, ys, 4)
+    params = state(net)
     # every rank must hold bit-identical parameters after the all-reduced update
-    flat = np.concatenate([p.ravel() for p in params]).astype(np.float32)
-    mine = be.from_numpy(flat)
-    dist.allreduce_sum(mine)
-    assert np.array_equal(mine.numpy(), flat * world), "replicas diverged"
+    assert same_on_every_rank(params, world), "replicas diverged"
 
     if rank == 0:
         np.random.seed(0)
@@ -65,22 +48,9 @@ def main():
         n = Net([Dense(24, num_in=D), ReLU(), Dense(C, num_in=24)])
         return n, Model(net=n, loss=SoftmaxCrossEntropyLoss(), optimizer=SGD(lr=0.5))
 
-    xs, ys = Tensor(x[lo:hi]), Tensor(labels[lo:hi])
     net_e, model_e = fresh()
-    eager = []
-    for _ in range(6):
-        model_e.zero_grad()
-        loss = model_e.loss.loss(model_e.forward(xs), ys)
-        loss.backward()
-        model_e.step()
-        eager.append(float(loss.values))
-    net_g, model_g = fresh()
-    replayed = [float(model_g.train_step(xs, ys).values) for _ in range(6)]
-    assert any(hasattr(v, "graph") for v in model_g._captured.values()), "step was not captured"
-    assert eager == replayed, (eager, replayed)
-    for pe, pg in zip(net_e.get_parameters(), net_g.get_parameters()):
-        for k in pe:
-            assert np.array_equal(pe[k].values, pg[k].values)
+    eager = eager_steps(model_e, xs, ys, 6)
+    assert_replay_matches(fresh, xs, ys, eager, state(net_e))
     if rank == 0:
         print("GRAPH_DIST_OK world=%d" % world)
 
@@ -93,14 +63,7 @@ def main():
         np.random.seed(2)
         n = Net([Dense(24, num_in=D), ReLU(), Dense(C, num_in=24)])
         m = Model(net=n, loss=SoftmaxCrossEntropyLoss(), optimizer=Adam(lr=1e-2))
-        ls = []
-        for _ in range(5):
-            m.zero_grad()
-            loss = m.loss.loss(m.forward(xs), ys)
-            loss.backward()
-            m.step()
-            ls.append(float(loss.values))
-        results.append((ls, [p.values.copy() for layer in n.get_parameters() for p in layer.values()]))
+        results.append((eager_steps(m, xs, ys, 5), state(n)))
     dist.MIN_CHUNK_ELEMS, dist.ALLREDUCE_CHUNKS = 1 << 20, 1
     assert results[0][0] == results[1][0], (results[0][0], results[1][0])
     for a, b in zip(results[0][1], results[1][1]):

@@ -4,25 +4,18 @@ SigmoidCrossEntropyLoss.  Checks that 1/m covers the GLOBAL batch (losses and pa
 single-process oracle on the full batch), that replicas hold bit-identical parameters, and that the
 recorded step (the loss all-reduce and the gradient all-reduce inside the graph) gives the eager
 loop's bits."""
-import os
-import sys
-
 import numpy as np
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "oracle"))
-
-import core._backend as be  # noqa: E402
-import core._dist as dist  # noqa: E402
-import ref_losses as RL  # noqa: E402
-import ref_numpy as R  # noqa: E402
-from core.layers import Dense, ReLU  # noqa: E402
-from core.losses import MSELoss, SigmoidCrossEntropyLoss  # noqa: E402
-from core.model import Model  # noqa: E402
-from core.nn import Net  # noqa: E402
-from core.optimizer import SGD  # noqa: E402
-from core.tensor import Tensor  # noqa: E402
+from dist_common import assert_replay_matches, eager_steps, same_on_every_rank, state  # sets sys.path
+import core._dist as dist
+import ref_losses as RL
+import ref_numpy as R
+from core.layers import Dense, ReLU
+from core.losses import MSELoss, SigmoidCrossEntropyLoss
+from core.model import Model
+from core.nn import Net
+from core.optimizer import SGD
+from core.tensor import Tensor
 
 B, DIN, DH, DOUT = 16, 6, 12, 3     # 16 rows: shards of 8 per rank
 
@@ -33,32 +26,15 @@ def _model(seed, loss):
     return net, Model(net=net, loss=loss, optimizer=SGD(lr=0.2))
 
 
-def _state(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
-
-def _same_on_every_rank(arrays, world):
-    flat = np.concatenate([a.ravel() for a in arrays]).astype(np.float64)
-    mine = be.from_numpy(flat)
-    dist.allreduce_sum(mine)
-    return np.array_equal(mine.numpy(), flat * world)
-
-
 def check(kind, loss_cls, x, y, rank, world):
     lo, hi = dist.shard_bounds(B, rank, world)
     xs, ys = Tensor(x[lo:hi]), Tensor(y[lo:hi])
     net, model = _model(0, loss_cls())
-    start = _state(net)
-    eager = []
-    for _ in range(4):
-        model.zero_grad()
-        loss = model.loss.loss(model.forward(xs), ys)
-        loss.backward()
-        model.step()
-        eager.append(float(loss.values))
-    final = _state(net)
-    assert _same_on_every_rank(final, world), "replicas diverged"
-    assert _same_on_every_rank([np.array(eager)], world), "ranks report different losses"
+    start = state(net)
+    eager = eager_steps(model, xs, ys, 4)
+    final = state(net)
+    assert same_on_every_rank(final, world), "replicas diverged"
+    assert same_on_every_rank([np.array(eager)], world), "ranks report different losses"
 
     # the single-process oracle on the full batch
     p = [R.RefTensor(v, True) for v in start]
@@ -80,12 +56,7 @@ def check(kind, loss_cls, x, y, rank, world):
         assert err <= 1e-5, err
 
     # the recorded step, collectives inside the graph, gives the eager bits
-    net_g, model_g = _model(0, loss_cls())
-    replayed = [float(model_g.train_step(xs, ys).values) for _ in range(4)]
-    assert any(hasattr(v, "graph") for v in model_g._captured.values()), "step was not recorded"
-    assert replayed == eager, (replayed, eager)
-    for a, b in zip(_state(net_g), final):
-        assert np.array_equal(a, b)
+    assert_replay_matches(lambda: _model(0, loss_cls()), xs, ys, eager, final)
     if rank == 0:
         print("LOSS_DIST_%s_OK world=%d losses=%s" % (kind.upper(), world, eager))
 

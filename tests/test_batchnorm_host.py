@@ -3,16 +3,13 @@ torch.nn.functional.batch_norm on the CPU, the layer's argument checks, the data
 the statistics (two ranks over gloo with oracle compute, equal to the full-batch maths) and the
 checkpoint layout.  torch is test infrastructure here; nothing on the product path imports it."""
 import os
-import socket
-import sys
 
 import numpy as np
 import pytest
 
 import ref_bn as RB
 import ref_numpy as R
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from support import spawn_gloo
 
 
 def _close(a, b, tol=1e-12):
@@ -111,14 +108,6 @@ def test_checkpoint_layout_holds_buffers(tmp_path):
 
 
 # ---------------------------------------------------------------------------- data parallel scheme
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
-
-
 def _problem():
     rng = np.random.RandomState(0)
     x = rng.standard_normal((9, 3, 2, 5)) * 2.0 + 40.0
@@ -128,60 +117,40 @@ def _problem():
     return x, g, gamma, beta
 
 
-def _dp_worker(rank, world, port, queue):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
-    for p in (ROOT, os.path.join(ROOT, "oracle")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
+def _dp_worker(rank, world):
     import torch
     import torch.distributed as td
     import core._dist as dist
-    import ref_bn as RB
-    import ref_numpy as R
-    td.init_process_group("gloo", init_method="env://")
-    try:
-        x, g, gamma, beta = _problem()
-        lo, hi = dist.shard_bounds(x.shape[0], rank, world)      # 9 images: shards of 5 and 4
-        xs, gs = x[lo:hi], g[lo:hi]
-        C = x.shape[-1]
-        # forward: gather every rank's (count, mean, M2), merge in rank order
-        n, mean, m2 = RB.local_stats(xs.reshape(-1, C))
-        mine = torch.tensor(np.concatenate([[n], mean, m2]))
-        gathered = [torch.zeros(1 + 2 * C, dtype=torch.float64) for _ in range(world)]
-        td.all_gather(gathered, mine)
-        parts = [(float(t[0]), t[1:1 + C].numpy(), t[1 + C:].numpy()) for t in gathered]
-        stats = dist.merge_bn_stats_host(parts)
-        state = RB.RefBNState(C, momentum=0.2)
-        rx, rg, rb = R.RefTensor(xs, True), R.RefTensor(gamma, True), R.RefTensor(beta, True)
-        y = RB.batchnorm(rx, rg, rb, state, True, stats=stats)
+    x, g, gamma, beta = _problem()
+    lo, hi = dist.shard_bounds(x.shape[0], rank, world)      # 9 images: shards of 5 and 4
+    xs, gs = x[lo:hi], g[lo:hi]
+    C = x.shape[-1]
+    # forward: gather every rank's (count, mean, M2), merge in rank order
+    n, mean, m2 = RB.local_stats(xs.reshape(-1, C))
+    mine = torch.tensor(np.concatenate([[n], mean, m2]))
+    gathered = [torch.zeros(1 + 2 * C, dtype=torch.float64) for _ in range(world)]
+    td.all_gather(gathered, mine)
+    parts = [(float(t[0]), t[1:1 + C].numpy(), t[1 + C:].numpy()) for t in gathered]
+    stats = dist.merge_bn_stats_host(parts)
+    state = RB.RefBNState(C, momentum=0.2)
+    rx, rg, rb = R.RefTensor(xs, True), R.RefTensor(gamma, True), R.RefTensor(beta, True)
+    y = RB.batchnorm(rx, rg, rb, state, True, stats=stats)
 
-        # backward: SUM all-reduce of the two per-column sums before dx; local dgamma / dbeta
-        def global_sums(dy):
-            s = torch.tensor(np.concatenate(y.bn_local_sums(dy)))
-            td.all_reduce(s)
-            return s[:C].numpy(), s[C:].numpy()
+    # backward: SUM all-reduce of the two per-column sums before dx; local dgamma / dbeta
+    def global_sums(dy):
+        s = torch.tensor(np.concatenate(y.bn_local_sums(dy)))
+        td.all_reduce(s)
+        return s[:C].numpy(), s[C:].numpy()
 
-        y.bn_vjp_x.sums = global_sums
-        y.backward(gs)
-        flat = torch.tensor(np.concatenate([rg.grad.ravel(), rb.grad.ravel()]))
-        td.all_reduce(flat)       # the gradient arena's all-reduce completes the local partials
-        queue.put((rank, y.values, rx.grad, flat.numpy().copy(), state.running_mean, state.running_var))
-    finally:
-        td.destroy_process_group()
+    y.bn_vjp_x.sums = global_sums
+    y.backward(gs)
+    flat = torch.tensor(np.concatenate([rg.grad.ravel(), rb.grad.ravel()]))
+    td.all_reduce(flat)       # the gradient arena's all-reduce completes the local partials
+    return y.values, rx.grad, flat.numpy().copy(), state.running_mean, state.running_var
 
 
 def test_sharded_statistics_equal_full_batch():
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_dp_worker, args=(r, 2, port, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    got = dict((r[0], r[1:]) for r in (q.get(timeout=120), q.get(timeout=120)))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    got = spawn_gloo(_dp_worker)
     x, g, gamma, beta = _problem()
     state = RB.RefBNState(5, momentum=0.2)
     rx, rg, rb = R.RefTensor(x, True), R.RefTensor(gamma, True), R.RefTensor(beta, True)

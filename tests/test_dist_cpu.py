@@ -3,82 +3,48 @@ the cross-entropy's (max, sum-exp) pair is exchanged and merged exactly as core/
 tnn_ce_merge_stats do, per-rank gradients are SUM-all-reduced -- and the result must equal the
 single-process reference maths on the full batch (SURVEY 8e).  The per-rank compute is the numpy
 oracle here (no GPU in this container); the N>1 GPU path runs the same host logic over NCCL."""
-import os
-import socket
-import sys
-
 import numpy as np
-import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
+import ref_numpy as R
+from support import spawn_gloo
 
 
-def _worker(rank, world, port, queue):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
-    for p in (ROOT, os.path.join(ROOT, "oracle")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
+def _worker(rank, world):
     import torch
     import torch.distributed as td
     import core._dist as dist
-    import ref_numpy as R
-    td.init_process_group("gloo", init_method="env://")
-    try:
-        rng = np.random.RandomState(0)
-        B, D, C = 48, 20, 12
-        x = rng.rand(B, D)
-        labels = np.eye(C)[rng.randint(0, C, B)]
-        w = rng.standard_normal((D, C)) * 0.3
-        b = rng.standard_normal((1, C)) * 0.1
-        lo, hi = dist.shard_bounds(B, rank, world)
-        xs, ys = x[lo:hi], labels[lo:hi]
-        # local forward up to the logits
-        W, Bv = R.RefTensor(w, True), R.RefTensor(b, True)
-        z = R.matmul(R.lift(xs), W) + Bv
-        # stage 1: local stats, all-gather, merge
-        m_r = z.values.max()
-        s_r = np.exp(z.values - m_r).sum()
-        gathered = [torch.zeros(2, dtype=torch.float64) for _ in range(world)]
-        td.all_gather(gathered, torch.tensor([m_r, s_r], dtype=torch.float64))
-        M, S = dist.merge_stats_host([g.numpy() for g in gathered])
-        # stage 2: local loss share and dz with the GLOBAL normaliser and batch size
-        e = np.exp(z.values - M)
-        p = e / S
-        q = (p * ys).sum(1)
-        loss_part = torch.tensor([-(np.log(q)).sum() / B], dtype=torch.float64)
-        dz = p - ys * p / (B * q[:, None])
-        z.backward(dz)
-        flat = torch.from_numpy(np.concatenate([W.grad.ravel(), Bv.grad.ravel()]))
-        td.all_reduce(flat)            # SUM, not mean
-        td.all_reduce(loss_part)
-        if rank == 0:
-            queue.put((float(loss_part[0]), flat.numpy().copy()))
-    finally:
-        td.destroy_process_group()
+    rng = np.random.RandomState(0)
+    B, D, C = 48, 20, 12
+    x = rng.rand(B, D)
+    labels = np.eye(C)[rng.randint(0, C, B)]
+    w = rng.standard_normal((D, C)) * 0.3
+    b = rng.standard_normal((1, C)) * 0.1
+    lo, hi = dist.shard_bounds(B, rank, world)
+    xs, ys = x[lo:hi], labels[lo:hi]
+    # local forward up to the logits
+    W, Bv = R.RefTensor(w, True), R.RefTensor(b, True)
+    z = R.matmul(R.lift(xs), W) + Bv
+    # stage 1: local stats, all-gather, merge
+    m_r = z.values.max()
+    s_r = np.exp(z.values - m_r).sum()
+    gathered = [torch.zeros(2, dtype=torch.float64) for _ in range(world)]
+    td.all_gather(gathered, torch.tensor([m_r, s_r], dtype=torch.float64))
+    M, S = dist.merge_stats_host([g.numpy() for g in gathered])
+    # stage 2: local loss share and dz with the GLOBAL normaliser and batch size
+    e = np.exp(z.values - M)
+    p = e / S
+    q = (p * ys).sum(1)
+    loss_part = torch.tensor([-(np.log(q)).sum() / B], dtype=torch.float64)
+    dz = p - ys * p / (B * q[:, None])
+    z.backward(dz)
+    flat = torch.from_numpy(np.concatenate([W.grad.ravel(), Bv.grad.ravel()]))
+    td.all_reduce(flat)            # SUM, not mean
+    td.all_reduce(loss_part)
+    return float(loss_part[0]), flat.numpy().copy()
 
 
 def test_sharded_ce_and_grad_allreduce_equals_full_batch():
-    import torch.multiprocessing as mp
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import ref_numpy as R
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    loss_dp, flat_dp = q.get(timeout=120)
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    loss_dp, flat_dp = spawn_gloo(_worker)[0]
     # single-process reference maths on the full batch
     rng = np.random.RandomState(0)
     B, D, C = 48, 20, 12

@@ -4,11 +4,7 @@ counts (up to many split CTAs), layouts, phases and dtypes; offset data, a const
 empty TEST batch, reproducibility, accumulation into an arena slot; and a small CNN with two
 BatchNormalization layers trained eagerly, through the recorded train_step and the recorded
 five-line loop, predicted in the TEST phase and checkpointed."""
-import ctypes
 import os
-import socket
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -17,9 +13,9 @@ import ref_bn as RB
 import ref_conv as RC
 import ref_fp32
 import ref_numpy as R
+from support import gpu_count, params, run_two_ranks
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
@@ -204,10 +200,6 @@ def _data(n):
     return x.reshape(n, 28, 28, 1), onehot
 
 
-def _params(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
-
 def _buffers(net):
     return [b.values.copy() for layer in net.layers for b in layer.buffers.values()]
 
@@ -217,7 +209,7 @@ class _RefCNN(object):
     running statistics"""
 
     def __init__(self, net):
-        self.p = [R.RefTensor(v, True) for v in _params(net)]
+        self.p = [R.RefTensor(v, True) for v in params(net)]
         bufs = _buffers(net)
         self.st = [RB.RefBNState(8, running_mean=bufs[0], running_var=bufs[1]),
                    RB.RefBNState(16, running_mean=bufs[2], running_var=bufs[3])]
@@ -313,7 +305,7 @@ def test_cnn_train_step_replay_is_bit_identical(be):
         for ba, bb in zip(_buffers(net_a), _buffers(net_b)):
             assert np.array_equal(ba, bb)
     assert len([s for s in model_b._captured.values() if hasattr(s, "graph")]) == 2
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
     # TRAIN and TEST recordings are kept apart
     keys = [k for k in model_b._captured]
@@ -341,7 +333,7 @@ def test_cnn_five_line_loop_recording_is_bit_identical(be):
         out.append(losses)
     assert out[0] == out[1]
     assert [s for s in model_b._captured.values() if hasattr(s, "graph")]
-    for pa, pb in zip(_params(net_a) + _buffers(net_a), _params(net_b) + _buffers(net_b)):
+    for pa, pb in zip(params(net_a) + _buffers(net_a), params(net_b) + _buffers(net_b)):
         assert np.array_equal(pa, pb)
 
 
@@ -382,46 +374,29 @@ def test_cnn_checkpoint_round_trip_and_replay_from_loaded_statistics(be, tmp_pat
     with open(path, "rb") as f:
         state = pickle.load(f)
     assert list(state[1]) == ["gamma", "beta", "running_mean", "running_var"]
-    saved = _params(net_a) + _buffers(net_a)
+    saved = params(net_a) + _buffers(net_a)
     for xb, yb in batches[3:6]:
         model_a.train_step(xb, yb)
     bufs = [b._data for layer in net_a.layers for b in layer.buffers.values()]
     model_a.load(path)
     assert [b._data for layer in net_a.layers for b in layer.buffers.values()] == bufs   # in place
-    for a, b in zip(_params(net_a) + _buffers(net_a), saved):
+    for a, b in zip(params(net_a) + _buffers(net_a), saved):
         assert np.array_equal(a, b)
     net_b, model_b = _cnn(7, SGD(lr=0.05))
     model_b.load(path)
-    for a, b in zip(_params(net_b) + _buffers(net_b), saved):
+    for a, b in zip(params(net_b) + _buffers(net_b), saved):
         assert np.array_equal(a, b)
     for xb, yb in batches[6:]:
         la = float(model_a.train_step(xb, yb).values)
         lb = float(_eager(model_b, xb, yb).values)
         assert la == lb
     assert [s for s in model_a._captured.values() if hasattr(s, "graph")]
-    for a, b in zip(_params(net_a) + _buffers(net_a), _params(net_b) + _buffers(net_b)):
+    for a, b in zip(params(net_a) + _buffers(net_a), params(net_b) + _buffers(net_b)):
         assert np.array_equal(a, b)
 
 
 # ---------------------------------------------------------------------------- two ranks
-def _gpu_count():
-    import core._backend as be
-    n = ctypes.c_int(0)
-    if be.load_library().tnn_device_count(ctypes.byref(n)):
-        return 0
-    return n.value
-
-
 def test_two_rank_batchnorm_equals_full_batch_oracle():
-    if _gpu_count() < 2:
+    if gpu_count() < 2:
         pytest.skip("needs 2 GPUs")
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", str(port),
-           os.path.join(ROOT, "tests", "bn_dist_worker.py")]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=200, cwd=ROOT)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    assert "BN_DIST_OK world=2" in r.stdout
+    assert "BN_DIST_OK world=2" in run_two_ranks("bn_dist_worker.py", timeout=200)

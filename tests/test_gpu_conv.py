@@ -12,6 +12,7 @@ import op_cases
 import ref_conv as RC
 import ref_fp32
 import ref_numpy as R
+from support import params
 
 pytestmark = pytest.mark.gpu
 
@@ -217,15 +218,11 @@ def _data(n):
     return x.reshape(n, 28, 28, 1), onehot
 
 
-def _params(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
-
 class _RefCNN(object):
     """the same network in the float64 oracle, starting from the engine model's parameters"""
 
     def __init__(self, net):
-        vals = _params(net)
+        vals = params(net)
         self.p = [R.RefTensor(v, True) for v in vals]
         self.opt = R.RefAdam(lr=1e-3)
 
@@ -311,7 +308,7 @@ def test_cnn_train_step_replay_is_bit_identical(be):
     states = [s for s in model_b._captured.values() if hasattr(s, "graph")]
     assert len(states) == 2
     assert model_b._fused_mlp_plan(Tensor(x[:128]), Tensor(y[:128])) is None
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
 
 
@@ -340,7 +337,7 @@ def test_cnn_five_line_loop_recording_is_bit_identical(be):
     assert out[0] == out[1]
     assert [s for s in model_b._captured.values() if hasattr(s, "graph")]
     assert not [s for s in model_a._captured.values() if hasattr(s, "graph")]
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
 
 
@@ -357,9 +354,9 @@ def test_cnn_predict_and_checkpoint(be, tmp_path):
     path = os.path.join(str(tmp_path), "cnn.pkl")
     model.save(path)
     net2, model2 = _cnn(6)
-    assert not np.array_equal(_params(net)[0], _params(net2)[0])
+    assert not np.array_equal(params(net)[0], params(net2)[0])
     model2.load(path)
-    for pa, pb in zip(_params(net), _params(net2)):
+    for pa, pb in zip(params(net), params(net2)):
         assert np.array_equal(pa, pb)
     assert net2.layers[0].params["w"].shape == (5, 5, 1, 8)
     assert np.array_equal(model2.predict(Tensor(x)).values, pred.values)

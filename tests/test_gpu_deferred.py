@@ -6,6 +6,8 @@ is the fused small-MLP pass (other summation orders, as in test_gpu_graph.py).""
 import numpy as np
 import pytest
 
+from support import params
+
 pytestmark = pytest.mark.gpu
 
 MNIST = [200, 100, 70, 30, 10]
@@ -37,10 +39,6 @@ def _batches(d_in, classes, sizes, seed=0):
     rng = np.random.RandomState(seed)
     return [(Tensor(rng.rand(b, d_in).astype(np.float32)), Tensor(np.eye(classes)[rng.randint(0, classes, b)]))
             for b in sizes]
-
-
-def _params(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
 
 
 def _recordings(model):
@@ -83,7 +81,7 @@ def test_five_line_loop_replays_the_generic_recording_bit_identically(opt):
     n0 = be.launch_count()
     lb = _loop(model_b, batches)
     assert [float(v) for v in la] == [float(v) for v in lb]
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
     assert len(_recordings(model_b)) == 2 and not _recordings(model_a)
     assert all(v.dtype == np.float32 and v.shape == () for v in lb)
@@ -105,7 +103,7 @@ def test_defaults_record_layer_by_layer():
         model = Model(net=net, loss=SoftmaxCrossEntropyLoss(), optimizer=Adam(lr=1e-3))
         if not defer:
             model.defer_loop = False
-        out.append(([float(v) for v in _loop(model, batches)], _params(net)))
+        out.append(([float(v) for v in _loop(model, batches)], params(net)))
     assert Model.defer_loop is True and Model.defer_loop_may_fuse is False
     rec = _recordings(model)
     assert len(rec) == 1 and rec[0].info()["kernel_nodes"] >= 10
@@ -128,7 +126,7 @@ def test_five_line_loop_can_reach_the_fused_small_mlp_pass():
         assert abs(float(a) - float(b)) <= 2e-6 * abs(float(a))
     rec = _recordings(model_b)
     assert len(rec) == 2 and all(s.info()["kernel_nodes"] <= 8 for s in rec)
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.max(np.abs(pa - pb)) <= 1e-5 * np.max(np.abs(pa))
 
 
@@ -166,7 +164,7 @@ def test_values_and_gradients_read_around_a_replayed_step(fuse):
     for defer in (False, True):
         net, model = _model(widths, 5, 96, defer=defer, fuse=fuse)
         losses = _loop(model, batches, probe=make_probe(seen[defer]))
-        out[defer] = (losses, _params(net))
+        out[defer] = (losses, params(net))
         if defer:
             assert len(_recordings(model)) == 1
             if fuse:
@@ -221,7 +219,7 @@ def test_anything_else_runs_the_postponed_lines_as_written():
             model.step()
             log.append(float(loss.values))
             assert T._DEFERRED[0] is None
-        res[defer] = (log, _params(net))
+        res[defer] = (log, params(net))
     assert res[False][0] == res[True][0]
     for pa, pb in zip(res[False][1], res[True][1]):
         assert np.array_equal(pa, pb)
@@ -287,7 +285,7 @@ def test_batch_iterator_epochs_through_the_postponed_loop():
         losses = []
         for epoch in range(3):
             losses += _loop(model, [(b.inputs, b.targets) for b in it(x, y)])
-        res[defer] = ([float(v) for v in losses], _params(net))
+        res[defer] = ([float(v) for v in losses], params(net))
         if defer:
             assert len(_recordings(model)) == 2
     assert res[False][0] == res[True][0]
@@ -304,7 +302,7 @@ def test_recordings_are_capped_for_loops_over_many_shapes():
     for defer in (False, True):
         net, model = _model([24, 6], 2, 40, defer=defer, fuse=False)
         model.defer_loop_max_recordings = 3
-        res[defer] = ([float(v) for v in _loop(model, batches)], _params(net))
+        res[defer] = ([float(v) for v in _loop(model, batches)], params(net))
         if defer:
             assert len(_recordings(model)) == 3
     assert res[False][0] == res[True][0]
@@ -321,7 +319,7 @@ import test_gpu_deferred as td
 net, model = td._model(td.MNIST, 3, 784, defer=True, fuse=False)
 losses = td._loop(model, td._batches(784, 10, [128] * 8))
 print("RESULT " + json.dumps([float(v).hex() for v in losses]
-                             + [float(np.sum(p.astype(np.float64))).hex() for p in td._params(net)]))
+                             + [float(np.sum(p.astype(np.float64))).hex() for p in td.params(net)]))
 """
 
 
@@ -370,7 +368,7 @@ def test_gradient_accumulation_over_prefetched_batches():
             if i % 2 == 1:
                 model.step()
             losses.append(float(loss.values) if i % 3 == 0 else None)
-        res[defer] = (losses, _params(net))
+        res[defer] = (losses, params(net))
     assert res[False][0] == res[True][0]
     for pa, pb in zip(res[False][1], res[True][1]):
         assert np.array_equal(pa, pb)
@@ -394,7 +392,7 @@ def test_a_changed_layer_list_is_not_served_by_an_old_recording():
                 losses.append(float(model.train_step(x, y).values))
             else:
                 losses += [float(v) for v in _loop(model, [(x, y)])]
-        res[mode] = (losses, _params(net))
+        res[mode] = (losses, params(net))
         if mode != "eager":
             assert len(_recordings(model)) == 2
     for mode in ("loop", "train_step"):

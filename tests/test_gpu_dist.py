@@ -1,37 +1,16 @@
 """Data-parallel parity on real GPUs (skipped on a 1-GPU box): 2 ranks over NCCL vs the
 single-process oracle on the full batch."""
-import ctypes
-import os
-import socket
-import subprocess
-import sys
-
 import pytest
 
+from support import gpu_count, run_two_ranks
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _gpu_count():
-    import core._backend as be
-    n = ctypes.c_int(0)
-    if be.load_library().tnn_device_count(ctypes.byref(n)):
-        return 0
-    return n.value
 
 
 def test_two_rank_training_equals_full_batch_oracle():
-    if _gpu_count() < 2:
+    if gpu_count() < 2:
         pytest.skip("needs 2 GPUs")
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", str(port),
-           os.path.join(ROOT, "tests", "dist_worker.py")]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=150, cwd=ROOT)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    assert "DIST_OK world=2" in r.stdout
-    assert "GRAPH_DIST_OK world=2" in r.stdout
-    assert "CHUNKED_DIST_OK world=2" in r.stdout
+    out = run_two_ranks("dist_worker.py", timeout=150)
+    assert "DIST_OK world=2" in out
+    assert "GRAPH_DIST_OK world=2" in out
+    assert "CHUNKED_DIST_OK world=2" in out

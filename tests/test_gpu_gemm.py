@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import op_cases
+from support import gemm_route
 
 pytestmark = pytest.mark.gpu
 
@@ -78,41 +79,28 @@ def test_tf32x3_gemm_shapes(be, cg, shape, split, mn_major):
     "tf32x3": three tf32 MMAs.  mn_major=True feeds transposed operands MN-major from the plain
     planes (default), False goes through transposed planes (both operands K-major)"""
     M, N, K = shape
-    be.set_gemm_cta_group(cg)
-    old_mn, old_split = be.TC_MN_MAJOR, be.TC_SPLIT
-    be.TC_MN_MAJOR = mn_major
-    be.TC_SPLIT = split
-    try:
+    with gemm_route(cta_group=cg, TC_MN_MAJOR=mn_major, TC_SPLIT=split, TC_MIN_MNK=0):
         rng = np.random.RandomState(M * 7 + N * 3 + K)
         a = rng.standard_normal((M, K)).astype(np.float32)
         b = rng.standard_normal((K, N)).astype(np.float32)
         bias = rng.standard_normal((1, N)).astype(np.float32)
         da, db, dbias = be.from_numpy(a), be.from_numpy(b), be.from_numpy(bias)
-        old = be.TC_MIN_MNK
-        be.TC_MIN_MNK = 0
-        try:
-            out = be.matmul(da, db, bias=dbias).numpy()
-            ref = _ref(a, b, False, False, bias)
-            assert op_cases.rel_err(out, ref) <= TOL
-            # NT: (M,K) @ (N,K)^T
-            bt = np.ascontiguousarray(b.T)
-            out = be.matmul(da, be.from_numpy(bt), tb=True).numpy()
-            assert op_cases.rel_err(out, _ref(a, bt, False, True, None)) <= TOL
-            # TN: (K,M)^T @ (K,N), accumulate into an existing buffer
-            at = np.ascontiguousarray(a.T)
-            c0 = rng.standard_normal((M, N)).astype(np.float32)
-            dc = be.from_numpy(c0)
-            be.matmul(be.from_numpy(at), db, ta=True, out=dc, accumulate=True)
-            assert op_cases.rel_err(dc.numpy(), _ref(at, b, True, False, None) + c0) <= TOL
-            # relu epilogue
-            out = be.matmul(da, db, bias=dbias, relu=True).numpy()
-            assert op_cases.rel_err(out, np.maximum(ref, 0)) <= TOL
-        finally:
-            be.TC_MIN_MNK = old
-    finally:
-        be.TC_MN_MAJOR = old_mn
-        be.TC_SPLIT = old_split
-        be.set_gemm_cta_group(0)
+        out = be.matmul(da, db, bias=dbias).numpy()
+        ref = _ref(a, b, False, False, bias)
+        assert op_cases.rel_err(out, ref) <= TOL
+        # NT: (M,K) @ (N,K)^T
+        bt = np.ascontiguousarray(b.T)
+        out = be.matmul(da, be.from_numpy(bt), tb=True).numpy()
+        assert op_cases.rel_err(out, _ref(a, bt, False, True, None)) <= TOL
+        # TN: (K,M)^T @ (K,N), accumulate into an existing buffer
+        at = np.ascontiguousarray(a.T)
+        c0 = rng.standard_normal((M, N)).astype(np.float32)
+        dc = be.from_numpy(c0)
+        be.matmul(be.from_numpy(at), db, ta=True, out=dc, accumulate=True)
+        assert op_cases.rel_err(dc.numpy(), _ref(at, b, True, False, None) + c0) <= TOL
+        # relu epilogue
+        out = be.matmul(da, db, bias=dbias, relu=True).numpy()
+        assert op_cases.rel_err(out, np.maximum(ref, 0)) <= TOL
 
 
 @pytest.mark.parametrize("split", ["mix", "tf32x3"])
@@ -125,10 +113,7 @@ def test_fused_activation_outputs(be, split):
     b = rng.standard_normal((K, N)).astype(np.float32)
     bias = rng.standard_normal((1, N)).astype(np.float32)
     w2 = rng.standard_normal((N, 72)).astype(np.float32)
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK = 0
-    be.TC_SPLIT = split
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT=split):
         z, act = be.matmul(be.from_numpy(a), be.from_numpy(b), bias=be.from_numpy(bias), act=True)
         zr = _ref(a, b, False, False, bias)
         assert op_cases.rel_err(z.numpy(), zr) <= TOL
@@ -150,8 +135,6 @@ def test_fused_activation_outputs(be, split):
         pre = rng.standard_normal((M, N)).astype(np.float32)
         g, masked = be.matmul(be.from_numpy(a), be.from_numpy(b), act=True, mask_src=be.from_numpy(pre))
         assert np.array_equal(masked.numpy(), g.numpy() * (pre >= 0))
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 def _meta(rec):
@@ -198,9 +181,7 @@ def test_f16_gemm_shapes(be, shape):
     """default path: NN / NT / TN (+ accumulate) / relu epilogue on operands of very different
     magnitudes (the per-tensor scale exponents are exercised), rel 1e-5 of max|ref|"""
     M, N, K = shape
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "f16"
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="f16"):
         rng = np.random.RandomState(M * 7 + N * 3 + K)
         a = (rng.standard_normal((M, K)) * 3.7e-6).astype(np.float32)
         b = (rng.standard_normal((K, N)) * 4.1e4).astype(np.float32)
@@ -223,8 +204,6 @@ def test_f16_gemm_shapes(be, shape):
         assert np.array_equal(outs[0], outs[1])                       # run-to-run identical
         out = be.matmul(da, db, bias=dbias, relu=True).numpy()
         assert op_cases.rel_err(out, np.maximum(ref, 0)) <= TOL
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 @pytest.mark.parametrize("shape", [(256, 512, 128), (384, 768, 200), (300, 300, 96), (1000, 520, 260),
@@ -234,9 +213,7 @@ def test_f16_gemm_multicast_clusters(be, shape):
     their A rows by TMA multicast (odd tile-column counts leave the second pair of the last cluster
     without a tile).  Bit-identical to the pair kernel: same products, same order."""
     M, N, K = shape
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "f16"
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="f16"):
         rng = np.random.RandomState(M + 5 * N + K)
         a = rng.standard_normal((M, K)).astype(np.float32)
         b = rng.standard_normal((K, N)).astype(np.float32)
@@ -244,17 +221,14 @@ def test_f16_gemm_multicast_clusters(be, shape):
         at, bt = np.ascontiguousarray(a.T), np.ascontiguousarray(b.T)
         res = {}
         for cl in (2, 4):
-            be.set_gemm_f16_cluster(cl)
-            da, db = be.from_numpy(a), be.from_numpy(b)
-            res[cl] = [be.matmul(da, db, bias=be.from_numpy(bias)).numpy(),
-                       be.matmul(da, be.from_numpy(bt), tb=True).numpy(),
-                       be.matmul(be.from_numpy(at), db, ta=True).numpy()]
+            with gemm_route(f16_cluster=cl):
+                da, db = be.from_numpy(a), be.from_numpy(b)
+                res[cl] = [be.matmul(da, db, bias=be.from_numpy(bias)).numpy(),
+                           be.matmul(da, be.from_numpy(bt), tb=True).numpy(),
+                           be.matmul(be.from_numpy(at), db, ta=True).numpy()]
         assert op_cases.rel_err(res[4][0], _ref(a, b, False, False, bias)) <= TOL
         for x, y in zip(res[2], res[4]):
             assert np.array_equal(x, y)
-    finally:
-        be.set_gemm_f16_cluster(2)
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 def test_f16_fused_outputs(be):
@@ -267,9 +241,7 @@ def test_f16_fused_outputs(be):
     b = rng.standard_normal((K, N)).astype(np.float32)
     bias = rng.standard_normal((1, N)).astype(np.float32)
     w2 = rng.standard_normal((N, 72)).astype(np.float32)
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "f16"
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="f16"):
         z, act = be.matmul(be.from_numpy(a), be.from_numpy(b), bias=be.from_numpy(bias), act=True)
         assert op_cases.rel_err(z.numpy(), _ref(a, b, False, False, bias)) <= TOL
         assert type(act) is be.LazyReLU and act._real is None
@@ -287,8 +259,6 @@ def test_f16_fused_outputs(be):
         y1 = be.matmul(masked, be.from_numpy(w2)).numpy()
         y2 = be.matmul(be.from_numpy(masked.numpy()), be.from_numpy(w2)).numpy()
         assert np.array_equal(y1, y2)
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 def test_f16_guard_falls_back_on_device(be):
@@ -301,9 +271,7 @@ def test_f16_guard_falls_back_on_device(be):
     a = rng.standard_normal((M, K)).astype(np.float32)
     a[::2] *= np.float32(1e-30)
     b = rng.standard_normal((K, N)).astype(np.float32)
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "f16"
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="f16"):
         da, db = be.from_numpy(a), be.from_numpy(b)
         z, act = be.matmul(da, db, act=True)
         assert _meta(da.split["f"][3])["safe"] == 0 and _meta(db.split["f"][3])["safe"] == 1
@@ -323,8 +291,6 @@ def test_f16_guard_falls_back_on_device(be):
         assert np.all(~np.isfinite(out[3])) and np.all(np.isfinite(np.delete(out, 3, axis=0)))
         zero = be.matmul(be.from_numpy(np.zeros((M, K), np.float32)), db)
         assert np.all(zero.numpy() == 0)
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 def test_f16_tensor_relative_bound(be):
@@ -337,14 +303,10 @@ def test_f16_tensor_relative_bound(be):
     a = rng.standard_normal((M, K)).astype(np.float32)
     a[7] *= np.float32(2.0 ** -25)
     b = rng.standard_normal((K, N)).astype(np.float32)
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "f16"
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="f16"):
         da = be.from_numpy(a)
         c = be.matmul(da, be.from_numpy(b)).numpy().astype(np.float64)
         assert _meta(da.split["f"][3])["safe"] == 1
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
     a64, b64 = a.astype(np.float64), b.astype(np.float64)
     err = np.abs(c - a64 @ b64)
     comp = np.abs(a64) @ np.abs(b64)
@@ -366,11 +328,7 @@ def test_tf32x3_ordered_split_k(be, cg, ks):
     c0 = rng.standard_normal((M, N)).astype(np.float32)
     da, db, dbias = be.from_numpy(a), be.from_numpy(b), be.from_numpy(bias)
     ref = _ref(a, b, False, False, bias) + c0
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, "mix"
-    be.set_gemm_cta_group(cg)
-    be.set_gemm_ksplit(ks)
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT="mix", cta_group=cg, ksplit=ks):
         outs = []
         for _ in range(3):
             dc = be.from_numpy(c0)
@@ -378,10 +336,6 @@ def test_tf32x3_ordered_split_k(be, cg, ks):
             outs.append(dc.numpy())
         assert op_cases.rel_err(outs[0], ref) <= TOL
         assert np.array_equal(outs[0], outs[1]) and np.array_equal(outs[0], outs[2])
-    finally:
-        be.set_gemm_ksplit(0)
-        be.set_gemm_cta_group(0)
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 def test_tf32x3_better_than_plain_tf32(be):
@@ -390,12 +344,8 @@ def test_tf32x3_better_than_plain_tf32(be):
     M, N, K = 512, 512, 4096
     a = rng.rand(M, K).astype(np.float32)
     b = rng.rand(K, N).astype(np.float32)
-    old = be.TC_MIN_MNK
-    be.TC_MIN_MNK = 0
-    try:
+    with gemm_route(TC_MIN_MNK=0):
         out = be.matmul(be.from_numpy(a), be.from_numpy(b)).numpy()
-    finally:
-        be.TC_MIN_MNK = old
     ref = a.astype(np.float64) @ b.astype(np.float64)
     # all-positive data is the worst case for the tensor core's round-toward-zero accumulation
     # inside a chunk (8 K-blocks = 256 k since r02: between 2e-6 and 3e-6 here, 1.3e-6 on signed data)
@@ -414,16 +364,12 @@ def test_simt_gemm(be, dtype, shape):
     b = rng.standard_normal((K, N)).astype(dtype)
     bias = rng.standard_normal((1, N)).astype(dtype)
     tol = 2e-6 if dtype == np.float32 else 1e-13
-    old = be.TC_ENABLED
-    be.TC_ENABLED = False
-    try:
+    with gemm_route(TC_ENABLED=False):
         da, db = be.from_numpy(a), be.from_numpy(b)
         assert op_cases.rel_err(be.matmul(da, db, bias=be.from_numpy(bias)).numpy(), _ref(a, b, False, False, bias)) <= tol
         at, bt = np.ascontiguousarray(a.T), np.ascontiguousarray(b.T)
         assert op_cases.rel_err(be.matmul(be.from_numpy(at), db, ta=True).numpy(), _ref(at, b, True, False, None)) <= tol
         assert op_cases.rel_err(be.matmul(da, be.from_numpy(bt), tb=True).numpy(), _ref(a, bt, False, True, None)) <= tol
-    finally:
-        be.TC_ENABLED = old
 
 
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])
@@ -438,9 +384,7 @@ def test_simt_gemm_fused_outputs(be, dtype, shape):
     pre = rng.standard_normal((M, N)).astype(dtype)
     pre[0, 0] = 0.0
     tol = 2e-6 if dtype == np.float32 else 1e-13
-    old = be.TC_ENABLED
-    be.TC_ENABLED = False
-    try:
+    with gemm_route(TC_ENABLED=False):
         da, dbt = be.from_numpy(a), be.from_numpy(bt)
         ref = a.astype(np.float64) @ bt.astype(np.float64).T
         z, act = be.matmul(da, dbt, tb=True, act=True)
@@ -449,5 +393,3 @@ def test_simt_gemm_fused_outputs(be, dtype, shape):
         g, masked = be.matmul(da, dbt, tb=True, act=True, mask_src=be.from_numpy(pre))
         assert np.array_equal(g.numpy(), z.numpy())
         assert np.array_equal(masked.numpy(), g.numpy() * (pre >= 0))
-    finally:
-        be.TC_ENABLED = old

@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import ref_numpy as R
+from support import gemm_route, params
 
 pytestmark = pytest.mark.gpu
 
@@ -46,10 +47,6 @@ def _eager(model, x, y):
     return loss
 
 
-def _params(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
-
 def _batches(n_rows, d_in, classes, sizes, seed=0):
     from core.tensor import Tensor
     rng = np.random.RandomState(seed)
@@ -77,7 +74,7 @@ def test_captured_mnist_step_is_bit_identical(opt):
     assert len(states) == 2 and all(hasattr(s, "graph") for s in states)   # both shapes were recorded
     info = states[0].info()
     assert info["kernel_nodes"] >= 10 and info["blocks"] > 0
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
 
 
@@ -105,7 +102,7 @@ def test_fused_small_mlp_step_matches_eager(opt, label_dtype):
     states = [s for s in model_b._captured.values()]
     assert len(states) == 2 and all(hasattr(s, "graph") for s in states)
     assert all(s.info()["kernel_nodes"] <= 8 for s in states)          # the fused pass was recorded
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.max(np.abs(pa - pb)) <= 1e-5 * np.max(np.abs(pa))
 
 
@@ -124,7 +121,7 @@ def test_fused_small_mlp_other_shapes(widths, d_in, batch):
         lb = float(model_b.train_step(x, y).values)
         assert abs(la - lb) <= 2e-6 * abs(la), (la, lb)
     assert all(s.info()["kernel_nodes"] <= 8 for s in model_b._captured.values() if hasattr(s, "graph"))
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.max(np.abs(pa - pb)) <= 1e-5 * np.max(np.abs(pa))
 
 
@@ -154,7 +151,7 @@ def test_fused_small_mlp_is_not_used_where_it_does_not_apply():
             model = Model(net=net, loss=loss, optimizer=Adam(lr=1e-3))
             losses = [float((model.train_step(x, y) if use_graph else _eager(model, x, y)).values)
                       for _ in range(5)]
-            out.append((losses, _params(net)))
+            out.append((losses, params(net)))
             if use_graph:
                 assert model._fused_mlp_plan(x, y) is None
         assert out[0][0] == out[1][0]
@@ -211,7 +208,7 @@ def test_fused_small_mlp_teacher_forced_on_learnable_data():
         assert abs(la - lb) <= 1e-6 * abs(la), (k, la, lb)
         if k >= 2:                                   # from the third call on the fused recording runs
             compared += 1
-            for pa, pb in zip(_params(net_a), _params(net_b)):
+            for pa, pb in zip(params(net_a), params(net_b)):
                 assert np.max(np.abs(pa - pb)) <= 1e-6 * np.max(np.abs(pa)), k
     assert compared == 38 and any(hasattr(s, "graph") and s.info()["kernel_nodes"] <= 8
                                   for s in b._captured.values())
@@ -221,9 +218,7 @@ def test_captured_tensor_core_step_is_bit_identical():
     """256-wide layers at batch 1024: every product is above the tensor-core threshold"""
     import core._backend as be
     widths = [256, 256, 256]
-    old = be.TC_MIN_MNK
-    be.TC_MIN_MNK = 1 << 26
-    try:
+    with gemm_route(TC_MIN_MNK=1 << 26):
         assert be.use_tensor_cores(1024, 256, 256, be.F32)
         batches = _batches(0, 256, 256, [1024] * 6)
         net_a, model_a = _model(widths, 5, d_in=256)
@@ -232,10 +227,8 @@ def test_captured_tensor_core_step_is_bit_identical():
             la = float(_eager(model_a, x, y).values)
             lb = float(model_b.train_step(x, y).values)
             assert la == lb
-        for pa, pb in zip(_params(net_a), _params(net_b)):
+        for pa, pb in zip(params(net_a), params(net_b)):
             assert np.array_equal(pa, pb)
-    finally:
-        be.TC_MIN_MNK = old
 
 
 def test_replay_does_not_touch_other_tensors():
@@ -334,6 +327,6 @@ def test_recorded_step_is_dropped_when_a_parameter_is_rebound():
         la = float(_eager(model_a, x, y).values)
         lb = float(model_b.train_step(x, y).values)
         assert la == lb, i
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
     assert any(hasattr(s, "graph") for s in model_b._captured.values())

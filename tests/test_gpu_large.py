@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import op_cases
+from support import gemm_route
 
 pytestmark = pytest.mark.gpu
 
@@ -68,8 +69,7 @@ def test_row_gather_permutation_roundtrip(be):
 def test_wide_gemm_spot_check(be, cg):
     """config 4's GEMM shape (8192 x 4096 x 4096) in all three orientations of a Dense layer;
     512 random output entries checked against float64 dot products, plus linearity in A"""
-    be.set_gemm_cta_group(cg)
-    try:
+    with gemm_route(cta_group=cg):
         rng = np.random.RandomState(2)
         M, N, K = 8192, 4096, 4096
         a = rng.rand(M, K).astype(np.float32)
@@ -92,5 +92,3 @@ def test_wide_gemm_spot_check(be, cg):
         # linearity: (2a) @ w == 2 (a @ w) exactly (scaling by 2 is exact in every split plane)
         y2 = be.matmul(be.ew(be.SCALE, da, p0=2.0, p1=0.0), dw).numpy()
         assert np.array_equal(y2, 2.0 * y)
-    finally:
-        be.set_gemm_cta_group(0)

@@ -6,21 +6,15 @@ reproducibility, NaN / inf, an empty row and a 2^26-element case; then training 
 a regression MLP with MSELoss and an NHWC CNN head with SigmoidCrossEntropyLoss against the oracle,
 train_step and the recorded five-line loop against the eager step, and a loop alternating two Huber
 deltas."""
-import ctypes
-import os
-import socket
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
 import ref_conv as RC
 import ref_losses as RL
 import ref_numpy as R
+from support import gpu_count, params, run_two_ranks
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
@@ -234,13 +228,9 @@ def _mlp(seed, loss):
     return net, Model(net=net, loss=loss, optimizer=Adam(lr=1e-3))
 
 
-def _params(net):
-    return [p.values.copy() for layer in net.get_parameters() for p in layer.values()]
-
-
 class _RefMLP(object):
     def __init__(self, net, kind, delta=1.0):
-        self.p = [R.RefTensor(v, True) for v in _params(net)]
+        self.p = [R.RefTensor(v, True) for v in params(net)]
         self.kind, self.delta = kind, delta
         self.opt = R.RefAdam(lr=1e-3)
 
@@ -317,7 +307,7 @@ def _cnn(seed):
 
 class _RefCNN(object):
     def __init__(self, net):
-        self.p = [R.RefTensor(v, True) for v in _params(net)]
+        self.p = [R.RefTensor(v, True) for v in params(net)]
         self.opt = R.RefAdam(lr=1e-3)
 
     def step(self, x, y):
@@ -386,7 +376,7 @@ def test_train_step_and_recorded_loop_are_bit_identical_to_eager(be, which):
     assert [s for s in model_b._captured.values() if hasattr(s, "graph")]
     if which.startswith("mlp"):
         assert [s for s in model_c._captured.values() if hasattr(s, "graph")]
-    for pa, pb, pc in zip(_params(net_a), _params(net_b), _params(net_c)):
+    for pa, pb, pc in zip(params(net_a), params(net_b), params(net_c)):
         assert np.array_equal(pa, pb) and np.array_equal(pa, pc)
 
 
@@ -413,7 +403,7 @@ def test_alternating_huber_deltas_in_the_recorded_loop(be):
     assert np.max(np.abs(np.array(out_a) - np.array(rl))) <= 1e-4
     recorded = [k for k, s in model_b._captured.items() if hasattr(s, "graph")]
     assert sorted(k[-1] for k in recorded) == [(1.0,), (2.0,)]
-    for pa, pb in zip(_params(net_a), _params(net_b)):
+    for pa, pb in zip(params(net_a), params(net_b)):
         assert np.array_equal(pa, pb)
     # train_step with the model's loss swapped between the two deltas: the same bits again
     net_c, model_c = _mlp(2, HuberLoss(1.0))
@@ -425,24 +415,7 @@ def test_alternating_huber_deltas_in_the_recorded_loop(be):
 
 
 # ---------------------------------------------------------------------------- two ranks
-def _gpu_count():
-    import core._backend as be
-    n = ctypes.c_int(0)
-    if be.load_library().tnn_device_count(ctypes.byref(n)):
-        return 0
-    return n.value
-
-
 def test_two_rank_losses_equal_full_batch_oracle():
-    if _gpu_count() < 2:
+    if gpu_count() < 2:
         pytest.skip("needs 2 GPUs")
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", str(port),
-           os.path.join(ROOT, "tests", "loss_dist_worker.py")]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=200, cwd=ROOT)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    assert "LOSS_DIST_OK world=2" in r.stdout
+    assert "LOSS_DIST_OK world=2" in run_two_ranks("loss_dist_worker.py", timeout=200)

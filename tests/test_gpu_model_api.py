@@ -8,6 +8,7 @@ import pytest
 
 import op_cases
 import ref_numpy as R
+from support import params
 
 pytestmark = pytest.mark.gpu
 
@@ -36,7 +37,7 @@ def _pair(widths, optimizer, ref_optimizer, seed, x):
     np.random.seed(seed)
     ref = R.RefMLP(widths, ref_optimizer)
     ref.forward(R.lift(x))
-    for p, rp in zip(_params(net), ref.params()):
+    for p, rp in zip(_param_tensors(net), ref.params()):
         assert np.array_equal(p.values, rp.values)
     return net, model, ref
 
@@ -46,7 +47,7 @@ def _data(seed=2, B=16, D=20, C=10):
     return rng.rand(B, D).astype(np.float32), np.eye(C, dtype=np.float32)[rng.randint(0, C, B)]
 
 
-def _params(net):
+def _param_tensors(net):
     return [p for layer in net.get_parameters() for p in layer.values()]
 
 
@@ -79,15 +80,15 @@ def test_user_defined_optimizer_is_called():
     np.random.seed(3)
     net, model = _mlp([13, 10], SignSGD(lr=0.01))
     model.forward(__import__("core.tensor", fromlist=["Tensor"]).Tensor(x))
-    before = [p.values.copy() for p in _params(net)]
+    before = params(net)
     from core.tensor import Tensor
     model.zero_grad()
     loss = model.loss.loss(model.forward(Tensor(x)), Tensor(y))
     loss.backward()
-    grads = [p.grad.copy() for p in _params(net)]
+    grads = [p.grad.copy() for p in _param_tensors(net)]
     model.step()
     assert SignSGD.calls == 1
-    for b, g, p in zip(before, grads, _params(net)):
+    for b, g, p in zip(before, grads, _param_tensors(net)):
         assert np.allclose(p.values, b - 0.01 * np.sign(g), atol=1e-7)
 
 
@@ -110,7 +111,7 @@ def test_subclass_overriding_compute_step_is_not_bypassed():
         params = ref.params()
         for p, s in zip(params, ref.optimizer.compute_steps(params)):
             p.assign((p.values + np.clip(s, -5e-4, 5e-4)).astype(np.float32))
-    for p, rp in zip(_params(net), ref.params()):
+    for p, rp in zip(_param_tensors(net), ref.params()):
         assert op_cases.rel_err(p.values, rp.values) <= 1e-5
 
 
@@ -129,16 +130,16 @@ def test_assigned_gradient_stays_on_the_fused_path():
         ref.zero_grad()
         R.softmax_cross_entropy(ref.forward(R.lift(x)), y).backward()
         if it >= 1:                                  # the arenas exist from the first step on
-            for p in _params(net):
+            for p in _param_tensors(net):
                 p.grad = np.clip(p.grad, -1e-3, 1e-3)
             for rp in ref.params():
                 rp.grad = np.clip(rp.grad, -1e-3, 1e-3)
         model.step()
-        assert model._arena is not None and all(p._gslot is not None for p in _params(net))
+        assert model._arena is not None and all(p._gslot is not None for p in _param_tensors(net))
         ref.step()
         for rp in ref.params():
             rp.assign(rp.values.astype(np.float32).astype(np.float64))
-    for p, rp in zip(_params(net), ref.params()):
+    for p, rp in zip(_param_tensors(net), ref.params()):
         assert op_cases.rel_err(p.values, rp.values) <= 1e-5
 
 
@@ -174,7 +175,7 @@ def test_weight_decay_is_opt_in(name, fused):
                 if apply:
                     s = s - 0.1 * p.values
                 p.assign((p.values + s).astype(np.float32))
-        for p, rp in zip(_params(net), ref.params()):
+        for p, rp in zip(_param_tensors(net), ref.params()):
             assert op_cases.rel_err(p.values, rp.values) <= 1e-5, (name, apply)
 
 
@@ -244,7 +245,7 @@ def test_failed_capture_falls_back_to_eager():
         if peek:
             model.loss = PeekingLoss()
         losses = [float(model.train_step(Tensor(x), Tensor(y)).values) for _ in range(5)]
-        results.append((losses, [p.values.copy() for p in _params(net)]))
+        results.append((losses, params(net)))
     assert np.allclose(results[0][0], results[1][0], rtol=0, atol=1e-6)
     for a, b in zip(results[0][1], results[1][1]):
         assert op_cases.rel_err(a, b) <= 1e-6
@@ -285,16 +286,16 @@ def test_optimizer_that_only_offers_compute_step():
     net, model = _mlp([13, 10], Plain())
     losses = []
     for _ in range(4):
-        before = [p.values.copy() for p in _params(net)] if net.layers[0].is_init else None
+        before = params(net) if net.layers[0].is_init else None
         model.zero_grad()
         pred = model.forward(Tensor(x))
         assert type(pred) is Tensor
         loss = model.loss.loss(pred, Tensor(y))
         loss.backward()
-        grads = [p.grad.copy() for p in _params(net)]
+        grads = [p.grad.copy() for p in _param_tensors(net)]
         model.step()
         if before is not None:
-            for b, g, p in zip(before, grads, _params(net)):
+            for b, g, p in zip(before, grads, _param_tensors(net)):
                 assert np.allclose(p.values, b - 0.05 * g, atol=1e-7)
         losses.append(float(loss.values))
     assert losses[-1] < losses[0] and not model._captured

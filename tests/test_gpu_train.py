@@ -7,6 +7,7 @@ import pytest
 
 import op_cases
 import ref_numpy as R
+from support import gemm_route
 
 pytestmark = pytest.mark.gpu
 
@@ -181,10 +182,7 @@ def test_tensor_core_mlp_step_teacher_forced(cg):
     compared with the oracle started from the same parameters (teacher forcing, SURVEY 7.3)"""
     import core._backend as be
     from core.tensor import Tensor
-    be.set_gemm_cta_group(cg)
-    old = be.TC_MIN_MNK
-    be.TC_MIN_MNK = 1 << 20
-    try:
+    with gemm_route(cta_group=cg, TC_MIN_MNK=1 << 20):
         np.random.seed(1)
         rng = np.random.RandomState(1)
         B, D = 1024, 512
@@ -222,9 +220,6 @@ def test_tensor_core_mlp_step_teacher_forced(cg):
             expect = a + flat_step[pos:pos + g.size].reshape(g.shape)
             pos += g.size
             assert op_cases.rel_err(p.values, expect) <= 1e-5
-    finally:
-        be.TC_MIN_MNK = old
-        be.set_gemm_cta_group(0)
 
 
 @pytest.mark.parametrize("fuse_bwd", [False, True])
@@ -243,33 +238,31 @@ def test_dense_relu_fusion_is_transparent(size, fuse_bwd):
     rng = np.random.RandomState(7)
     x = rng.standard_normal((B, D)).astype(np.float32)
     labels = np.eye(C, dtype=np.float32)[rng.randint(0, C, B)]
-    old = be.TC_MIN_MNK
     old_bwd = ops.FUSE_RELU_BWD
-    be.TC_MIN_MNK = 1 << 22
     ops.FUSE_RELU_BWD = fuse_bwd   # also fold the ReLU-backward mask into the dX launch
     try:
-        outs = []
-        for fused in (True, False):
-            np.random.seed(11)
-            layers = [Dense(H), ReLU(), Dense(H), ReLU(), Dense(C)]
-            net = Net(layers)
-            be.new_split_epoch()
-            if fused:
-                pred = net.forward(Tensor(x))
-            else:
-                pred = Tensor(x)
-                for layer in layers:
-                    pred = layer.forward(pred)
-            loss = SoftmaxCrossEntropyLoss().loss(pred, Tensor(labels))
-            loss.backward()
-            grads = [p.grad.copy() for layer in net.get_parameters() for p in layer.values()]
-            outs.append((pred.values.copy(), layers[1].inputs.values.copy(), layers[2].inputs.values.copy(), grads))
-        a, b = outs
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
-        for ga, gb in zip(a[3], b[3]):
-            assert np.array_equal(ga, gb)
+        with gemm_route(TC_MIN_MNK=1 << 22):
+            outs = []
+            for fused in (True, False):
+                np.random.seed(11)
+                layers = [Dense(H), ReLU(), Dense(H), ReLU(), Dense(C)]
+                net = Net(layers)
+                be.new_split_epoch()
+                if fused:
+                    pred = net.forward(Tensor(x))
+                else:
+                    pred = Tensor(x)
+                    for layer in layers:
+                        pred = layer.forward(pred)
+                loss = SoftmaxCrossEntropyLoss().loss(pred, Tensor(labels))
+                loss.backward()
+                grads = [p.grad.copy() for layer in net.get_parameters() for p in layer.values()]
+                outs.append((pred.values.copy(), layers[1].inputs.values.copy(), layers[2].inputs.values.copy(), grads))
+            a, b = outs
+            assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
+            for ga, gb in zip(a[3], b[3]):
+                assert np.array_equal(ga, gb)
     finally:
-        be.TC_MIN_MNK = old
         ops.FUSE_RELU_BWD = old_bwd
 
 
@@ -687,9 +680,7 @@ def test_tensor_core_mlp_teacher_forced_over_steps(split):
     the arithmetic."""
     import core._backend as be
     from core.tensor import Tensor
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 1 << 20, split
-    try:
+    with gemm_route(TC_MIN_MNK=1 << 20, TC_SPLIT=split):
         rng = np.random.RandomState(8)
         B, D = 512, 256
         np.random.seed(8)
@@ -732,8 +723,6 @@ def test_tensor_core_mlp_teacher_forced_over_steps(split):
             for rp in mlp.params():
                 rp.assign(rp.values.astype(np.float32).astype(np.float64))
         assert compared >= 9
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
 
 
 @pytest.mark.parametrize("dtype,tol", [(np.float32, 2e-6), (np.float64, 1e-12)])

@@ -10,6 +10,7 @@ import pytest
 
 import op_cases
 import ref_numpy as R
+from support import gemm_route
 
 pytestmark = pytest.mark.gpu
 
@@ -64,63 +65,61 @@ def test_wide_mlp_step_matches_oracle(wide_case, split):
     import core._backend as be
     from core.tensor import Tensor
     x, labels, mlp = wide_case["x"], wide_case["labels"], wide_case["mlp"]
-    old_split = be.TC_SPLIT
-    be.TC_SPLIT = split
-    be.set_gemm_cta_group(0)            # production default: CTA pairs, tail split-K on ragged waves
     try:
-        np.random.seed(1)
-        net, model = _engine_model(wide_case["init"])
-        params = [p for layer in net.get_parameters() for p in layer.values()]
-        assert be.use_tensor_cores(B, D, D, be.F32)
-        model.zero_grad()
-        loss = model.loss.loss(model.forward(Tensor(x)), Tensor(labels))
-        pre = [layer.inputs.values for layer in net.layers if layer.name == "ReLU"]
+        # cta_group 0 is the production default: CTA pairs, tail split-K on ragged waves
+        with gemm_route(TC_SPLIT=split, cta_group=0):
+            np.random.seed(1)
+            net, model = _engine_model(wide_case["init"])
+            params = [p for layer in net.get_parameters() for p in layer.values()]
+            assert be.use_tensor_cores(B, D, D, be.F32)
+            model.zero_grad()
+            loss = model.loss.loss(model.forward(Tensor(x)), Tensor(labels))
+            pre = [layer.inputs.values for layer in net.layers if layer.name == "ReLU"]
 
-        # ---- oracle forward; pre-activations within rounding distance of the ReLU kink -------------
-        relus = [layer for layer in mlp.layers if isinstance(layer, R.RefReLU)]
-        for r in relus:
-            r.keep_override = None
-        mlp.zero_grad()
-        hcur, ref_pre = R.lift(x), []
-        for layer in mlp.layers:
-            hcur = layer.forward(hcur)
-            if isinstance(layer, R.RefDense):
-                ref_pre.append(hcur.values)
-        flips = 0
-        for z, zr in zip(pre, ref_pre[:3]):
-            assert op_cases.rel_err(z, zr) <= 1e-5
-            differ = (z >= 0) != (zr >= 0)
-            flips += int(differ.sum())
-            # only entries that are zero to rounding may land on the other side of the kink
-            assert np.all(np.abs(zr[differ]) <= 1e-5 * np.max(np.abs(zr)))
-        assert flips <= 256, flips          # of 12.6 M pre-activations (expected: a few tens)
+            # ---- oracle forward; pre-activations within rounding distance of the ReLU kink -------------
+            relus = [layer for layer in mlp.layers if isinstance(layer, R.RefReLU)]
+            for r in relus:
+                r.keep_override = None
+            mlp.zero_grad()
+            hcur, ref_pre = R.lift(x), []
+            for layer in mlp.layers:
+                hcur = layer.forward(hcur)
+                if isinstance(layer, R.RefDense):
+                    ref_pre.append(hcur.values)
+            flips = 0
+            for z, zr in zip(pre, ref_pre[:3]):
+                assert op_cases.rel_err(z, zr) <= 1e-5
+                differ = (z >= 0) != (zr >= 0)
+                flips += int(differ.sum())
+                # only entries that are zero to rounding may land on the other side of the kink
+                assert np.all(np.abs(zr[differ]) <= 1e-5 * np.max(np.abs(zr)))
+            assert flips <= 256, flips          # of 12.6 M pre-activations (expected: a few tens)
 
-        # ---- oracle backward with the device's masks on those few entries -------------------------
-        for r, z in zip(relus, pre):
-            r.keep_override = (z >= 0)
-        mlp.zero_grad()
-        rloss = R.softmax_cross_entropy(mlp.forward(R.lift(x)), labels)
-        assert abs(float(loss.values) - float(rloss.values)) <= 1e-5
-        loss.backward()
-        rloss.backward()
-        for k, (p, rp) in enumerate(zip(params, mlp.params())):
-            assert op_cases.rel_err(p.grad, rp.grad) <= 1e-5, (split, k)
+            # ---- oracle backward with the device's masks on those few entries -------------------------
+            for r, z in zip(relus, pre):
+                r.keep_override = (z >= 0)
+            mlp.zero_grad()
+            rloss = R.softmax_cross_entropy(mlp.forward(R.lift(x)), labels)
+            assert abs(float(loss.values) - float(rloss.values)) <= 1e-5
+            loss.backward()
+            rloss.backward()
+            for k, (p, rp) in enumerate(zip(params, mlp.params())):
+                assert op_cases.rel_err(p.grad, rp.grad) <= 1e-5, (split, k)
 
-        # ---- fused arena Adam over all 67 M parameters, fed the engine's own gradients (Adam's
-        # first step is -lr*g/(|g|+eps): entries with |g| ~ eps turn a 1e-9 gradient difference into
-        # an O(lr) step difference, so both sides get the same gradient) ---------------------------
-        p0 = [p.values.astype(np.float64) for p in params]
-        g0 = [p.grad.astype(np.float64) for p in params]
-        model.step()
-        assert model._arena is not None and model._arena["p"].size >= 4 * D * D + 4 * D
-        flat_step = R.RefAdam(lr=1e-3)._step(np.concatenate([g.ravel() for g in g0]))
-        pos = 0
-        for p, a, g in zip(params, p0, g0):
-            expect = a + flat_step[pos:pos + g.size].reshape(g.shape)
-            pos += g.size
-            assert op_cases.rel_err(p.values, expect) <= 1e-5
+            # ---- fused arena Adam over all 67 M parameters, fed the engine's own gradients (Adam's
+            # first step is -lr*g/(|g|+eps): entries with |g| ~ eps turn a 1e-9 gradient difference into
+            # an O(lr) step difference, so both sides get the same gradient) ---------------------------
+            p0 = [p.values.astype(np.float64) for p in params]
+            g0 = [p.grad.astype(np.float64) for p in params]
+            model.step()
+            assert model._arena is not None and model._arena["p"].size >= 4 * D * D + 4 * D
+            flat_step = R.RefAdam(lr=1e-3)._step(np.concatenate([g.ravel() for g in g0]))
+            pos = 0
+            for p, a, g in zip(params, p0, g0):
+                expect = a + flat_step[pos:pos + g.size].reshape(g.shape)
+                pos += g.size
+                assert op_cases.rel_err(p.values, expect) <= 1e-5
     finally:
-        be.TC_SPLIT = old_split
         for r in [layer for layer in mlp.layers if isinstance(layer, R.RefReLU)]:
             r.keep_override = None
 
@@ -190,13 +189,9 @@ def test_operand_split_on_adversarial_data(split, case):
         a, b = ones_tail((M, K)), ones_tail((K, N))
     a, b = a.astype(np.float32), b.astype(np.float32)
     assert np.all(np.isfinite(a)) and np.all(np.isfinite(b))
-    old, old_split = be.TC_MIN_MNK, be.TC_SPLIT
-    be.TC_MIN_MNK, be.TC_SPLIT = 0, split
-    try:
+    with gemm_route(TC_MIN_MNK=0, TC_SPLIT=split):
         assert be.use_tensor_cores(M, N, K, be.F32)
         c = be.matmul(be.from_numpy(a), be.from_numpy(b)).numpy()
-    finally:
-        be.TC_MIN_MNK, be.TC_SPLIT = old, old_split
     assert np.all(np.isfinite(c))
     err = _componentwise_err(c, a.astype(np.float64), b.astype(np.float64))
     # ("f16", the default: wide_exponents and tiny_and_huge_rows are outside its guard and are done

@@ -4,17 +4,12 @@ binary_cross_entropy_with_logits on the CPU, every argument the losses refuse, t
 scheme (two ranks over gloo with oracle compute: 1/m_global inside each rank's gradient, losses and
 gradients SUM-reduced, equal to the full batch), and the recorded-step key.  torch is test
 infrastructure here; nothing on the product path imports it."""
-import os
-import socket
-import sys
-
 import numpy as np
 import pytest
 
 import ref_losses as RL
 import ref_numpy as R
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from support import spawn_gloo
 
 
 def _close(a, b, tol=1e-12):
@@ -226,14 +221,6 @@ def test_fused_small_mlp_plan_declines_pointwise_losses():
 
 
 # ---------------------------------------------------------------------------- data parallel scheme
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
-
-
 def _dp_problem():
     """a linear model pred = x @ w on 8 rows, per loss kind"""
     rng = np.random.RandomState(11)
@@ -246,46 +233,27 @@ def _dp_problem():
     return x, w, t
 
 
-def _dp_worker(rank, world, port, queue):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
-    for p in (ROOT, os.path.join(ROOT, "oracle")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
+def _dp_worker(rank, world):
     import torch
     import torch.distributed as td
     import core._dist as dist
-    import ref_losses as RL
-    td.init_process_group("gloo", init_method="env://")
-    try:
-        x, w, t = _dp_problem()
-        lo, hi = dist.shard_bounds(x.shape[0], rank, world)    # equal shards of 4
-        out = {}
-        for kind in RL.KINDS:
-            pred = x[lo:hi] @ w
-            m_global = (hi - lo) * world
-            L, dp = RL.loss_and_grad(pred, t[kind][lo:hi], kind, delta=0.7, m=m_global)
-            loss = torch.tensor([L])
-            td.all_reduce(loss)                    # the loss node's all-reduce
-            dw = torch.tensor(x[lo:hi].T @ dp)
-            td.all_reduce(dw)                      # the gradient arena's SUM all-reduce
-            out[kind] = (float(loss[0]), dw.numpy().copy())
-        queue.put((rank, out))
-    finally:
-        td.destroy_process_group()
+    x, w, t = _dp_problem()
+    lo, hi = dist.shard_bounds(x.shape[0], rank, world)    # equal shards of 4
+    out = {}
+    for kind in RL.KINDS:
+        pred = x[lo:hi] @ w
+        m_global = (hi - lo) * world
+        L, dp = RL.loss_and_grad(pred, t[kind][lo:hi], kind, delta=0.7, m=m_global)
+        loss = torch.tensor([L])
+        td.all_reduce(loss)                    # the loss node's all-reduce
+        dw = torch.tensor(x[lo:hi].T @ dp)
+        td.all_reduce(dw)                      # the gradient arena's SUM all-reduce
+        out[kind] = (float(loss[0]), dw.numpy().copy())
+    return out
 
 
 def test_sharded_losses_equal_full_batch():
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_dp_worker, args=(r, 2, port, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    got = dict(q.get(timeout=120) for _ in range(2))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    got = spawn_gloo(_dp_worker)
     x, w, t = _dp_problem()
     for kind in RL.KINDS:
         L, dp = RL.loss_and_grad(x @ w, t[kind], kind, delta=0.7)
