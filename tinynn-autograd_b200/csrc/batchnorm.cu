@@ -26,11 +26,6 @@
 namespace tnn {
 namespace {
 
-template <typename T, int EL>
-struct alignas(sizeof(T) * EL) BnPack {
-  T v[EL];
-};
-
 constexpr int kThreads = 256;
 
 // sum the per-thread (a, b) over the TY row lanes of the CTA, in lane order; valid where ty == 0
@@ -58,7 +53,7 @@ __device__ __forceinline__ void fold_lanes(double (&a)[EL], double (&b)[EL], dou
 template <typename T, int EL, typename F>
 __device__ __forceinline__ void walk_rows(const T* __restrict__ p, const T* __restrict__ q, int64_t lo, int64_t hi,
                                           int64_t ncol, int64_t col, F&& f) {
-  using P = BnPack<T, EL>;
+  using P = Pack<T, EL>;
   const int64_t TY = blockDim.y;
   const P* __restrict__ pp = reinterpret_cast<const P*>(p);
   const P* __restrict__ qq = reinterpret_cast<const P*>(q);
@@ -146,7 +141,7 @@ bn_stats_kernel(const T* __restrict__ x, SplitArgs s, double momentum, double ep
     s1[k] = s2[k] = 0.0;
   }
   if (active)
-    walk_rows<T, EL>(x, nullptr, lo, hi, ncol, col, [&](const BnPack<T, EL>& u, const BnPack<T, EL>&) {
+    walk_rows<T, EL>(x, nullptr, lo, hi, ncol, col, [&](const Pack<T, EL>& u, const Pack<T, EL>&) {
 #pragma unroll
       for (int k = 0; k < EL; ++k) {
         const double d = (double)u.v[k] - K[k];
@@ -211,7 +206,7 @@ template <typename T, int EL>
 __global__ void __launch_bounds__(kThreads)
 bn_apply_kernel(T* __restrict__ y, const T* __restrict__ x, int64_t M, int64_t C, const T* gamma, const T* beta,
                 double* mr, const T* run_mean, const T* run_var, double eps) {
-  using P = BnPack<T, EL>;
+  using P = Pack<T, EL>;
   const int64_t ncol = C / EL;
   const int64_t col = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (col >= ncol) return;
@@ -260,7 +255,7 @@ bn_bwd_reduce_kernel(const T* __restrict__ dy, const T* __restrict__ x, SplitArg
   for (int k = 0; k < EL; ++k) a[k] = b[k] = mean[k] = r[k] = 0.0;
   if (active) {
     column_stats<T, EL>(c0, s.C, mr, (const T*)nullptr, (const T*)nullptr, 0.0, mean, r);
-    walk_rows<T, EL>(dy, x, lo, hi, ncol, col, [&](const BnPack<T, EL>& g, const BnPack<T, EL>& u) {
+    walk_rows<T, EL>(dy, x, lo, hi, ncol, col, [&](const Pack<T, EL>& g, const Pack<T, EL>& u) {
 #pragma unroll
       for (int k = 0; k < EL; ++k) {
         const double gd = (double)g.v[k];
@@ -285,7 +280,7 @@ template <typename T, int EL, bool TRAIN>
 __global__ void __launch_bounds__(kThreads)
 bn_dx_kernel(T* __restrict__ dx, const T* __restrict__ dy, const T* __restrict__ x, int64_t M, int64_t C,
              const double* mr, const T* gamma, const double* sums) {
-  using P = BnPack<T, EL>;
+  using P = Pack<T, EL>;
   const int64_t ncol = C / EL;
   const int64_t col = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (col >= ncol) return;
@@ -325,8 +320,6 @@ bn_dx_kernel(T* __restrict__ dx, const T* __restrict__ dy, const T* __restrict__
 }
 
 // ---- host side --------------------------------------------------------------------------------
-bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 struct Plan {
   int el;       // channels per access
   int tx, ty;   // CTA shape
@@ -385,11 +378,10 @@ int stats_impl(const void* x, int64_t M, int64_t C, double momentum, double eps,
   SplitArgs s;
   if (prepare_split("tnn_bn_stats", p, M, C, &s)) return 1;
   const dim3 grid((unsigned)p.gx, (unsigned)s.nsplit), block(p.tx, p.ty);
-  cudaStream_t st = ctx().stream;
-  if (p.el == 1)
-    bn_stats_kernel<T, 1><<<grid, block, 0, st>>>((const T*)x, s, momentum, eps, (T*)rm, (T*)rv, mr, part);
-  else
-    bn_stats_kernel<T, 16 / sizeof(T)><<<grid, block, 0, st>>>((const T*)x, s, momentum, eps, (T*)rm, (T*)rv, mr, part);
+  with_bool(p.el == 1, [&](auto scalar) {
+    bn_stats_kernel<T, scalar ? 1 : 16 / sizeof(T)><<<grid, block, 0, ctx().stream>>>(
+        (const T*)x, s, momentum, eps, (T*)rm, (T*)rv, mr, part);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
@@ -408,13 +400,10 @@ int apply_impl(void* y, const void* x, int64_t M, int64_t C, const void* gamma, 
                const void* rm, const void* rv, double eps) {
   const Plan p = make_plan<T>(C, aligned16(x) && aligned16(y));
   const dim3 grid((unsigned)p.gx, (unsigned)row_blocks(p, M)), block(p.tx, p.ty);
-  cudaStream_t st = ctx().stream;
-  if (p.el == 1)
-    bn_apply_kernel<T, 1><<<grid, block, 0, st>>>((T*)y, (const T*)x, M, C, (const T*)gamma, (const T*)beta, mr,
-                                                  (const T*)rm, (const T*)rv, eps);
-  else
-    bn_apply_kernel<T, 16 / sizeof(T)><<<grid, block, 0, st>>>((T*)y, (const T*)x, M, C, (const T*)gamma,
-                                                               (const T*)beta, mr, (const T*)rm, (const T*)rv, eps);
+  with_bool(p.el == 1, [&](auto scalar) {
+    bn_apply_kernel<T, scalar ? 1 : 16 / sizeof(T)><<<grid, block, 0, ctx().stream>>>(
+        (T*)y, (const T*)x, M, C, (const T*)gamma, (const T*)beta, mr, (const T*)rm, (const T*)rv, eps);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
@@ -426,36 +415,26 @@ int bwd_reduce_impl(const void* dy, const void* x, int64_t M, int64_t C, const d
   SplitArgs s;
   if (prepare_split("tnn_bn_bwd_reduce", p, M, C, &s)) return 1;
   const dim3 grid((unsigned)p.gx, (unsigned)s.nsplit), block(p.tx, p.ty);
-  cudaStream_t st = ctx().stream;
-  if (p.el == 1)
-    bn_bwd_reduce_kernel<T, 1><<<grid, block, 0, st>>>((const T*)dy, (const T*)x, s, mr, sums, (T*)dgamma,
-                                                       acc_gamma, (T*)dbeta, acc_beta);
-  else
-    bn_bwd_reduce_kernel<T, 16 / sizeof(T)><<<grid, block, 0, st>>>((const T*)dy, (const T*)x, s, mr, sums,
-                                                                    (T*)dgamma, acc_gamma, (T*)dbeta, acc_beta);
+  with_bool(p.el == 1, [&](auto scalar) {
+    bn_bwd_reduce_kernel<T, scalar ? 1 : 16 / sizeof(T)><<<grid, block, 0, ctx().stream>>>(
+        (const T*)dy, (const T*)x, s, mr, sums, (T*)dgamma, acc_gamma, (T*)dbeta, acc_beta);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
 
-template <typename T, int EL>
-void launch_dx(dim3 grid, dim3 block, void* dx, const void* dy, const void* x, int64_t M, int64_t C,
-               const double* mr, const void* gamma, const double* sums) {
-  cudaStream_t st = ctx().stream;
-  if (sums)
-    bn_dx_kernel<T, EL, true><<<grid, block, 0, st>>>((T*)dx, (const T*)dy, (const T*)x, M, C, mr, (const T*)gamma,
-                                                      sums);
-  else
-    bn_dx_kernel<T, EL, false><<<grid, block, 0, st>>>((T*)dx, (const T*)dy, (const T*)x, M, C, mr,
-                                                       (const T*)gamma, sums);
-}
-
+// TRAIN when the backward sums are given
 template <typename T>
 int dx_impl(void* dx, const void* dy, const void* x, int64_t M, int64_t C, const double* mr, const void* gamma,
             const double* sums) {
   const Plan p = make_plan<T>(C, aligned16(dx) && aligned16(dy) && (!sums || aligned16(x)));
   const dim3 grid((unsigned)p.gx, (unsigned)row_blocks(p, M)), block(p.tx, p.ty);
-  if (p.el == 1) launch_dx<T, 1>(grid, block, dx, dy, x, M, C, mr, gamma, sums);
-  else launch_dx<T, 16 / sizeof(T)>(grid, block, dx, dy, x, M, C, mr, gamma, sums);
+  with_bool(p.el == 1, [&](auto scalar) {
+    with_bool(sums != nullptr, [&](auto train) {
+      bn_dx_kernel<T, scalar ? 1 : 16 / sizeof(T), train><<<grid, block, 0, ctx().stream>>>(
+          (T*)dx, (const T*)dy, (const T*)x, M, C, mr, (const T*)gamma, sums);
+    });
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
@@ -470,13 +449,6 @@ int check_shape(const char* name, int64_t M, int64_t C) {
 
 using namespace tnn;
 
-#define TNN_BN_DISPATCH(name, call)                                  \
-  do {                                                               \
-    if (dtype == TNN_F32) return call(float);                        \
-    if (dtype == TNN_F64) return call(double);                       \
-    TNN_FAIL(name ": bad dtype");                                    \
-  } while (0)
-
 extern "C" {
 
 int tnn_bn_stats(int dtype, const void* x, int64_t M, int64_t C, double momentum, double eps, void* running_mean,
@@ -484,9 +456,9 @@ int tnn_bn_stats(int dtype, const void* x, int64_t M, int64_t C, double momentum
   TNN_REQUIRE_INIT();
   if (check_shape("tnn_bn_stats", M, C)) return 1;
   if (!part && M < 2) TNN_FAIL("tnn_bn_stats: the unbiased running variance needs at least two rows");
-#define TNN_BN_CALL(T) stats_impl<T>(x, M, C, momentum, eps, running_mean, running_var, mr, part)
-  TNN_BN_DISPATCH("tnn_bn_stats", TNN_BN_CALL);
-#undef TNN_BN_CALL
+  return with_float_type(dtype, "tnn_bn_stats", [&](auto tag) {
+    return stats_impl<decltype(tag)>(x, M, C, momentum, eps, running_mean, running_var, mr, part);
+  });
 }
 
 int tnn_bn_merge(int dtype, const double* gathered, int world, int64_t C, double momentum, double eps,
@@ -494,9 +466,9 @@ int tnn_bn_merge(int dtype, const double* gathered, int world, int64_t C, double
   TNN_REQUIRE_INIT();
   if (check_shape("tnn_bn_merge", 0, C)) return 1;
   if (world < 1) TNN_FAIL("tnn_bn_merge: bad world size");
-#define TNN_BN_CALL(T) merge_impl<T>(gathered, world, C, momentum, eps, running_mean, running_var, mr)
-  TNN_BN_DISPATCH("tnn_bn_merge", TNN_BN_CALL);
-#undef TNN_BN_CALL
+  return with_float_type(dtype, "tnn_bn_merge", [&](auto tag) {
+    return merge_impl<decltype(tag)>(gathered, world, C, momentum, eps, running_mean, running_var, mr);
+  });
 }
 
 int tnn_bn_apply(int dtype, void* y, const void* x, int64_t M, int64_t C, const void* gamma, const void* beta,
@@ -504,18 +476,18 @@ int tnn_bn_apply(int dtype, void* y, const void* x, int64_t M, int64_t C, const 
   TNN_REQUIRE_INIT();
   if (check_shape("tnn_bn_apply", M, C)) return 1;
   if (M == 0) return 0;
-#define TNN_BN_CALL(T) apply_impl<T>(y, x, M, C, gamma, beta, mr, running_mean, running_var, eps)
-  TNN_BN_DISPATCH("tnn_bn_apply", TNN_BN_CALL);
-#undef TNN_BN_CALL
+  return with_float_type(dtype, "tnn_bn_apply", [&](auto tag) {
+    return apply_impl<decltype(tag)>(y, x, M, C, gamma, beta, mr, running_mean, running_var, eps);
+  });
 }
 
 int tnn_bn_bwd_reduce(int dtype, const void* dy, const void* x, int64_t M, int64_t C, const double* mr,
                       double* sums, void* dgamma, int acc_gamma, void* dbeta, int acc_beta) {
   TNN_REQUIRE_INIT();
   if (check_shape("tnn_bn_bwd_reduce", M, C)) return 1;
-#define TNN_BN_CALL(T) bwd_reduce_impl<T>(dy, x, M, C, mr, sums, dgamma, acc_gamma, dbeta, acc_beta)
-  TNN_BN_DISPATCH("tnn_bn_bwd_reduce", TNN_BN_CALL);
-#undef TNN_BN_CALL
+  return with_float_type(dtype, "tnn_bn_bwd_reduce", [&](auto tag) {
+    return bwd_reduce_impl<decltype(tag)>(dy, x, M, C, mr, sums, dgamma, acc_gamma, dbeta, acc_beta);
+  });
 }
 
 int tnn_bn_dx(int dtype, void* dx, const void* dy, const void* x, int64_t M, int64_t C, const double* mr,
@@ -523,9 +495,9 @@ int tnn_bn_dx(int dtype, void* dx, const void* dy, const void* x, int64_t M, int
   TNN_REQUIRE_INIT();
   if (check_shape("tnn_bn_dx", M, C)) return 1;
   if (M == 0) return 0;
-#define TNN_BN_CALL(T) dx_impl<T>(dx, dy, x, M, C, mr, gamma, sums)
-  TNN_BN_DISPATCH("tnn_bn_dx", TNN_BN_CALL);
-#undef TNN_BN_CALL
+  return with_float_type(dtype, "tnn_bn_dx", [&](auto tag) {
+    return dx_impl<decltype(tag)>(dx, dy, x, M, C, mr, gamma, sums);
+  });
 }
 
 }  // extern "C"

@@ -34,6 +34,13 @@ struct Api {
   const char* (*GetErrorString)(ncclResult_t) = nullptr;
 };
 
+// NCCL's element type for a dtype code, -1 for any other code
+static int nccl_type(int dtype) {
+  if (dtype == TNN_F32) return ncclFloat32;
+  if (dtype == TNN_F64) return ncclFloat64;
+  return -1;
+}
+
 static Api g_api;
 static ncclComm_t g_comm = nullptr;
 static int g_world = 1, g_rank = 0;
@@ -119,9 +126,9 @@ int tnn_nccl_destroy(void) {
 int tnn_allreduce_sum(int dtype, void* buf, int64_t n) {
   TNN_REQUIRE_INIT();
   if (!g_comm) TNN_FAIL("tnn_allreduce_sum: call tnn_nccl_init first");
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("tnn_allreduce_sum: bad dtype");
-  TNN_NCCL(g_api.AllReduce(buf, buf, (size_t)n, dtype == TNN_F32 ? ncclFloat32 : ncclFloat64, ncclSum,
-                           g_comm, ctx().stream));
+  const int type = nccl_type(dtype);
+  if (type < 0) TNN_FAIL("tnn_allreduce_sum: bad dtype");
+  TNN_NCCL(g_api.AllReduce(buf, buf, (size_t)n, type, ncclSum, g_comm, ctx().stream));
   ctx().launches++;
   return 0;
 }
@@ -152,9 +159,9 @@ int tnn_compute_wait_comm(void) {
 int tnn_allreduce_sum_comm(int dtype, void* buf, int64_t n) {
   TNN_REQUIRE_INIT();
   if (!g_comm) TNN_FAIL("tnn_allreduce_sum_comm: call tnn_nccl_init first");
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("tnn_allreduce_sum_comm: bad dtype");
-  TNN_NCCL(g_api.AllReduce(buf, buf, (size_t)n, dtype == TNN_F32 ? ncclFloat32 : ncclFloat64, ncclSum,
-                           g_comm, ctx().comm_stream));
+  const int type = nccl_type(dtype);
+  if (type < 0) TNN_FAIL("tnn_allreduce_sum_comm: bad dtype");
+  TNN_NCCL(g_api.AllReduce(buf, buf, (size_t)n, type, ncclSum, g_comm, ctx().comm_stream));
   ctx().launches++;
   return 0;
 }
@@ -162,9 +169,9 @@ int tnn_allreduce_sum_comm(int dtype, void* buf, int64_t n) {
 int tnn_allgather(int dtype, void* recv, const void* send, int64_t n_per_rank) {
   TNN_REQUIRE_INIT();
   if (!g_comm) TNN_FAIL("tnn_allgather: call tnn_nccl_init first");
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("tnn_allgather: bad dtype");
-  TNN_NCCL(g_api.AllGather(send, recv, (size_t)n_per_rank, dtype == TNN_F32 ? ncclFloat32 : ncclFloat64,
-                           g_comm, ctx().stream));
+  const int type = nccl_type(dtype);
+  if (type < 0) TNN_FAIL("tnn_allgather: bad dtype");
+  TNN_NCCL(g_api.AllGather(send, recv, (size_t)n_per_rank, type, g_comm, ctx().stream));
   ctx().launches++;
   return 0;
 }

@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string>
+#include <type_traits>
 
 #include "../../include/tnn_b200.h"
 
@@ -131,16 +132,29 @@ inline cudaError_t launch_small(void (*kernel)(KArgs...), dim3 grid, dim3 block,
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-template <typename T>
-struct Vec4;
-template <>
-struct Vec4<float> {
-  using type = float4;
+// EL consecutive elements moved as one access (16 bytes for EL = 16 / sizeof(T))
+template <typename T, int EL>
+struct alignas(sizeof(T) * EL) Pack {
+  T v[EL];
 };
-template <>
-struct Vec4<double> {
-  using type = double4;
-};
+
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// The C++ type of a float dtype code: f(float{}) for TNN_F32, f(double{}) for TNN_F64.  Any other
+// code fails with a message naming the entry point `name`.  f returns int like the entry points.
+template <typename F>
+inline int with_float_type(int dtype, const char* name, F&& f) {
+  if (dtype == TNN_F32) return f(float{});
+  if (dtype == TNN_F64) return f(double{});
+  TNN_FAIL(std::string(name) + ": bad dtype");
+}
+
+// A runtime choice (a vector path, a phase) as a template argument: f(std::true_type{}) or
+// f(std::false_type{}), whose parameter converts to a bool template argument
+template <typename F>
+inline decltype(auto) with_bool(bool flag, F&& f) {
+  return flag ? f(std::true_type{}) : f(std::false_type{});
+}
 
 __host__ __device__ inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

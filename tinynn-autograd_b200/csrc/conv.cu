@@ -9,16 +9,6 @@
 
 namespace tnn {
 
-// EL consecutive elements moved as one access (16 bytes for EL = 16 / sizeof(T))
-template <typename T, int EL>
-struct alignas(sizeof(T) * EL) Pack {
-  T v[EL];
-};
-template <int EL>
-struct alignas(4 * EL) IPack {
-  int32_t v[EL];
-};
-
 struct Geom {
   int64_t N, H, W, C;   // input (NHWC)
   int64_t KH, KW;       // window
@@ -106,7 +96,7 @@ template <typename T, int EL>
 __global__ void __launch_bounds__(256)
 maxpool_fwd_kernel(T* __restrict__ y, int32_t* __restrict__ arg, const T* __restrict__ x, Geom g) {
   using P = Pack<T, EL>;
-  using I = IPack<EL>;
+  using I = Pack<int32_t, EL>;
   const int64_t Cv = g.C / EL;
   const int64_t n_vec = g.N * g.OH * g.OW * Cv;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -154,7 +144,7 @@ template <typename T, int EL>
 __global__ void __launch_bounds__(256) maxpool_bwd_kernel(T* __restrict__ dx, const T* __restrict__ dy,
                                                           const int32_t* __restrict__ arg, Geom g) {
   using P = Pack<T, EL>;
-  using I = IPack<EL>;
+  using I = Pack<int32_t, EL>;
   const int64_t Cv = g.C / EL;
   const int64_t n_vec = g.N * g.H * g.W * Cv;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -191,8 +181,6 @@ __global__ void __launch_bounds__(256) maxpool_bwd_kernel(T* __restrict__ dx, co
   }
 }
 
-static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 static int check_geom(const char* name, const Geom& g) {
   if (g.N < 0 || g.H < 0 || g.W < 0 || g.C <= 0 || g.KH <= 0 || g.KW <= 0 || g.SH <= 0 || g.SW <= 0 ||
       g.PH0 < 0 || g.PW0 < 0 || g.PH0 >= g.KH || g.PW0 >= g.KW || g.OH < 0 || g.OW < 0)
@@ -205,44 +193,21 @@ static int check_geom(const char* name, const Geom& g) {
   return 0;
 }
 
-// K(T, EL) is launched with EL = 16 / sizeof(T) when C is a multiple of it and every pointer is
-// 16-byte aligned, with EL = 1 otherwise
-template <typename T, template <typename, int> class Launch, typename... Args>
-static int dispatch_vec(bool vec_ok, int64_t n_elems, Args... args) {
-  constexpr int V = 16 / sizeof(T);
-  const int64_t work = vec_ok ? n_elems / V : n_elems;
-  if (work == 0) return 0;
-  const int grid = ew_grid(work, 256);
-  if (vec_ok) Launch<T, V>::run(grid, args...);
-  else Launch<T, 1>::run(grid, args...);
-  TNN_POST_LAUNCH();
-  return 0;
+// Launches f(T{}, std::integral_constant<int, EL>{}, grid) over n elements: EL = 16 / sizeof(T) when C
+// is a multiple of it and every pointer is 16-byte aligned, EL = 1 otherwise
+template <typename F>
+static int launch_vec(const char* name, int dtype, bool ptrs_aligned, const Geom& g, int64_t n, F&& f) {
+  return with_float_type(dtype, name, [&](auto tag) {
+    constexpr int V = 16 / sizeof(tag);
+    const bool vec = ptrs_aligned && g.C % V == 0;
+    const int64_t work = vec ? n / V : n;
+    if (work == 0) return 0;
+    const int grid = ew_grid(work, 256);
+    with_bool(vec, [&](auto v) { f(tag, std::integral_constant<int, v ? V : 1>{}, grid); });
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
-
-template <typename T, int EL>
-struct Im2col {
-  static void run(int grid, void* col, const void* x, Geom g) {
-    im2col_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)col, (const T*)x, g);
-  }
-};
-template <typename T, int EL>
-struct Col2im {
-  static void run(int grid, void* dx, const void* dcol, Geom g) {
-    col2im_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)dx, (const T*)dcol, g);
-  }
-};
-template <typename T, int EL>
-struct PoolFwd {
-  static void run(int grid, void* y, int32_t* arg, const void* x, Geom g) {
-    maxpool_fwd_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)y, arg, (const T*)x, g);
-  }
-};
-template <typename T, int EL>
-struct PoolBwd {
-  static void run(int grid, void* dx, const void* dy, const int32_t* arg, Geom g) {
-    maxpool_bwd_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)dx, (const T*)dy, arg, g);
-  }
-};
 
 static Geom make_geom(int64_t N, int64_t H, int64_t W, int64_t C, int64_t KH, int64_t KW, int64_t SH,
                       int64_t SW, int64_t PH0, int64_t PW0, int64_t OH, int64_t OW) {
@@ -263,11 +228,11 @@ int tnn_im2col(int dtype, void* col, const void* x, int64_t N, int64_t H, int64_
   TNN_REQUIRE_INIT();
   const Geom g = make_geom(N, H, W, C, KH, KW, SH, SW, PH0, PW0, OH, OW);
   if (check_geom("tnn_im2col", g)) return 1;
-  const int64_t n = N * OH * OW * KH * KW * C;
-  const bool vec = aligned16(col) && aligned16(x);
-  if (dtype == TNN_F32) return dispatch_vec<float, Im2col>(vec && C % 4 == 0, n, col, x, g);
-  if (dtype == TNN_F64) return dispatch_vec<double, Im2col>(vec && C % 2 == 0, n, col, x, g);
-  TNN_FAIL("tnn_im2col: bad dtype");
+  return launch_vec("tnn_im2col", dtype, aligned16(col) && aligned16(x), g, N * OH * OW * KH * KW * C,
+                    [&](auto tag, auto EL, int grid) {
+                      using T = decltype(tag);
+                      im2col_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)col, (const T*)x, g);
+                    });
 }
 
 int tnn_col2im(int dtype, void* dx, const void* dcol, int64_t N, int64_t H, int64_t W, int64_t C, int64_t KH,
@@ -275,11 +240,11 @@ int tnn_col2im(int dtype, void* dx, const void* dcol, int64_t N, int64_t H, int6
   TNN_REQUIRE_INIT();
   const Geom g = make_geom(N, H, W, C, KH, KW, SH, SW, PH0, PW0, OH, OW);
   if (check_geom("tnn_col2im", g)) return 1;
-  const int64_t n = N * H * W * C;
-  const bool vec = aligned16(dx) && aligned16(dcol);
-  if (dtype == TNN_F32) return dispatch_vec<float, Col2im>(vec && C % 4 == 0, n, dx, dcol, g);
-  if (dtype == TNN_F64) return dispatch_vec<double, Col2im>(vec && C % 2 == 0, n, dx, dcol, g);
-  TNN_FAIL("tnn_col2im: bad dtype");
+  return launch_vec("tnn_col2im", dtype, aligned16(dx) && aligned16(dcol), g, N * H * W * C,
+                    [&](auto tag, auto EL, int grid) {
+                      using T = decltype(tag);
+                      col2im_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)dx, (const T*)dcol, g);
+                    });
 }
 
 int tnn_maxpool_fwd(int dtype, void* y, int32_t* arg, const void* x, int64_t N, int64_t H, int64_t W,
@@ -288,11 +253,11 @@ int tnn_maxpool_fwd(int dtype, void* y, int32_t* arg, const void* x, int64_t N, 
   TNN_REQUIRE_INIT();
   const Geom g = make_geom(N, H, W, C, PH, PW, SH, SW, PH0, PW0, OH, OW);
   if (check_geom("tnn_maxpool_fwd", g)) return 1;
-  const int64_t n = N * OH * OW * C;
-  const bool vec = aligned16(y) && aligned16(arg) && aligned16(x);
-  if (dtype == TNN_F32) return dispatch_vec<float, PoolFwd>(vec && C % 4 == 0, n, y, arg, x, g);
-  if (dtype == TNN_F64) return dispatch_vec<double, PoolFwd>(vec && C % 2 == 0, n, y, arg, x, g);
-  TNN_FAIL("tnn_maxpool_fwd: bad dtype");
+  return launch_vec("tnn_maxpool_fwd", dtype, aligned16(y) && aligned16(arg) && aligned16(x), g, N * OH * OW * C,
+                    [&](auto tag, auto EL, int grid) {
+                      using T = decltype(tag);
+                      maxpool_fwd_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)y, arg, (const T*)x, g);
+                    });
 }
 
 int tnn_maxpool_bwd(int dtype, void* dx, const void* dy, const int32_t* arg, int64_t N, int64_t H, int64_t W,
@@ -301,11 +266,11 @@ int tnn_maxpool_bwd(int dtype, void* dx, const void* dy, const int32_t* arg, int
   TNN_REQUIRE_INIT();
   const Geom g = make_geom(N, H, W, C, PH, PW, SH, SW, PH0, PW0, OH, OW);
   if (check_geom("tnn_maxpool_bwd", g)) return 1;
-  const int64_t n = N * H * W * C;
-  const bool vec = aligned16(dx) && aligned16(dy) && aligned16(arg);
-  if (dtype == TNN_F32) return dispatch_vec<float, PoolBwd>(vec && C % 4 == 0, n, dx, dy, arg, g);
-  if (dtype == TNN_F64) return dispatch_vec<double, PoolBwd>(vec && C % 2 == 0, n, dx, dy, arg, g);
-  TNN_FAIL("tnn_maxpool_bwd: bad dtype");
+  return launch_vec("tnn_maxpool_bwd", dtype, aligned16(dx) && aligned16(dy) && aligned16(arg), g, N * H * W * C,
+                    [&](auto tag, auto EL, int grid) {
+                      using T = decltype(tag);
+                      maxpool_bwd_kernel<T, EL><<<grid, 256, 0, ctx().stream>>>((T*)dx, (const T*)dy, arg, g);
+                    });
 }
 
 }  // extern "C"

@@ -63,41 +63,14 @@ __host__ __device__ constexpr int op_arity(int op) {
   return (op >= 20 && op < 40) ? 3 : ((op >= 40 && op != TNN_OP_CLIP_BWD && op != TNN_OP_RECIP_MUL) ? 1 : 2);
 }
 
-template <typename T, int VEC>
-struct VecT;
-template <>
-struct VecT<float, 4> {
-  using type = float4;
-};
-template <>
-struct VecT<double, 2> {
-  using type = double2;
-};
-template <typename T>
-struct VecW;
-template <>
-struct VecW<float> {
-  static constexpr int value = 4;
-};
-template <>
-struct VecW<double> {
-  static constexpr int value = 2;
-};
-
-template <typename T, int VEC>
-union VecU {
-  typename VecT<T, VEC>::type v;
-  T e[VEC];
-};
-
 // ---- flat ------------------------------------------------------------------------------------
 template <int OP, typename T>
 __global__ void __launch_bounds__(256)
 ew_flat_vec_kernel(T* out, const T* x, const T* y, const T* z, int64_t n, int scalar_mask,
                    EwParams<T> p) {
-  constexpr int VEC = VecW<T>::value;
+  constexpr int VEC = 16 / sizeof(T);
   constexpr int AR = op_arity(OP);
-  using V = typename VecT<T, VEC>::type;
+  using V = Pack<T, VEC>;
   const int64_t nv = n / VEC;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   const bool xs = scalar_mask & 1, ys = scalar_mask & 2, zs = scalar_mask & 4;
@@ -106,14 +79,14 @@ ew_flat_vec_kernel(T* out, const T* x, const T* y, const T* z, int64_t n, int sc
   T z0 = (AR >= 3 && zs) ? z[0] : T(0);
   constexpr int U = AR == 1 ? 4 : 2;   // independent vector loads in flight per operand and thread
   for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < nv; i0 += U * stride) {
-    VecU<T, VEC> a[U], b[U], c[U], r;
+    V a[U], b[U], c[U], r;
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int64_t i = i0 + u * stride;
       if (i < nv) {
-        if (!xs) a[u].v = reinterpret_cast<const V*>(x)[i];
-        if (AR >= 2 && !ys) b[u].v = reinterpret_cast<const V*>(y)[i];
-        if (AR >= 3 && !zs) c[u].v = reinterpret_cast<const V*>(z)[i];
+        if (!xs) a[u] = reinterpret_cast<const V*>(x)[i];
+        if (AR >= 2 && !ys) b[u] = reinterpret_cast<const V*>(y)[i];
+        if (AR >= 3 && !zs) c[u] = reinterpret_cast<const V*>(z)[i];
       }
     }
 #pragma unroll
@@ -122,9 +95,9 @@ ew_flat_vec_kernel(T* out, const T* x, const T* y, const T* z, int64_t n, int sc
       if (i < nv) {
 #pragma unroll
         for (int k = 0; k < VEC; ++k)
-          r.e[k] = ew_apply<OP, T>(xs ? x0 : a[u].e[k], (AR >= 2) ? (ys ? y0 : b[u].e[k]) : T(0),
-                                   (AR >= 3) ? (zs ? z0 : c[u].e[k]) : T(0), p);
-        reinterpret_cast<V*>(out)[i] = r.v;
+          r.v[k] = ew_apply<OP, T>(xs ? x0 : a[u].v[k], (AR >= 2) ? (ys ? y0 : b[u].v[k]) : T(0),
+                                   (AR >= 3) ? (zs ? z0 : c[u].v[k]) : T(0), p);
+        reinterpret_cast<V*>(out)[i] = r;
       }
     }
   }
@@ -156,7 +129,7 @@ struct RowsArgs {
 template <int OP, typename T, bool VECTOR>
 __global__ void __launch_bounds__(256)
 ew_rows_kernel(T* out, const T* x, const T* y, const T* z, RowsArgs a, EwParams<T> p) {
-  constexpr int VEC = VECTOR ? VecW<T>::value : 1;
+  constexpr int VEC = VECTOR ? 16 / sizeof(T) : 1;
   constexpr int AR = op_arity(OP);
   const int64_t ncol = a.C / VEC;  // VECTOR path requires C % VEC == 0
   const int64_t col = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -185,19 +158,18 @@ ew_rows_kernel(T* out, const T* x, const T* y, const T* z, RowsArgs a, EwParams<
 #pragma unroll
         for (int k = 0; k < VEC; ++k) v[o][k] = s;
       } else if (VECTOR) {
-        VecU<T, VecW<T>::value> u;
-        u.v = *reinterpret_cast<const typename VecT<T, VecW<T>::value>::type*>(ptr[o] + r * a.rs[o] + c0);
+        const Pack<T, VEC> u = *reinterpret_cast<const Pack<T, VEC>*>(ptr[o] + r * a.rs[o] + c0);
 #pragma unroll
-        for (int k = 0; k < VEC; ++k) v[o][k] = u.e[k];
+        for (int k = 0; k < VEC; ++k) v[o][k] = u.v[k];
       } else {
         v[o][0] = ptr[o][r * a.rs[o] + c0];
       }
     }
     if (VECTOR) {
-      VecU<T, VecW<T>::value> u;
+      Pack<T, VEC> u;
 #pragma unroll
-      for (int k = 0; k < VEC; ++k) u.e[k] = ew_apply<OP, T>(v[0][k], v[1][k], v[2][k], p);
-      *reinterpret_cast<typename VecT<T, VecW<T>::value>::type*>(out + r * a.C + c0) = u.v;
+      for (int k = 0; k < VEC; ++k) u.v[k] = ew_apply<OP, T>(v[0][k], v[1][k], v[2][k], p);
+      *reinterpret_cast<Pack<T, VEC>*>(out + r * a.C + c0) = u;
     } else {
       out[r * a.C + c0] = ew_apply<OP, T>(v[0][0], v[1][0], v[2][0], p);
     }
@@ -232,14 +204,12 @@ ew_nd_kernel(T* out, const T* x, const T* y, const T* z, int64_t n, NdArgs a, Ew
 }
 
 // ---- host dispatch -------------------------------------------------------------------------
-static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 template <int OP, typename T>
 static int launch_flat(T* out, const T* x, const T* y, const T* z, int64_t n, int scalar_mask,
                        EwParams<T> p) {
   if (n <= 0) return 0;
   constexpr int AR = op_arity(OP);
-  constexpr int VEC = VecW<T>::value;
+  constexpr int VEC = 16 / sizeof(T);
   bool vec_ok = aligned16(out) && n >= VEC;
   if (!(scalar_mask & 1)) vec_ok = vec_ok && aligned16(x);
   if (AR >= 2 && !(scalar_mask & 2)) vec_ok = vec_ok && aligned16(y);
@@ -260,22 +230,18 @@ template <int OP, typename T>
 static int launch_rows(T* out, const T* x, const T* y, const T* z, const RowsArgs& a,
                        EwParams<T> p) {
   constexpr int AR = op_arity(OP);
-  constexpr int VEC = VecW<T>::value;
+  constexpr int VEC = 16 / sizeof(T);
   const T* ptr[3] = {x, y, z};
   bool vec_ok = (a.C % VEC == 0) && aligned16(out);
   for (int o = 0; o < AR; ++o)
     if (a.cs[o] == 1) vec_ok = vec_ok && aligned16(ptr[o]) && (a.rs[o] % VEC == 0);
-  cudaStream_t s = ctx().stream;
   int64_t ncol = vec_ok ? a.C / VEC : a.C;
   int gx = (int)ceil_div(ncol, 256);
   int64_t want_y = ceil_div((int64_t)ctx().sm_count * 8, gx);
   int gy = (int)(want_y < 1 ? 1 : (want_y > a.R ? a.R : want_y));
   if (gy > 65535) gy = 65535;
   dim3 grid(gx, gy);
-  if (vec_ok)
-    ew_rows_kernel<OP, T, true><<<grid, 256, 0, s>>>(out, x, y, z, a, p);
-  else
-    ew_rows_kernel<OP, T, false><<<grid, 256, 0, s>>>(out, x, y, z, a, p);
+  with_bool(vec_ok, [&](auto vec) { ew_rows_kernel<OP, T, vec><<<grid, 256, 0, ctx().stream>>>(out, x, y, z, a, p); });
   TNN_POST_LAUNCH();
   return 0;
 }
@@ -385,44 +351,51 @@ __global__ void __launch_bounds__(256) fill_kernel(T* dst, T v, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) dst[i] = v;
 }
 
+// f(std::integral_constant<int, OP>{}) for an op code; any other code fails, naming the entry point
+#define TNN_EW_CASE(OPC) \
+  case OPC:              \
+    return f(std::integral_constant<int, OPC>{});
+
+template <typename F>
+static int with_op(int op, const char* name, F&& f) {
+  switch (op) {
+    TNN_EW_CASE(TNN_OP_ADD)
+    TNN_EW_CASE(TNN_OP_SUB)
+    TNN_EW_CASE(TNN_OP_MUL)
+    TNN_EW_CASE(TNN_OP_DIV)
+    TNN_EW_CASE(TNN_OP_POW)
+    TNN_EW_CASE(TNN_OP_MAXIMUM)
+    TNN_EW_CASE(TNN_OP_MINIMUM)
+    TNN_EW_CASE(TNN_OP_GE)
+    TNN_EW_CASE(TNN_OP_GT)
+    TNN_EW_CASE(TNN_OP_LE)
+    TNN_EW_CASE(TNN_OP_LT)
+    TNN_EW_CASE(TNN_OP_EQ)
+    TNN_EW_CASE(TNN_OP_MUL_GE)
+    TNN_EW_CASE(TNN_OP_MUL_GT)
+    TNN_EW_CASE(TNN_OP_MUL_LE)
+    TNN_EW_CASE(TNN_OP_MUL_LT)
+    TNN_EW_CASE(TNN_OP_MUL_EQ)
+    TNN_EW_CASE(TNN_OP_DIV_BWD_B)
+    TNN_EW_CASE(TNN_OP_POW_BWD_A)
+    TNN_EW_CASE(TNN_OP_POW_BWD_B)
+    TNN_EW_CASE(TNN_OP_NEG)
+    TNN_EW_CASE(TNN_OP_EXP)
+    TNN_EW_CASE(TNN_OP_LOG)
+    TNN_EW_CASE(TNN_OP_COPY)
+    TNN_EW_CASE(TNN_OP_CLIP)
+    TNN_EW_CASE(TNN_OP_SCALE)
+    TNN_EW_CASE(TNN_OP_CLIP_BWD)
+    TNN_EW_CASE(TNN_OP_RECIP_MUL)
+    default:
+      TNN_FAIL(std::string(name) + ": unknown op code " + std::to_string(op));
+  }
+}
+#undef TNN_EW_CASE
+
 }  // namespace tnn
 
 using namespace tnn;
-
-#define TNN_EW_CASE(OPC, CALL)                                        \
-  case OPC:                                                           \
-    if (dtype == TNN_F32) return CALL(OPC, float);                    \
-    return CALL(OPC, double);
-
-#define TNN_EW_ALL_OPS(CALL)               \
-  TNN_EW_CASE(TNN_OP_ADD, CALL)            \
-  TNN_EW_CASE(TNN_OP_SUB, CALL)            \
-  TNN_EW_CASE(TNN_OP_MUL, CALL)            \
-  TNN_EW_CASE(TNN_OP_DIV, CALL)            \
-  TNN_EW_CASE(TNN_OP_POW, CALL)            \
-  TNN_EW_CASE(TNN_OP_MAXIMUM, CALL)        \
-  TNN_EW_CASE(TNN_OP_MINIMUM, CALL)        \
-  TNN_EW_CASE(TNN_OP_GE, CALL)             \
-  TNN_EW_CASE(TNN_OP_GT, CALL)             \
-  TNN_EW_CASE(TNN_OP_LE, CALL)             \
-  TNN_EW_CASE(TNN_OP_LT, CALL)             \
-  TNN_EW_CASE(TNN_OP_EQ, CALL)             \
-  TNN_EW_CASE(TNN_OP_MUL_GE, CALL)         \
-  TNN_EW_CASE(TNN_OP_MUL_GT, CALL)         \
-  TNN_EW_CASE(TNN_OP_MUL_LE, CALL)         \
-  TNN_EW_CASE(TNN_OP_MUL_LT, CALL)         \
-  TNN_EW_CASE(TNN_OP_MUL_EQ, CALL)         \
-  TNN_EW_CASE(TNN_OP_DIV_BWD_B, CALL)      \
-  TNN_EW_CASE(TNN_OP_POW_BWD_A, CALL)      \
-  TNN_EW_CASE(TNN_OP_POW_BWD_B, CALL)      \
-  TNN_EW_CASE(TNN_OP_NEG, CALL)            \
-  TNN_EW_CASE(TNN_OP_EXP, CALL)            \
-  TNN_EW_CASE(TNN_OP_LOG, CALL)            \
-  TNN_EW_CASE(TNN_OP_COPY, CALL)           \
-  TNN_EW_CASE(TNN_OP_CLIP, CALL)           \
-  TNN_EW_CASE(TNN_OP_SCALE, CALL)          \
-  TNN_EW_CASE(TNN_OP_CLIP_BWD, CALL)       \
-  TNN_EW_CASE(TNN_OP_RECIP_MUL, CALL)
 
 extern "C" {
 
@@ -430,29 +403,22 @@ int tnn_ew(int op, int dtype, void* out, const void* x, const void* y, const voi
            const int64_t* shape, const int64_t* xs, const int64_t* ys, const int64_t* zs,
            double p0, double p1, int flags) {
   TNN_REQUIRE_INIT();
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("tnn_ew: dtype must be TNN_F32 or TNN_F64");
   if (ndim < 0 || ndim > TNN_MAX_DIMS) TNN_FAIL("tnn_ew: rank above TNN_MAX_DIMS");
-#define CALL_ND(OPC, T) ew_dispatch<OPC, T>(out, x, y, z, ndim, shape, xs, ys, zs, p0, p1, flags)
-  switch (op) {
-    TNN_EW_ALL_OPS(CALL_ND)
-    default:
-      TNN_FAIL("tnn_ew: unknown op code " + std::to_string(op));
-  }
-#undef CALL_ND
+  return with_op(op, "tnn_ew", [&](auto OP) {
+    return with_float_type(dtype, "tnn_ew", [&](auto tag) {
+      return ew_dispatch<OP, decltype(tag)>(out, x, y, z, ndim, shape, xs, ys, zs, p0, p1, flags);
+    });
+  });
 }
 
 int tnn_ew_flat(int op, int dtype, void* out, const void* x, const void* y, const void* z,
                 int64_t n, int scalar_mask, double p0, double p1, int flags) {
   TNN_REQUIRE_INIT();
-  if (dtype != TNN_F32 && dtype != TNN_F64)
-    TNN_FAIL("tnn_ew_flat: dtype must be TNN_F32 or TNN_F64");
-#define CALL_FLAT(OPC, T) ew_flat_dispatch<OPC, T>(out, x, y, z, n, scalar_mask, p0, p1, flags)
-  switch (op) {
-    TNN_EW_ALL_OPS(CALL_FLAT)
-    default:
-      TNN_FAIL("tnn_ew_flat: unknown op code " + std::to_string(op));
-  }
-#undef CALL_FLAT
+  return with_op(op, "tnn_ew_flat", [&](auto OP) {
+    return with_float_type(dtype, "tnn_ew_flat", [&](auto tag) {
+      return ew_flat_dispatch<OP, decltype(tag)>(out, x, y, z, n, scalar_mask, p0, p1, flags);
+    });
+  });
 }
 
 int tnn_cast(int dst_dtype, void* dst, int src_dtype, const void* src, int64_t n) {
@@ -475,16 +441,12 @@ int tnn_cast(int dst_dtype, void* dst, int src_dtype, const void* src, int64_t n
 int tnn_fill(int dtype, void* dst, double value, int64_t n) {
   TNN_REQUIRE_INIT();
   if (n <= 0) return 0;
-  int grid = ew_grid(n, 256);
-  cudaStream_t s = ctx().stream;
-  if (dtype == TNN_F32)
-    fill_kernel<float><<<grid, 256, 0, s>>>((float*)dst, (float)value, n);
-  else if (dtype == TNN_F64)
-    fill_kernel<double><<<grid, 256, 0, s>>>((double*)dst, value, n);
-  else
-    TNN_FAIL("tnn_fill: dtype must be TNN_F32 or TNN_F64");
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, "tnn_fill", [&](auto tag) {
+    using T = decltype(tag);
+    fill_kernel<T><<<ew_grid(n, 256), 256, 0, ctx().stream>>>((T*)dst, (T)value, n);
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
 
 }  // extern "C"

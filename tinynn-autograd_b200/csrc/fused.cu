@@ -14,35 +14,24 @@
 
 namespace tnn {
 
-template <typename T>
-struct V4 {
-  static constexpr int W = sizeof(T) == 4 ? 4 : 2;
-  using type = typename std::conditional<sizeof(T) == 4, float4, double2>::type;
-  union U {
-    type v;
-    T e[W];
-  };
-};
-
-static inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 // ---- ReLU ------------------------------------------------------------------------------------
 // forward: np.clip(x, 0.0, None) = maximum(x, 0) (NaN propagates); backward: g * (x >= 0)
 template <typename T, bool BWD, bool VEC>
 __global__ void __launch_bounds__(256) relu_kernel(T* out, const T* g, const T* x, int64_t n) {
-  constexpr int W = VEC ? V4<T>::W : 1;
+  constexpr int W = VEC ? 16 / sizeof(T) : 1;
   constexpr int U = 4;   // independent 128-bit loads in flight per thread (a 1-read stream needs them)
   const int64_t nv = n / W;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < nv; i0 += U * stride) {
     if constexpr (VEC) {
-      typename V4<T>::U a[U], b[U], r;
+      using V = Pack<T, W>;
+      V a[U], b[U], r;
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int64_t i = i0 + u * stride;
         if (i < nv) {
-          a[u].v = reinterpret_cast<const typename V4<T>::type*>(x)[i];
-          if (BWD) b[u].v = reinterpret_cast<const typename V4<T>::type*>(g)[i];
+          a[u] = reinterpret_cast<const V*>(x)[i];
+          if (BWD) b[u] = reinterpret_cast<const V*>(g)[i];
         }
       }
 #pragma unroll
@@ -51,8 +40,8 @@ __global__ void __launch_bounds__(256) relu_kernel(T* out, const T* g, const T* 
         if (i < nv) {
 #pragma unroll
           for (int k = 0; k < W; ++k)
-            r.e[k] = BWD ? (a[u].e[k] >= T(0) ? b[u].e[k] : b[u].e[k] * T(0)) : m_max(a[u].e[k], T(0));
-          reinterpret_cast<typename V4<T>::type*>(out)[i] = r.v;
+            r.v[k] = BWD ? (a[u].v[k] >= T(0) ? b[u].v[k] : b[u].v[k] * T(0)) : m_max(a[u].v[k], T(0));
+          reinterpret_cast<V*>(out)[i] = r;
         }
       }
     } else {
@@ -78,12 +67,11 @@ __global__ void __launch_bounds__(256) relu_kernel(T* out, const T* g, const T* 
 template <typename T, bool BWD>
 static int relu_launch(T* out, const T* g, const T* x, int64_t n) {
   if (n <= 0) return 0;
-  bool vec = al16(out) && al16(x) && (!BWD || al16(g)) && n >= V4<T>::W;
-  cudaStream_t st = ctx().stream;
-  if (vec)
-    relu_kernel<T, BWD, true><<<ew_grid(ceil_div(n, V4<T>::W), 256), 256, 0, st>>>(out, g, x, n);
-  else
-    relu_kernel<T, BWD, false><<<ew_grid(n, 256), 256, 0, st>>>(out, g, x, n);
+  constexpr int W = 16 / sizeof(T);
+  const bool vec = aligned16(out) && aligned16(x) && (!BWD || aligned16(g)) && n >= W;
+  with_bool(vec, [&](auto V) {
+    relu_kernel<T, BWD, V><<<ew_grid(V ? ceil_div(n, W) : n, 256), 256, 0, ctx().stream>>>(out, g, x, n);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
@@ -136,16 +124,15 @@ template <typename T, bool VEC>
 __global__ void __launch_bounds__(256)
 ce_partial_max_kernel(const T* z, int64_t n, T* partial) {
   __shared__ T sm[8];
-  constexpr int W = VEC ? V4<T>::W : 1;
+  constexpr int W = VEC ? 16 / sizeof(T) : 1;
   const int64_t nv = n / W;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   T mx = -INFINITY;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride) {
     if constexpr (VEC) {
-      typename V4<T>::U a;
-      a.v = reinterpret_cast<const typename V4<T>::type*>(z)[i];
+      const Pack<T, W> a = reinterpret_cast<const Pack<T, W>*>(z)[i];
 #pragma unroll
-      for (int k = 0; k < W; ++k) mx = m_max(mx, a.e[k]);
+      for (int k = 0; k < W; ++k) mx = m_max(mx, a.v[k]);
     } else {
       mx = m_max(mx, z[i]);
     }
@@ -166,7 +153,7 @@ ce_partial_sumexp_kernel(const T* z, int64_t n, const T* pmax, int n_pmax, T* ps
   T mx = -INFINITY;
   for (int i = threadIdx.x; i < n_pmax; i += 256) mx = m_max(mx, pmax[i]);
   mx = block_all_reduce<T, true>(mx, sm);
-  constexpr int W = VEC ? V4<T>::W : 1;
+  constexpr int W = VEC ? 16 / sizeof(T) : 1;
   const int64_t nv = n / W;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   T s = T(0);
@@ -175,17 +162,17 @@ ce_partial_sumexp_kernel(const T* z, int64_t n, const T* pmax, int n_pmax, T* ps
     // HBM bandwidth (measured 3.5 TB/s with one)
     constexpr int U = 4;
     for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < nv; i0 += U * stride) {
-      typename V4<T>::U a[U];
+      Pack<T, W> a[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int64_t i = i0 + u * stride;
-        if (i < nv) a[u].v = reinterpret_cast<const typename V4<T>::type*>(z)[i];
+        if (i < nv) a[u] = reinterpret_cast<const Pack<T, W>*>(z)[i];
       }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         if (i0 + u * stride < nv) {
 #pragma unroll
-          for (int k = 0; k < W; ++k) s += m_exp(a[u].e[k] - mx);
+          for (int k = 0; k < W; ++k) s += m_exp(a[u].v[k] - mx);
         }
       }
     }
@@ -551,31 +538,29 @@ __global__ void __launch_bounds__(256)
 adam_vec_kernel(T* param, const T* grad, T* s0, T* s1, int64_t nv, OptH hh, const OptH* hdev) {
   pdl_sync();
   if (hdev) hh = *hdev;
-  using VT = typename V4<T>::type;
-  using U = typename V4<T>::U;
-  constexpr int W = V4<T>::W;
+  constexpr int W = 16 / sizeof(T);
+  using V = Pack<T, W>;
   const T lr = (T)hh.h[0], omb1 = (T)(1.0 - hh.h[1]), omb2 = (T)(1.0 - hh.h[2]), eps = (T)hh.h[3];
   const T bc1 = (T)hh.h[4], bc2 = (T)hh.h[5];
   const T wd = (T)hh.h[7];   // weight decay, 0 = off (optimizer.py:28-29)
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride) {
-    U g, m, v, p;
-    g.v = reinterpret_cast<const VT*>(grad)[i];
-    m.v = reinterpret_cast<const VT*>(s0)[i];
-    v.v = reinterpret_cast<const VT*>(s1)[i];
-    p.v = reinterpret_cast<const VT*>(param)[i];
+    const V g = reinterpret_cast<const V*>(grad)[i];
+    V m = reinterpret_cast<const V*>(s0)[i];
+    V v = reinterpret_cast<const V*>(s1)[i];
+    V p = reinterpret_cast<const V*>(param)[i];
 #pragma unroll
     for (int k = 0; k < W; ++k) {
-      m.e[k] += omb1 * (g.e[k] - m.e[k]);
-      v.e[k] += omb2 * (g.e[k] * g.e[k] - v.e[k]);
-      T mh = m.e[k] / bc1, vh = v.e[k] / bc2;
+      m.v[k] += omb1 * (g.v[k] - m.v[k]);
+      v.v[k] += omb2 * (g.v[k] * g.v[k] - v.v[k]);
+      T mh = m.v[k] / bc1, vh = v.v[k] / bc2;
       T step = -lr * mh / (m_sqrt(vh) + eps);
-      if (wd != T(0)) step -= wd * p.e[k];
-      p.e[k] += step;
+      if (wd != T(0)) step -= wd * p.v[k];
+      p.v[k] += step;
     }
-    reinterpret_cast<VT*>(s0)[i] = m.v;
-    reinterpret_cast<VT*>(s1)[i] = v.v;
-    reinterpret_cast<VT*>(param)[i] = p.v;
+    reinterpret_cast<V*>(s0)[i] = m;
+    reinterpret_cast<V*>(s1)[i] = v;
+    reinterpret_cast<V*>(param)[i] = p;
   }
 }
 
@@ -586,44 +571,32 @@ static int opt_dispatch(int opt, T* param, T* step_out, const T* grad, T* s0, T*
   int grid = ew_grid(n, 256);
   // a small arena is the tail of a launch-bound chain (the MNIST-sized step): programmatic dependency
   const bool pdl = grid <= 2 * ctx().sm_count;
-  switch (opt) {
-    case TNN_OPT_SGD:
-      TNN_CUDA(launch_small(opt_kernel<TNN_OPT_SGD, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      break;
-    case TNN_OPT_ADAM: {
-      constexpr int W = V4<T>::W;
-      if (param && !step_out && al16(param) && al16(grad) && al16(s0) && al16(s1) && n >= W) {
-        int64_t nv = n / W;
-        TNN_CUDA(launch_small(adam_vec_kernel<T>, dim3(ew_grid(nv, 256)), dim3(256), st, pdl, 1u, param, grad, s0, s1, nv, hh, hdev));
-        ctx().launches++;
-        int64_t done = nv * W;
-        if (done < n)
-          TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADAM, T>, dim3(1), dim3(256), st, pdl, 1u, param + done,
-                                (T*)nullptr, grad + done, s0 + done, s1 + done, n - done, hh, hdev));
-        else
-          return 0;
-      } else {
-        TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADAM, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      }
-      break;
-    }
-    case TNN_OPT_RMSPROP:
-      TNN_CUDA(launch_small(opt_kernel<TNN_OPT_RMSPROP, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      break;
-    case TNN_OPT_MOMENTUM:
-      TNN_CUDA(launch_small(opt_kernel<TNN_OPT_MOMENTUM, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      break;
-    case TNN_OPT_ADAGRAD:
-      TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADAGRAD, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      break;
-    case TNN_OPT_ADADELTA:
-      TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADADELTA, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
-      break;
-    default:
-      TNN_FAIL("tnn_opt_step: unknown optimizer code");
+  constexpr int W = 16 / sizeof(T);
+  if (opt == TNN_OPT_ADAM && param && !step_out && aligned16(param) && aligned16(grad) && aligned16(s0) &&
+      aligned16(s1) && n >= W) {
+    const int64_t nv = n / W, done = nv * W;
+    TNN_CUDA(launch_small(adam_vec_kernel<T>, dim3(ew_grid(nv, 256)), dim3(256), st, pdl, 1u, param, grad, s0, s1, nv, hh, hdev));
+    ctx().launches++;
+    if (done == n) return 0;
+    TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADAM, T>, dim3(1), dim3(256), st, pdl, 1u, param + done, (T*)nullptr,
+                          grad + done, s0 + done, s1 + done, n - done, hh, hdev));
+    TNN_POST_LAUNCH();
+    return 0;
   }
-  TNN_POST_LAUNCH();
-  return 0;
+  auto run = [&](auto OPT) {
+    TNN_CUDA(launch_small(opt_kernel<OPT, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
+    TNN_POST_LAUNCH();
+    return 0;
+  };
+  switch (opt) {
+    case TNN_OPT_SGD: return run(std::integral_constant<int, TNN_OPT_SGD>{});
+    case TNN_OPT_ADAM: return run(std::integral_constant<int, TNN_OPT_ADAM>{});
+    case TNN_OPT_RMSPROP: return run(std::integral_constant<int, TNN_OPT_RMSPROP>{});
+    case TNN_OPT_MOMENTUM: return run(std::integral_constant<int, TNN_OPT_MOMENTUM>{});
+    case TNN_OPT_ADAGRAD: return run(std::integral_constant<int, TNN_OPT_ADAGRAD>{});
+    case TNN_OPT_ADADELTA: return run(std::integral_constant<int, TNN_OPT_ADADELTA>{});
+  }
+  TNN_FAIL("tnn_opt_step: unknown optimizer code");
 }
 
 // ---- CE host drivers ---------------------------------------------------------------------------
@@ -637,18 +610,16 @@ static int ce_stats_impl(const T* z, int64_t B, int64_t C, T* stats) {
     TNN_POST_LAUNCH();
     return 0;
   }
-  const bool vec = al16(z);
-  const int W = vec ? V4<T>::W : 1;
+  const bool vec = aligned16(z);
+  const int W = vec ? 16 / sizeof(T) : 1;
   int grid = ew_grid(ceil_div(n, W), 256, 4);
   void* scratch;
   if (get_scratch((size_t)grid * 2 * sizeof(T), &scratch)) return 1;
   T* pmax = (T*)scratch;
   T* psum = pmax + grid;
-  if (vec) ce_partial_max_kernel<T, true><<<grid, 256, 0, st>>>(z, n, pmax);
-  else ce_partial_max_kernel<T, false><<<grid, 256, 0, st>>>(z, n, pmax);
+  with_bool(vec, [&](auto V) { ce_partial_max_kernel<T, V><<<grid, 256, 0, st>>>(z, n, pmax); });
   TNN_POST_LAUNCH();
-  if (vec) ce_partial_sumexp_kernel<T, true><<<grid, 256, 0, st>>>(z, n, pmax, grid, psum, stats);
-  else ce_partial_sumexp_kernel<T, false><<<grid, 256, 0, st>>>(z, n, pmax, grid, psum, stats);
+  with_bool(vec, [&](auto V) { ce_partial_sumexp_kernel<T, V><<<grid, 256, 0, st>>>(z, n, pmax, grid, psum, stats); });
   TNN_POST_LAUNCH();
   ce_fold_sum_kernel<T><<<1, 256, 0, st>>>(psum, grid, stats + 1);
   TNN_POST_LAUNCH();
@@ -670,16 +641,16 @@ static int ce_loss_impl(const T* z, const TY* y, int64_t B, int64_t C, const T* 
     return 0;
   }
   int grid = (int)std::min<int64_t>(ceil_div(B, 8), (int64_t)ctx().sm_count * 8);
-  bool vec = false;
-  if constexpr (sizeof(T) == 4 && sizeof(TY) == 4)
-    vec = C >= 512 && C % 4 == 0 && al16(z) && al16(y);
-  if (vec) {
-    if constexpr (sizeof(T) == 4 && sizeof(TY) == 4)
+  // the 128-bit path is float32 logits and labels in wide 16-byte-aligned rows
+  constexpr bool f32 = sizeof(T) == 4 && sizeof(TY) == 4;
+  const bool vec = f32 && C >= 512 && C % 4 == 0 && aligned16(z) && aligned16(y);
+  with_bool(vec, [&](auto V) {
+    if constexpr (V && f32)
       ce_rows_vec_kernel<<<grid, 256, 0, st>>>((const float*)z, (const float*)y, B, C, (const float*)stats,
-                                               (float*)q, nll);
-  } else {
-    ce_rows_kernel<T, TY><<<grid, 256, 0, st>>>(z, y, B, C, stats, q, nll);
-  }
+                                               (float*)q, (float*)nll);
+    else
+      ce_rows_kernel<T, TY><<<grid, 256, 0, st>>>(z, y, B, C, stats, q, nll);
+  });
   TNN_POST_LAUNCH();
   ce_fold_loss_kernel<T><<<1, 256, 0, st>>>(nll, B, (T)m, loss);
   TNN_POST_LAUNCH();
@@ -689,25 +660,23 @@ static int ce_loss_impl(const T* z, const TY* y, int64_t B, int64_t C, const T* 
 template <typename T, typename TY>
 static int ce_bwd_impl(T* dz, const T* z, const TY* y, int64_t B, int64_t C, const T* stats,
                        const T* q, double m, const T* g, unsigned int* absmax_out, const int32_t* labels) {
-  cudaStream_t st = ctx().stream;
   // the 128-bit path is float32 logits with 4-column-aligned rows
-  const bool vec = sizeof(T) == 4 && (C % 4 == 0) && al16(dz) && al16(z) && (labels || al16(y));
+  constexpr bool f32 = sizeof(T) == 4;
+  const bool vec = f32 && (C % 4 == 0) && aligned16(dz) && aligned16(z) && (labels || aligned16(y));
   const int64_t nslot = vec ? C / 4 : C;
   int gx = (int)std::min<int64_t>(ceil_div(nslot, 256), 64);
   int64_t gy = std::min<int64_t>(B, std::max<int64_t>(1, (int64_t)ctx().sm_count * 8 / gx));
   if (gy > 65535) gy = 65535;
   // a small grid is part of a launch-bound chain (the MNIST-sized step): programmatic dependency
   const bool pdl = (int64_t)gx * gy <= 2 * (int64_t)ctx().sm_count;
-  if (vec) {
-    if constexpr (sizeof(T) == 4)
-      TNN_CUDA(launch_small(ce_bwd_kernel<T, TY, true>, dim3(gx, (unsigned)gy), dim3(256), st, pdl, 1u,
+  return with_bool(vec, [&](auto V) {
+    if constexpr (!V || f32) {
+      TNN_CUDA(launch_small(ce_bwd_kernel<T, TY, V>, dim3(gx, (unsigned)gy), dim3(256), ctx().stream, pdl, 1u,
                             dz, z, y, B, C, stats, q, (T)m, g, absmax_out, labels));
-  } else {
-    TNN_CUDA(launch_small(ce_bwd_kernel<T, TY, false>, dim3(gx, (unsigned)gy), dim3(256), st, pdl, 1u,
-                          dz, z, y, B, C, stats, q, (T)m, g, absmax_out, labels));
-  }
-  ctx().launches++;
-  return 0;
+      ctx().launches++;
+    }
+    return 0;
+  });
 }
 
 }  // namespace tnn
@@ -718,36 +687,36 @@ extern "C" {
 
 int tnn_relu_fwd(int dtype, void* out, const void* x, int64_t n) {
   TNN_REQUIRE_INIT();
-  if (dtype == TNN_F32) return relu_launch<float, false>((float*)out, nullptr, (const float*)x, n);
-  if (dtype == TNN_F64) return relu_launch<double, false>((double*)out, nullptr, (const double*)x, n);
-  TNN_FAIL("tnn_relu_fwd: bad dtype");
+  return with_float_type(dtype, "tnn_relu_fwd", [&](auto tag) {
+    using T = decltype(tag);
+    return relu_launch<T, false>((T*)out, nullptr, (const T*)x, n);
+  });
 }
 
 int tnn_relu_bwd(int dtype, void* dx, const void* g, const void* x, int64_t n) {
   TNN_REQUIRE_INIT();
-  if (dtype == TNN_F32) return relu_launch<float, true>((float*)dx, (const float*)g, (const float*)x, n);
-  if (dtype == TNN_F64) return relu_launch<double, true>((double*)dx, (const double*)g, (const double*)x, n);
-  TNN_FAIL("tnn_relu_bwd: bad dtype");
+  return with_float_type(dtype, "tnn_relu_bwd", [&](auto tag) {
+    using T = decltype(tag);
+    return relu_launch<T, true>((T*)dx, (const T*)g, (const T*)x, n);
+  });
 }
 
 int tnn_ce_stats(int dtype, const void* z, int64_t B, int64_t C, void* stats_dev) {
   TNN_REQUIRE_INIT();
-  if (dtype == TNN_F32) return ce_stats_impl<float>((const float*)z, B, C, (float*)stats_dev);
-  if (dtype == TNN_F64) return ce_stats_impl<double>((const double*)z, B, C, (double*)stats_dev);
-  TNN_FAIL("tnn_ce_stats: bad dtype");
+  return with_float_type(dtype, "tnn_ce_stats", [&](auto tag) {
+    using T = decltype(tag);
+    return ce_stats_impl<T>((const T*)z, B, C, (T*)stats_dev);
+  });
 }
 
 int tnn_ce_merge_stats(int dtype, void* stats_out_dev, const void* stats_all_dev, int n_ranks) {
   TNN_REQUIRE_INIT();
-  cudaStream_t st = ctx().stream;
-  if (dtype == TNN_F32)
-    ce_merge_stats_kernel<float><<<1, 32, 0, st>>>((float*)stats_out_dev, (const float*)stats_all_dev, n_ranks);
-  else if (dtype == TNN_F64)
-    ce_merge_stats_kernel<double><<<1, 32, 0, st>>>((double*)stats_out_dev, (const double*)stats_all_dev, n_ranks);
-  else
-    TNN_FAIL("tnn_ce_merge_stats: bad dtype");
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, "tnn_ce_merge_stats", [&](auto tag) {
+    using T = decltype(tag);
+    ce_merge_stats_kernel<T><<<1, 32, 0, ctx().stream>>>((T*)stats_out_dev, (const T*)stats_all_dev, n_ranks);
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
 
 int tnn_ce_loss(int dtype, const void* z, int y_dtype, const void* y, int64_t B, int64_t C,
@@ -756,16 +725,14 @@ int tnn_ce_loss(int dtype, const void* z, int y_dtype, const void* y, int64_t B,
   TNN_REQUIRE_INIT();
   if (B <= 0 || C <= 0) TNN_FAIL("tnn_ce_loss: empty logits");
   if (!y && !labels_dev) TNN_FAIL("tnn_ce_loss: neither dense labels nor class indices");
-  const int32_t* lab = labels_dev;
-  if (dtype == TNN_F32 && y_dtype == TNN_F32)
-    return ce_loss_impl<float, float>((const float*)z, (const float*)y, B, C, (const float*)stats_dev, m_global, (float*)q_dev, (float*)loss_dev, lab);
-  if (dtype == TNN_F32 && y_dtype == TNN_F64)
-    return ce_loss_impl<float, double>((const float*)z, (const double*)y, B, C, (const float*)stats_dev, m_global, (float*)q_dev, (float*)loss_dev, lab);
-  if (dtype == TNN_F64 && y_dtype == TNN_F64)
-    return ce_loss_impl<double, double>((const double*)z, (const double*)y, B, C, (const double*)stats_dev, m_global, (double*)q_dev, (double*)loss_dev, lab);
-  if (dtype == TNN_F64 && y_dtype == TNN_F32)
-    return ce_loss_impl<double, float>((const double*)z, (const float*)y, B, C, (const double*)stats_dev, m_global, (double*)q_dev, (double*)loss_dev, lab);
-  TNN_FAIL("tnn_ce_loss: bad dtype");
+  return with_float_type(dtype, "tnn_ce_loss", [&](auto tag) {
+    return with_float_type(y_dtype, "tnn_ce_loss", [&](auto ytag) {
+      using T = decltype(tag);
+      using TY = decltype(ytag);
+      return ce_loss_impl<T, TY>((const T*)z, (const TY*)y, B, C, (const T*)stats_dev, m_global, (T*)q_dev,
+                                 (T*)loss_dev, labels_dev);
+    });
+  });
 }
 
 int tnn_ce_fwd_small(int dtype, const void* z, int y_dtype, const void* y, int64_t B, int64_t C,
@@ -773,19 +740,16 @@ int tnn_ce_fwd_small(int dtype, const void* z, int y_dtype, const void* y, int64
   TNN_REQUIRE_INIT();
   if (B <= 0 || C <= 0) TNN_FAIL("tnn_ce_fwd_small: empty logits");
   if (B > CE_SMALL_MAX_ROWS || B * C > 16384) TNN_FAIL("tnn_ce_fwd_small: at most 2048 rows and 16384 logits");
-  cudaStream_t st = ctx().stream;
-  if (dtype == TNN_F32 && y_dtype == TNN_F32)
-    TNN_CUDA(launch_small(ce_fwd_small_kernel<float, float>, dim3(1), dim3(1024), st, true, 1u, (const float*)z, (const float*)y, B, C, (float)m_global, (float*)stats_dev, (float*)q_dev, (float*)loss_dev, (float*)dz_dev));
-  else if (dtype == TNN_F32 && y_dtype == TNN_F64)
-    TNN_CUDA(launch_small(ce_fwd_small_kernel<float, double>, dim3(1), dim3(1024), st, true, 1u, (const float*)z, (const double*)y, B, C, (float)m_global, (float*)stats_dev, (float*)q_dev, (float*)loss_dev, (float*)dz_dev));
-  else if (dtype == TNN_F64 && y_dtype == TNN_F64)
-    TNN_CUDA(launch_small(ce_fwd_small_kernel<double, double>, dim3(1), dim3(1024), st, true, 1u, (const double*)z, (const double*)y, B, C, m_global, (double*)stats_dev, (double*)q_dev, (double*)loss_dev, (double*)dz_dev));
-  else if (dtype == TNN_F64 && y_dtype == TNN_F32)
-    TNN_CUDA(launch_small(ce_fwd_small_kernel<double, float>, dim3(1), dim3(1024), st, true, 1u, (const double*)z, (const float*)y, B, C, m_global, (double*)stats_dev, (double*)q_dev, (double*)loss_dev, (double*)dz_dev));
-  else
-    TNN_FAIL("tnn_ce_fwd_small: bad dtype");
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, "tnn_ce_fwd_small", [&](auto tag) {
+    return with_float_type(y_dtype, "tnn_ce_fwd_small", [&](auto ytag) {
+      using T = decltype(tag);
+      using TY = decltype(ytag);
+      TNN_CUDA(launch_small(ce_fwd_small_kernel<T, TY>, dim3(1), dim3(1024), ctx().stream, true, 1u, (const T*)z,
+                            (const TY*)y, B, C, (T)m_global, (T*)stats_dev, (T*)q_dev, (T*)loss_dev, (T*)dz_dev));
+      TNN_POST_LAUNCH();
+      return 0;
+    });
+  });
 }
 
 int tnn_ce_bwd(int dtype, void* dz, const void* z, int y_dtype, const void* y, int64_t B, int64_t C,
@@ -794,18 +758,16 @@ int tnn_ce_bwd(int dtype, void* dz, const void* z, int y_dtype, const void* y, i
   TNN_REQUIRE_INIT();
   if (B <= 0 || C <= 0) return 0;
   if (!y && !labels_dev) TNN_FAIL("tnn_ce_bwd: neither dense labels nor class indices");
-  const int32_t* lab = labels_dev;
   unsigned int* am = (unsigned int*)stat_meta;   // word 0 of an f16 operand record (gemm_f16.cu)
-  if (am && dtype != TNN_F32) TNN_FAIL("tnn_ce_bwd: operand statistics are float32 only");
-  if (dtype == TNN_F32 && y_dtype == TNN_F32)
-    return ce_bwd_impl<float, float>((float*)dz, (const float*)z, (const float*)y, B, C, (const float*)stats_dev, (const float*)q_dev, m_global, (const float*)g_dev, am, lab);
-  if (dtype == TNN_F32 && y_dtype == TNN_F64)
-    return ce_bwd_impl<float, double>((float*)dz, (const float*)z, (const double*)y, B, C, (const float*)stats_dev, (const float*)q_dev, m_global, (const float*)g_dev, am, lab);
-  if (dtype == TNN_F64 && y_dtype == TNN_F64)
-    return ce_bwd_impl<double, double>((double*)dz, (const double*)z, (const double*)y, B, C, (const double*)stats_dev, (const double*)q_dev, m_global, (const double*)g_dev, am, lab);
-  if (dtype == TNN_F64 && y_dtype == TNN_F32)
-    return ce_bwd_impl<double, float>((double*)dz, (const double*)z, (const float*)y, B, C, (const double*)stats_dev, (const double*)q_dev, m_global, (const double*)g_dev, am, lab);
-  TNN_FAIL("tnn_ce_bwd: bad dtype");
+  return with_float_type(dtype, "tnn_ce_bwd", [&](auto tag) {
+    using T = decltype(tag);
+    if (am && !std::is_same<T, float>::value) TNN_FAIL("tnn_ce_bwd: operand statistics are float32 only");
+    return with_float_type(y_dtype, "tnn_ce_bwd", [&](auto ytag) {
+      using TY = decltype(ytag);
+      return ce_bwd_impl<T, TY>((T*)dz, (const T*)z, (const TY*)y, B, C, (const T*)stats_dev, (const T*)q_dev,
+                                m_global, (const T*)g_dev, am, labels_dev);
+    });
+  });
 }
 
 int tnn_opt_step(int opt, int dtype, void* param, void* step_out, const void* grad, void* s0,
@@ -815,11 +777,10 @@ int tnn_opt_step(int opt, int dtype, void* param, void* step_out, const void* gr
   if (n_h < 0 || n_h > 8) TNN_FAIL("tnn_opt_step: at most 8 hyper-parameters");
   OptH hh;
   for (int i = 0; i < 8; ++i) hh.h[i] = i < n_h ? h[i] : 0.0;
-  if (dtype == TNN_F32)
-    return opt_dispatch<float>(opt, (float*)param, (float*)step_out, (const float*)grad, (float*)s0, (float*)s1, n, hh, nullptr);
-  if (dtype == TNN_F64)
-    return opt_dispatch<double>(opt, (double*)param, (double*)step_out, (const double*)grad, (double*)s0, (double*)s1, n, hh, nullptr);
-  TNN_FAIL("tnn_opt_step: bad dtype");
+  return with_float_type(dtype, "tnn_opt_step", [&](auto tag) {
+    using T = decltype(tag);
+    return opt_dispatch<T>(opt, (T*)param, (T*)step_out, (const T*)grad, (T*)s0, (T*)s1, n, hh, nullptr);
+  });
 }
 
 int tnn_opt_step_dev(int opt, int dtype, void* param, void* step_out, const void* grad, void* s0,
@@ -829,11 +790,10 @@ int tnn_opt_step_dev(int opt, int dtype, void* param, void* step_out, const void
   if (!h_dev) TNN_FAIL("tnn_opt_step_dev: h_dev is NULL");
   OptH hh = {};
   const OptH* hd = reinterpret_cast<const OptH*>(h_dev);
-  if (dtype == TNN_F32)
-    return opt_dispatch<float>(opt, (float*)param, (float*)step_out, (const float*)grad, (float*)s0, (float*)s1, n, hh, hd);
-  if (dtype == TNN_F64)
-    return opt_dispatch<double>(opt, (double*)param, (double*)step_out, (const double*)grad, (double*)s0, (double*)s1, n, hh, hd);
-  TNN_FAIL("tnn_opt_step_dev: bad dtype");
+  return with_float_type(dtype, "tnn_opt_step_dev", [&](auto tag) {
+    using T = decltype(tag);
+    return opt_dispatch<T>(opt, (T*)param, (T*)step_out, (const T*)grad, (T*)s0, (T*)s1, n, hh, hd);
+  });
 }
 
 }  // extern "C"

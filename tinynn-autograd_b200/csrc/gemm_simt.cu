@@ -378,15 +378,11 @@ extern "C" int tnn_dense_bwd_simt(int dtype, const void* g, const void* x, const
   if (dx_masked && (!dx || !mask_src)) TNN_FAIL("tnn_dense_bwd_simt: dx_masked needs dx and mask_src");
   if (ceil_div(K, 32) * ceil_div(N, 32) + ceil_div(B, 32) * ceil_div(K, 32) + ceil_div(N, 32) > 65535)
     TNN_FAIL("tnn_dense_bwd_simt: layer too large for the grouped SIMT launch");
-  if (dtype == TNN_F32)
-    return dense_bwd_impl<float>((const float*)g, (const float*)x, (const float*)w, (const float*)mask_src,
-                                 (float*)dx, (float*)dx_masked, (float*)dw, dw_accumulate, (float*)db,
-                                 db_accumulate, B, K, N);
-  if (dtype == TNN_F64)
-    return dense_bwd_impl<double>((const double*)g, (const double*)x, (const double*)w,
-                                  (const double*)mask_src, (double*)dx, (double*)dx_masked, (double*)dw,
-                                  dw_accumulate, (double*)db, db_accumulate, B, K, N);
-  TNN_FAIL("tnn_dense_bwd_simt: dtype must be TNN_F32 or TNN_F64");
+  return with_float_type(dtype, "tnn_dense_bwd_simt", [&](auto tag) {
+    using T = decltype(tag);
+    return dense_bwd_impl<T>((const T*)g, (const T*)x, (const T*)w, (const T*)mask_src, (T*)dx, (T*)dx_masked,
+                             (T*)dw, dw_accumulate, (T*)db, db_accumulate, B, K, N);
+  });
 }
 
 extern "C" int tnn_gemm_simt(int dtype, void* C, int64_t ldc, const void* A, int64_t a_rs,
@@ -396,13 +392,9 @@ extern "C" int tnn_gemm_simt(int dtype, void* C, int64_t ldc, const void* A, int
   TNN_REQUIRE_INIT();
   if (M < 0 || N < 0 || K < 0) TNN_FAIL("tnn_gemm_simt: negative extent");
   if (mask_src && !act_out) TNN_FAIL("tnn_gemm_simt: mask_src needs act_out");
-  if (dtype == TNN_F32)
-    return gemm_simt_impl<float>((float*)C, ldc, (const float*)A, a_rs, a_cs, (const float*)B, b_rs,
-                                 b_cs, M, N, K, (const float*)bias, flags, (float*)act_out,
-                                 (const float*)mask_src);
-  if (dtype == TNN_F64)
-    return gemm_simt_impl<double>((double*)C, ldc, (const double*)A, a_rs, a_cs, (const double*)B,
-                                  b_rs, b_cs, M, N, K, (const double*)bias, flags, (double*)act_out,
-                                  (const double*)mask_src);
-  TNN_FAIL("tnn_gemm_simt: dtype must be TNN_F32 or TNN_F64");
+  return with_float_type(dtype, "tnn_gemm_simt", [&](auto tag) {
+    using T = decltype(tag);
+    return gemm_simt_impl<T>((T*)C, ldc, (const T*)A, a_rs, a_cs, (const T*)B, b_rs, b_cs, M, N, K, (const T*)bias,
+                             flags, (T*)act_out, (const T*)mask_src);
+  });
 }

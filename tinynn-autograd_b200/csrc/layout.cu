@@ -173,36 +173,27 @@ int tnn_strided_copy(int dtype, void* dst, const void* src, int ndim, const int6
                      const int64_t* dst_strides, const int64_t* src_strides) {
   TNN_REQUIRE_INIT();
   if (ndim < 0 || ndim > TNN_MAX_DIMS) TNN_FAIL("tnn_strided_copy: rank above TNN_MAX_DIMS");
-  if (dtype == TNN_F32)
-    return strided_copy_impl<float>((float*)dst, (const float*)src, ndim, shape, dst_strides, src_strides);
-  if (dtype == TNN_F64)
-    return strided_copy_impl<double>((double*)dst, (const double*)src, ndim, shape, dst_strides, src_strides);
-  TNN_FAIL("tnn_strided_copy: dtype must be TNN_F32 or TNN_F64");
+  return with_float_type(dtype, "tnn_strided_copy", [&](auto tag) {
+    using T = decltype(tag);
+    return strided_copy_impl<T>((T*)dst, (const T*)src, ndim, shape, dst_strides, src_strides);
+  });
 }
 
 static int rows_common(bool gather, int dtype, void* out, const void* in, const int64_t* idx,
                        int64_t n_idx, int64_t row_elems, int64_t n_rows_other) {
   TNN_REQUIRE_INIT();
   if (n_idx <= 0 || row_elems <= 0) return 0;
-  const size_t esz = dtype == TNN_F32 ? 4 : 8;
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("rows gather/scatter: bad dtype");
-  int vec_ok = ((row_elems * esz) % 16 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0) &&
-               ((reinterpret_cast<uintptr_t>(in) & 15) == 0);
-  int grid = (int)std::min<int64_t>(ceil_div(n_idx, 8), (int64_t)ctx().sm_count * 16);
-  cudaStream_t st = ctx().stream;
-  if (dtype == TNN_F32) {
-    if (gather)
-      rows_kernel<float, true><<<grid, 256, 0, st>>>((float*)out, (const float*)in, idx, n_idx, row_elems, n_rows_other, vec_ok);
-    else
-      rows_kernel<float, false><<<grid, 256, 0, st>>>((float*)out, (const float*)in, idx, n_idx, row_elems, n_rows_other, vec_ok);
-  } else {
-    if (gather)
-      rows_kernel<double, true><<<grid, 256, 0, st>>>((double*)out, (const double*)in, idx, n_idx, row_elems, n_rows_other, vec_ok);
-    else
-      rows_kernel<double, false><<<grid, 256, 0, st>>>((double*)out, (const double*)in, idx, n_idx, row_elems, n_rows_other, vec_ok);
-  }
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, gather ? "tnn_gather_rows" : "tnn_scatter_rows", [&](auto tag) {
+    using T = decltype(tag);
+    const int vec_ok = (row_elems * sizeof(T)) % 16 == 0 && aligned16(out) && aligned16(in);
+    const int grid = (int)std::min<int64_t>(ceil_div(n_idx, 8), (int64_t)ctx().sm_count * 16);
+    with_bool(gather, [&](auto G) {
+      rows_kernel<T, G><<<grid, 256, 0, ctx().stream>>>((T*)out, (const T*)in, idx, n_idx, row_elems, n_rows_other,
+                                                        vec_ok);
+    });
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
 
 int tnn_gather_rows(int dtype, void* out, const void* x, const int64_t* idx_dev, int64_t n_idx,
@@ -219,19 +210,14 @@ static int flat_common(bool gather, int dtype, void* out, const void* in, const 
                        int64_t n) {
   TNN_REQUIRE_INIT();
   if (n <= 0) return 0;
-  int grid = ew_grid(n, 256);
-  cudaStream_t st = ctx().stream;
-  if (dtype == TNN_F32) {
-    if (gather) flat_index_kernel<float, true><<<grid, 256, 0, st>>>((float*)out, (const float*)in, idx, n);
-    else flat_index_kernel<float, false><<<grid, 256, 0, st>>>((float*)out, (const float*)in, idx, n);
-  } else if (dtype == TNN_F64) {
-    if (gather) flat_index_kernel<double, true><<<grid, 256, 0, st>>>((double*)out, (const double*)in, idx, n);
-    else flat_index_kernel<double, false><<<grid, 256, 0, st>>>((double*)out, (const double*)in, idx, n);
-  } else {
-    TNN_FAIL("flat gather/scatter: bad dtype");
-  }
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, gather ? "tnn_gather_flat" : "tnn_scatter_flat", [&](auto tag) {
+    using T = decltype(tag);
+    with_bool(gather, [&](auto G) {
+      flat_index_kernel<T, G><<<ew_grid(n, 256), 256, 0, ctx().stream>>>((T*)out, (const T*)in, idx, n);
+    });
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
 
 int tnn_gather_flat(int dtype, void* out, const void* x, const int64_t* idx_dev, int64_t n) {
@@ -245,18 +231,16 @@ int tnn_scatter_flat(int dtype, void* out, const void* g, const int64_t* idx_dev
 int tnn_one_hot(int dtype, void* out, const int32_t* labels_dev, int64_t B, int64_t C) {
   TNN_REQUIRE_INIT();
   if (B <= 0 || C <= 0) return 0;
-  cudaStream_t st = ctx().stream;
-  if (dtype == TNN_F32 && C % 4 == 0 && ((uintptr_t)out & 15) == 0) {
-    one_hot_vec_kernel<<<ew_grid(B * (C / 4), 256), 256, 0, st>>>((float4*)out, labels_dev, B, C / 4);
-  } else if (dtype == TNN_F32) {
-    one_hot_kernel<float><<<ew_grid(B * C, 256), 256, 0, st>>>((float*)out, labels_dev, B, C);
-  } else if (dtype == TNN_F64) {
-    one_hot_kernel<double><<<ew_grid(B * C, 256), 256, 0, st>>>((double*)out, labels_dev, B, C);
-  } else {
-    TNN_FAIL("tnn_one_hot: bad dtype");
-  }
-  TNN_POST_LAUNCH();
-  return 0;
+  return with_float_type(dtype, "tnn_one_hot", [&](auto tag) {
+    using T = decltype(tag);
+    cudaStream_t st = ctx().stream;
+    if (std::is_same<T, float>::value && C % 4 == 0 && aligned16(out))
+      one_hot_vec_kernel<<<ew_grid(B * (C / 4), 256), 256, 0, st>>>((float4*)out, labels_dev, B, C / 4);
+    else
+      one_hot_kernel<T><<<ew_grid(B * C, 256), 256, 0, st>>>((T*)out, labels_dev, B, C);
+    TNN_POST_LAUNCH();
+    return 0;
+  });
 }
 
 }  // extern "C"

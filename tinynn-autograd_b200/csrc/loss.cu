@@ -56,13 +56,6 @@ __device__ __forceinline__ void loss_term(double p, double t, double delta, doub
 template <typename T>
 __device__ __forceinline__ T grad_out(double d, double scale) { return (T)(d * scale); }
 
-// one 16-byte access: 4 floats or 2 doubles
-template <typename T>
-struct alignas(16) Pack {
-  static constexpr int W = 16 / sizeof(T);
-  T e[W];
-};
-
 // sum of one double per thread over the CTA, in a fixed order; the result is valid in thread 0
 __device__ __forceinline__ double cta_sum(double s, double* sm) {
 #pragma unroll
@@ -89,8 +82,8 @@ pointwise_loss_fwd_kernel(const T* __restrict__ p, const T* __restrict__ t, int6
   double s = 0.0, l, d;
   int64_t done = 0;
   if constexpr (VEC) {
-    constexpr int W = Pack<T>::W;
-    using V = Pack<T>;
+    constexpr int W = 16 / sizeof(T);
+    using V = Pack<T, W>;
     const int64_t nv = n / W;
     for (int64_t i0 = tid; i0 < nv; i0 += 2 * stride) {
       V a[2], b[2], r;
@@ -108,9 +101,9 @@ pointwise_loss_fwd_kernel(const T* __restrict__ p, const T* __restrict__ t, int6
         if (i < nv) {
 #pragma unroll
           for (int k = 0; k < W; ++k) {
-            loss_term<KIND, true>((double)a[u].e[k], (double)b[u].e[k], delta, l, d);
+            loss_term<KIND, true>((double)a[u].v[k], (double)b[u].v[k], delta, l, d);
             s += l;
-            r.e[k] = grad_out<T>(d, scale);
+            r.v[k] = grad_out<T>(d, scale);
           }
           if (dp) reinterpret_cast<V*>(dp)[i] = r;
         }
@@ -144,8 +137,8 @@ pointwise_loss_bwd_kernel(T* __restrict__ dp, const T* __restrict__ p, const T* 
   double l, d;
   int64_t done = 0;
   if constexpr (VEC) {
-    constexpr int W = Pack<T>::W;
-    using V = Pack<T>;
+    constexpr int W = 16 / sizeof(T);
+    using V = Pack<T, W>;
     const int64_t nv = n / W;
     for (int64_t i0 = tid; i0 < nv; i0 += 2 * stride) {
       V a[2], b[2], r;
@@ -163,8 +156,8 @@ pointwise_loss_bwd_kernel(T* __restrict__ dp, const T* __restrict__ p, const T* 
         if (i < nv) {
 #pragma unroll
           for (int k = 0; k < W; ++k) {
-            loss_term<KIND, false>((double)a[u].e[k], (double)b[u].e[k], delta, l, d);
-            r.e[k] = grad_out<T>(d, scale);
+            loss_term<KIND, false>((double)a[u].v[k], (double)b[u].v[k], delta, l, d);
+            r.v[k] = grad_out<T>(d, scale);
           }
           reinterpret_cast<V*>(dp)[i] = r;
         }
@@ -179,14 +172,12 @@ pointwise_loss_bwd_kernel(T* __restrict__ dp, const T* __restrict__ p, const T* 
 }
 
 // ---- host side --------------------------------------------------------------------------------
-bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
-
 // one grid for both passes of a given (n, vector path): the forward's sum order depends on nothing else
 int loss_grid(int64_t n, bool vec, int W) { return ew_grid(vec ? ceil_div(n, 2 * W) : ceil_div(n, 2), kThreads); }
 
 template <typename T, int KIND>
 int fwd_impl(const void* p, const void* t, int64_t n, double m, double delta, void* loss, void* dp) {
-  constexpr int W = Pack<T>::W;
+  constexpr int W = 16 / sizeof(T);
   const bool vec = n >= W && aligned16(p) && aligned16(t) && (!dp || aligned16(dp));
   const int grid = loss_grid(n, vec, W);
   double* partials = nullptr;
@@ -197,35 +188,27 @@ int fwd_impl(const void* p, const void* t, int64_t n, double m, double delta, vo
     partials = (double*)scratch;
     if (col_fold_counters(&counters)) return 1;
   }
-  cudaStream_t st = ctx().stream;
-  if (vec)
-    pointwise_loss_fwd_kernel<T, KIND, true><<<grid, kThreads, 0, st>>>((const T*)p, (const T*)t, n, m, delta,
-                                                                       (T*)loss, (T*)dp, partials, counters);
-  else
-    pointwise_loss_fwd_kernel<T, KIND, false><<<grid, kThreads, 0, st>>>((const T*)p, (const T*)t, n, m, delta,
-                                                                        (T*)loss, (T*)dp, partials, counters);
+  with_bool(vec, [&](auto V) {
+    pointwise_loss_fwd_kernel<T, KIND, V><<<grid, kThreads, 0, ctx().stream>>>(
+        (const T*)p, (const T*)t, n, m, delta, (T*)loss, (T*)dp, partials, counters);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
 
 template <typename T, int KIND>
 int bwd_impl(void* dp, const void* p, const void* t, int64_t n, double m, double delta, const void* g) {
-  constexpr int W = Pack<T>::W;
+  constexpr int W = 16 / sizeof(T);
   const bool vec = n >= W && aligned16(p) && aligned16(t) && aligned16(dp);
-  const int grid = loss_grid(n, vec, W);
-  cudaStream_t st = ctx().stream;
-  if (vec)
-    pointwise_loss_bwd_kernel<T, KIND, true><<<grid, kThreads, 0, st>>>((T*)dp, (const T*)p, (const T*)t, n, m,
-                                                                       delta, (const T*)g);
-  else
-    pointwise_loss_bwd_kernel<T, KIND, false><<<grid, kThreads, 0, st>>>((T*)dp, (const T*)p, (const T*)t, n, m,
-                                                                        delta, (const T*)g);
+  with_bool(vec, [&](auto V) {
+    pointwise_loss_bwd_kernel<T, KIND, V><<<loss_grid(n, vec, W), kThreads, 0, ctx().stream>>>(
+        (T*)dp, (const T*)p, (const T*)t, n, m, delta, (const T*)g);
+  });
   TNN_POST_LAUNCH();
   return 0;
 }
 
-int check_args(const char* name, int dtype, int kind, int64_t n, double m, double delta) {
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL(std::string(name) + ": bad dtype");
+int check_args(const char* name, int kind, int64_t n, double m, double delta) {
   if (kind < TNN_LOSS_MSE || kind > TNN_LOSS_SIGMOID_CE) TNN_FAIL(std::string(name) + ": bad loss kind");
   if (n < 0) TNN_FAIL(std::string(name) + ": negative element count");
   if (!(m >= 1.0)) TNN_FAIL(std::string(name) + ": m_global must be at least 1");
@@ -234,44 +217,41 @@ int check_args(const char* name, int dtype, int kind, int64_t n, double m, doubl
   return 0;
 }
 
+// f(std::integral_constant<int, KIND>{}) for a loss kind that check_args accepted
+template <typename F>
+int with_kind(int kind, F&& f) {
+  switch (kind) {
+    case TNN_LOSS_MSE: return f(std::integral_constant<int, TNN_LOSS_MSE>{});
+    case TNN_LOSS_MAE: return f(std::integral_constant<int, TNN_LOSS_MAE>{});
+    case TNN_LOSS_HUBER: return f(std::integral_constant<int, TNN_LOSS_HUBER>{});
+    default: return f(std::integral_constant<int, TNN_LOSS_SIGMOID_CE>{});
+  }
+}
+
 }  // namespace
 }  // namespace tnn
 
 using namespace tnn;
-
-#define TNN_LOSS_DISPATCH(impl, ...)                                                       \
-  do {                                                                                     \
-    if (dtype == TNN_F32) {                                                                \
-      switch (kind) {                                                                      \
-        case TNN_LOSS_MSE: return impl<float, TNN_LOSS_MSE>(__VA_ARGS__);                  \
-        case TNN_LOSS_MAE: return impl<float, TNN_LOSS_MAE>(__VA_ARGS__);                  \
-        case TNN_LOSS_HUBER: return impl<float, TNN_LOSS_HUBER>(__VA_ARGS__);              \
-        default: return impl<float, TNN_LOSS_SIGMOID_CE>(__VA_ARGS__);                     \
-      }                                                                                    \
-    }                                                                                      \
-    switch (kind) {                                                                        \
-      case TNN_LOSS_MSE: return impl<double, TNN_LOSS_MSE>(__VA_ARGS__);                   \
-      case TNN_LOSS_MAE: return impl<double, TNN_LOSS_MAE>(__VA_ARGS__);                   \
-      case TNN_LOSS_HUBER: return impl<double, TNN_LOSS_HUBER>(__VA_ARGS__);               \
-      default: return impl<double, TNN_LOSS_SIGMOID_CE>(__VA_ARGS__);                      \
-    }                                                                                      \
-  } while (0)
 
 extern "C" {
 
 int tnn_pointwise_loss(int dtype, int kind, const void* p, const void* t, int64_t n, double m_global,
                        double delta, void* loss_dev, void* dp) {
   TNN_REQUIRE_INIT();
-  if (check_args("tnn_pointwise_loss", dtype, kind, n, m_global, delta)) return 1;
-  TNN_LOSS_DISPATCH(fwd_impl, p, t, n, m_global, delta, loss_dev, dp);
+  return with_float_type(dtype, "tnn_pointwise_loss", [&](auto tag) {
+    if (check_args("tnn_pointwise_loss", kind, n, m_global, delta)) return 1;
+    return with_kind(kind, [&](auto K) { return fwd_impl<decltype(tag), K>(p, t, n, m_global, delta, loss_dev, dp); });
+  });
 }
 
 int tnn_pointwise_loss_bwd(int dtype, int kind, void* dp, const void* p, const void* t, int64_t n,
                            double m_global, double delta, const void* g_dev) {
   TNN_REQUIRE_INIT();
-  if (check_args("tnn_pointwise_loss_bwd", dtype, kind, n, m_global, delta)) return 1;
-  if (n == 0) return 0;
-  TNN_LOSS_DISPATCH(bwd_impl, dp, p, t, n, m_global, delta, g_dev);
+  return with_float_type(dtype, "tnn_pointwise_loss_bwd", [&](auto tag) {
+    if (check_args("tnn_pointwise_loss_bwd", kind, n, m_global, delta)) return 1;
+    if (n == 0) return 0;
+    return with_kind(kind, [&](auto K) { return bwd_impl<decltype(tag), K>(dp, p, t, n, m_global, delta, g_dev); });
+  });
 }
 
 }  // extern "C"

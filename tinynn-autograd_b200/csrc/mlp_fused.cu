@@ -552,30 +552,20 @@ int tnn_mlp_tail_step(int n_layers, const int64_t* in_dims, const int64_t* out_d
   attr[0].val.cooperative = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  static bool attr_set[2] = {false, false};
-  if (y_dtype == TNN_F32) {
-    auto kern = mlp::mlp_tail_kernel<float>;
-    if (!attr_set[0]) {
+  return with_float_type(y_dtype, "tnn_mlp_tail_step", [&](auto tag) {
+    using TY = decltype(tag);
+    auto kern = mlp::mlp_tail_kernel<TY>;
+    static bool attr_set = false;   // one per label type
+    if (!attr_set) {
       TNN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-      attr_set[0] = true;
+      attr_set = true;
     }
-    TNN_CUDA(cudaLaunchKernelEx(&cfg, kern, a, (const float*)z1, (int)B, (const float*)y, (float)m_global,
+    TNN_CUDA(cudaLaunchKernelEx(&cfg, kern, a, (const float*)z1, (int)B, (const TY*)y, (float)m_global,
                                 (float*)grad, (float*)scratch, (float*)dz1, (float2*)stats, (float*)loss_part,
                                 (float*)loss_out, (unsigned int*)counters, (float*)logits_out));
-  } else if (y_dtype == TNN_F64) {
-    auto kern = mlp::mlp_tail_kernel<double>;
-    if (!attr_set[1]) {
-      TNN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-      attr_set[1] = true;
-    }
-    TNN_CUDA(cudaLaunchKernelEx(&cfg, kern, a, (const float*)z1, (int)B, (const double*)y, (float)m_global,
-                                (float*)grad, (float*)scratch, (float*)dz1, (float2*)stats, (float*)loss_part,
-                                (float*)loss_out, (unsigned int*)counters, (float*)logits_out));
-  } else {
-    TNN_FAIL("tnn_mlp_tail_step: labels must be float32 or float64");
-  }
-  ctx().launches++;
-  return 0;
+    ctx().launches++;
+    return 0;
+  });
 }
 
 }  // extern "C"

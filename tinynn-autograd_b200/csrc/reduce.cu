@@ -106,33 +106,29 @@ reduce_row_warp_kernel(T* out, const T* x, int64_t outer, int64_t red) {
 template <int RED, typename T, int VEC>
 __device__ __forceinline__ void col_accumulate(const T* __restrict__ base, int64_t lo, int64_t hi,
                                                int64_t inner, int ty, T (&acc)[VEC]) {
-  using V = typename std::conditional<VEC == 1, T, typename std::conditional<sizeof(T) == 4, float4, double2>::type>::type;
-  union U {
-    V v;
-    T e[VEC];
-  };
+  using V = Pack<T, VEC>;
   int64_t r = lo + ty;
   for (; r + 56 < hi; r += 64) {
-    U u[8];
+    V u[8];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) u[i].v = *reinterpret_cast<const V*>(base + (r + 8 * i) * inner);
+    for (int i = 0; i < 8; ++i) u[i] = *reinterpret_cast<const V*>(base + (r + 8 * i) * inner);
 #pragma unroll
     for (int i = 0; i < 8; ++i)
 #pragma unroll
-      for (int k = 0; k < VEC; ++k) acc[k] = red_op<RED, T>(acc[k], u[i].e[k]);
+      for (int k = 0; k < VEC; ++k) acc[k] = red_op<RED, T>(acc[k], u[i].v[k]);
   }
   if (r < hi) {
     // the tail as ONE more batch of predicated loads (a serial tail would be up to seven exposed DRAM
     // round trips -- most of the time of a 64 MB reduction)
-    U u[8];
+    V u[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i)
-      if (r + 8 * i < hi) u[i].v = *reinterpret_cast<const V*>(base + (r + 8 * i) * inner);
+      if (r + 8 * i < hi) u[i] = *reinterpret_cast<const V*>(base + (r + 8 * i) * inner);
 #pragma unroll
     for (int i = 0; i < 8; ++i)
       if (r + 8 * i < hi) {
 #pragma unroll
-        for (int k = 0; k < VEC; ++k) acc[k] = red_op<RED, T>(acc[k], u[i].e[k]);
+        for (int k = 0; k < VEC; ++k) acc[k] = red_op<RED, T>(acc[k], u[i].v[k]);
       }
   }
 }
@@ -204,15 +200,16 @@ int col_fold_counters(unsigned int** out) {
   return 0;
 }
 
+// dtype: T's code, which the fill of an empty reduction takes
 template <int RED, typename T>
-static int reduce_impl(T* out, const T* x, int64_t outer, int64_t red, int64_t inner) {
+static int reduce_impl(int dtype, T* out, const T* x, int64_t outer, int64_t red, int64_t inner) {
   Context& c = ctx();
   cudaStream_t st = c.stream;
   if (outer * inner == 0) return 0;
   if (red == 0) {
     // numpy: sum over an empty axis is 0; max/min raise -- mirror that
     if (RED != TNN_RED_SUM) TNN_FAIL("tnn_reduce: zero-size reduction has no identity");
-    return tnn_fill(sizeof(T) == 4 ? TNN_F32 : TNN_F64, out, 0.0, outer * inner);
+    return tnn_fill(dtype, out, 0.0, outer * inner);
   }
   const int64_t target_ctas = (int64_t)c.sm_count * 4;
   if (inner == 1) {
@@ -252,8 +249,8 @@ static int reduce_impl(T* out, const T* x, int64_t outer, int64_t red, int64_t i
     return 0;
   }
   // inner > 1
-  constexpr int VW = sizeof(T) == 4 ? 4 : 2;
-  bool vec = (inner % VW == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  constexpr int VW = 16 / sizeof(T);
+  bool vec = (inner % VW == 0) && aligned16(x);
   int64_t ncol = vec ? inner / VW : inner;
   int64_t gx = ceil_div(ncol, 32);
   int64_t nsplit = 1;
@@ -285,26 +282,12 @@ static int reduce_impl(T* out, const T* x, int64_t outer, int64_t red, int64_t i
   unsigned int* counters = nullptr;
   if (nsplit > 1 && col_fold_counters(&counters)) return 1;
   dim3 grid((unsigned)gx, (unsigned)(outer * nsplit));
-  if (vec)
-    reduce_col_kernel<RED, T, VW><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, counters);
-  else
-    reduce_col_kernel<RED, T, 1><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit, counters);
+  with_bool(vec, [&](auto V) {
+    reduce_col_kernel<RED, T, V ? VW : 1><<<grid, 256, 0, st>>>(out, (T*)scratch, x, red, inner, (int)nsplit,
+                                                                counters);
+  });
   TNN_POST_LAUNCH();
   return 0;
-}
-
-template <typename T>
-static int reduce_dispatch(int red_op_code, T* out, const T* x, int64_t outer, int64_t red,
-                           int64_t inner) {
-  switch (red_op_code) {
-    case TNN_RED_SUM:
-      return reduce_impl<TNN_RED_SUM, T>(out, x, outer, red, inner);
-    case TNN_RED_MAX:
-      return reduce_impl<TNN_RED_MAX, T>(out, x, outer, red, inner);
-    case TNN_RED_MIN:
-      return reduce_impl<TNN_RED_MIN, T>(out, x, outer, red, inner);
-  }
-  TNN_FAIL("tnn_reduce: unknown reduction code");
 }
 
 }  // namespace tnn
@@ -317,11 +300,15 @@ int tnn_reduce(int red_op_code, int dtype, void* out, const void* x, int64_t out
                int64_t inner) {
   TNN_REQUIRE_INIT();
   if (outer < 0 || red < 0 || inner < 0) TNN_FAIL("tnn_reduce: negative extent");
-  if (dtype == TNN_F32)
-    return reduce_dispatch<float>(red_op_code, (float*)out, (const float*)x, outer, red, inner);
-  if (dtype == TNN_F64)
-    return reduce_dispatch<double>(red_op_code, (double*)out, (const double*)x, outer, red, inner);
-  TNN_FAIL("tnn_reduce: dtype must be TNN_F32 or TNN_F64");
+  return with_float_type(dtype, "tnn_reduce", [&](auto tag) {
+    using T = decltype(tag);
+    switch (red_op_code) {
+      case TNN_RED_SUM: return reduce_impl<TNN_RED_SUM>(dtype, (T*)out, (const T*)x, outer, red, inner);
+      case TNN_RED_MAX: return reduce_impl<TNN_RED_MAX>(dtype, (T*)out, (const T*)x, outer, red, inner);
+      case TNN_RED_MIN: return reduce_impl<TNN_RED_MIN>(dtype, (T*)out, (const T*)x, outer, red, inner);
+    }
+    TNN_FAIL("tnn_reduce: unknown reduction code");
+  });
 }
 
 int tnn_colsum(int dtype, void* out, const void* g, int64_t R, int64_t C) {
@@ -332,8 +319,8 @@ int tnn_unbroadcast(int dtype, void* out, const void* grad, int ndim, const int6
                     const int32_t* keep) {
   TNN_REQUIRE_INIT();
   if (ndim < 0 || ndim > TNN_MAX_DIMS) TNN_FAIL("tnn_unbroadcast: rank above TNN_MAX_DIMS");
-  const size_t esz = dtype == TNN_F32 ? 4 : 8;
-  if (dtype != TNN_F32 && dtype != TNN_F64) TNN_FAIL("tnn_unbroadcast: bad dtype");
+  size_t esz = 0;
+  if (with_float_type(dtype, "tnn_unbroadcast", [&](auto tag) { esz = sizeof(tag); return 0; })) return 1;
   // collapse into alternating groups; size-1 axes vanish (summing them is the identity)
   int64_t dims[TNN_MAX_DIMS];
   int kp[TNN_MAX_DIMS];
