@@ -26,6 +26,8 @@ MAX_DIMS = 8
 ADD, SUB, MUL, DIV, POW, MAXIMUM, MINIMUM, GE, GT, LE, LT, EQ = range(12)
 MUL_GE, MUL_GT, MUL_LE, MUL_LT, MUL_EQ, DIV_BWD_B, POW_BWD_A, POW_BWD_B = range(20, 28)
 NEG, EXP, LOG, COPY, CLIP, SCALE, CLIP_BWD, RECIP_MUL = range(40, 48)
+LEAKY_RELU, ELU, GELU, GELU_TANH, SOFTPLUS, SILU = range(48, 54)
+LEAKY_RELU_BWD, ELU_BWD, GELU_BWD, GELU_TANH_BWD, SOFTPLUS_BWD, SILU_BWD = range(60, 66)
 RED_SUM, RED_MAX, RED_MIN = 0, 1, 2
 OPT_SGD, OPT_ADAM, OPT_RMSPROP, OPT_MOMENTUM, OPT_ADAGRAD, OPT_ADADELTA = range(6)
 

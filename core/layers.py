@@ -1,13 +1,18 @@
 """Layers (interface of the reference's core/layers.py: Layer, Dense, Activation, Sigmoid, Tanh,
 ReLU; `params` dicts, `inputs` bookkeeping, lazy Dense initialisation), plus the NHWC image layers
-Conv2D, MaxPool2D and Flatten of the tinynn family.
+Conv2D, MaxPool2D and Flatten and the activations LeakyReLU, ELU, GELU, Softplus and SiLU of the
+tinynn family.
 
 Dense is one fused GEMM(+bias) node; together with a following ReLU it is one launch (see
-core/nn.py).  Activations are compositions of the op library, which routes `clip(x, 0.0)` to the
-fused ReLU kernels.  Conv2D is im2col + that same Dense node.
+core/nn.py).  ReLU, Sigmoid and Tanh are compositions of the op library, which routes `clip(x, 0.0)`
+to the fused ReLU kernels; the other activations are one elementwise launch each way
+(ops.activation_).  Conv2D is im2col + that same Dense node.
 """
+import math
+
 import numpy as np
 
+import core._backend as be
 import core.ops as ops
 from core.initializer import ConstantInit
 from core.initializer import XavierUniformInit
@@ -306,3 +311,113 @@ class Sigmoid(Activation):
 
     def func(self, x):
         return 1.0 / (1.0 + ops.exp(-x))
+
+
+# ---------------------------------------------------------------------------- elementwise activations
+# Conventions shared by LeakyReLU, ELU, GELU, Softplus and SiLU (include/tnn_b200.h states them
+# beside the op codes):
+#   - the kink at 0 goes to the x >= 0 branch, as ReLU's (ReLU'(0) = 1), so LeakyReLU(0.0) equals
+#     ReLU in value and gradient on non-NaN inputs (torch gives slope / alpha there instead);
+#   - NaN in x gives NaN in y and in dx; +-inf give the function's limit and the derivative's limit;
+#   - every finite x gives a finite y and dx;
+#   - the computation is in the input's dtype (float32 or float64);
+#   - slope / alpha / approximate are fixed at construction (read-only properties): a recorded
+#     training step bakes them into its kernel arguments.
+# Each layer is one node, ops.activation_: one launch forward, one backward.
+
+def _finite_number(layer, what, value):
+    if isinstance(value, (bool, np.bool_)) or not isinstance(value, (int, float, np.integer, np.floating)):
+        raise ValueError("%s: %s must be a number, got %r" % (layer, what, value))
+    value = float(value)
+    if not math.isfinite(value):
+        raise ValueError("%s: %s must be finite, got %r" % (layer, what, value))
+    return value
+
+
+class LeakyReLU(Activation):
+    """y = x if x >= 0 else slope * x;  dy/dx = 1 if x >= 0 else slope.
+
+    slope (default 0.01) is any finite number, fixed at construction.  The kink at 0 goes to the
+    x >= 0 branch, so LeakyReLU(0.0) is ReLU on non-NaN inputs; LeakyReLU(-inf) is 0 when slope = 0.
+    NaN gives NaN in y and dx."""
+
+    def __init__(self, slope=0.01):
+        Activation.__init__(self, "LeakyReLU")
+        self._slope = _finite_number("LeakyReLU", "slope", slope)
+
+    @property
+    def slope(self):
+        return self._slope
+
+    def func(self, x):
+        return ops.activation_(ops.as_tensor(x), be.LEAKY_RELU, be.LEAKY_RELU_BWD, self._slope)
+
+
+class ELU(Activation):
+    """y = x if x >= 0 else alpha * expm1(x);  dy/dx = 1 if x >= 0 else alpha * exp(x).
+
+    alpha (default 1.0) is any finite number, fixed at construction.  dy/dx(0) = 1 (the x >= 0
+    branch); ELU(-inf) = -alpha with gradient 0.  NaN gives NaN in y and dx."""
+
+    def __init__(self, alpha=1.0):
+        Activation.__init__(self, "ELU")
+        self._alpha = _finite_number("ELU", "alpha", alpha)
+
+    @property
+    def alpha(self):
+        return self._alpha
+
+    def func(self, x):
+        return ops.activation_(ops.as_tensor(x), be.ELU, be.ELU_BWD, self._alpha)
+
+
+class GELU(Activation):
+    """approximate="none" (default): y = x * Phi(x), Phi(x) = erfc(-x / sqrt 2) / 2, the normal CDF;
+        dy/dx = Phi(x) + x * phi(x), phi(x) = exp(-x^2 / 2) / sqrt(2 pi).
+    approximate="tanh": y = x * s, s = sigma(2u) (= (1 + tanh u) / 2), u = sqrt(2/pi) (x + 0.044715 x^3);
+        dy/dx = s + 2x * s(1 - s) * sqrt(2/pi) (1 + 0.134145 x^2), s(1 - s) as sigma(2u) sigma(-2u).
+
+    sigma is the logistic function evaluated without overflow.  GELU(-inf) = 0, GELU(+inf) = +inf,
+    with gradients 0 and 1; in float32 the tanh form's x^3 and x^2 overflow for large finite |x|,
+    and the value and gradient there are still finite (x and 1, or 0 and 0).  NaN gives NaN.
+    approximate is "none" or "tanh", fixed at construction."""
+
+    def __init__(self, approximate="none"):
+        Activation.__init__(self, "GELU")
+        if not isinstance(approximate, str) or approximate not in ("none", "tanh"):
+            raise ValueError("GELU: approximate must be 'none' or 'tanh', got %r" % (approximate,))
+        self._approximate = approximate
+
+    @property
+    def approximate(self):
+        return self._approximate
+
+    def func(self, x):
+        if self._approximate == "tanh":
+            return ops.activation_(ops.as_tensor(x), be.GELU_TANH, be.GELU_TANH_BWD)
+        return ops.activation_(ops.as_tensor(x), be.GELU, be.GELU_BWD)
+
+
+class Softplus(Activation):
+    """y = max(x, 0) + log1p(exp(-|x|)) (= log(1 + e^x) without overflow);  dy/dx = sigma(x).
+
+    Softplus(-inf) = 0, Softplus(+inf) = +inf, with gradients 0 and 1.  NaN gives NaN."""
+
+    def __init__(self):
+        Activation.__init__(self, "Softplus")
+
+    def func(self, x):
+        return ops.activation_(ops.as_tensor(x), be.SOFTPLUS, be.SOFTPLUS_BWD)
+
+
+class SiLU(Activation):
+    """y = x * sigma(x);  dy/dx = sigma(x) (1 + x (1 - sigma(x))), x (1 - sigma(x)) sigma(x) as
+    x sigma(x) sigma(-x).  sigma is the logistic function evaluated without overflow.
+
+    SiLU(-inf) = 0, SiLU(+inf) = +inf, with gradients 0 and 1.  NaN gives NaN."""
+
+    def __init__(self):
+        Activation.__init__(self, "SiLU")
+
+    def func(self, x):
+        return ops.activation_(ops.as_tensor(x), be.SILU, be.SILU_BWD)

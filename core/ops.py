@@ -7,8 +7,9 @@ A grad_fn receives the incoming gradient as a device array and returns a device 
 un-broadcast reduction the reference inlines twelve times (ops.py:41-46 ...) is one backend call.
 Three fused nodes are added for the training path (dense_, relu_, softmax_ce_); they are what
 core/layers.py and core/losses.py use.  Two more serve the NHWC image layers: im2col_ (Conv2D's
-window matrix) and maxpool2d_; batchnorm_ is BatchNormalization, and pointwise_loss_ the MSE, MAE,
-Huber and sigmoid cross-entropy losses.
+window matrix) and maxpool2d_; batchnorm_ is BatchNormalization, pointwise_loss_ the MSE, MAE,
+Huber and sigmoid cross-entropy losses, and activation_ the LeakyReLU, ELU, GELU, Softplus and SiLU
+layers.
 """
 import builtins as _bi
 
@@ -487,6 +488,21 @@ def relu_(ts):
 
     def grad_fn(grad):
         return be.relu_bwd(grad, x)
+
+    return build_unary_ops_tensor(ts, grad_fn, values)
+
+
+def activation_(ts, op, bwd_op, param=0.0):
+    """an elementwise activation (LeakyReLU, ELU, GELU, Softplus, SiLU of core/layers.py) as one node:
+    y = f(x) is one be.ew launch with code `op`, the gradient one launch of the binary `bwd_op`,
+    g * f'(x), with `param` (slope / alpha) as p0 both ways.  Computed in x's dtype."""
+    x = ts._data
+    values = be.ew(op, x, p0=param)
+
+    def grad_fn(grad):
+        if grad.dtype != x.dtype:
+            grad = be.astype(grad, x.dtype)
+        return be.ew(bwd_op, grad, x, p0=param)
 
     return build_unary_ops_tensor(ts, grad_fn, values)
 

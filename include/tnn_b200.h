@@ -62,7 +62,37 @@ enum {
   TNN_OP_CLIP = 44,       /* ops.py:334 x.clip(p0,p1); flags bit0 = has min, bit1 = has max */
   TNN_OP_SCALE = 45,      /* x*p0 + p1                                                */
   TNN_OP_CLIP_BWD = 46,   /* binary: x*(mask(y; p0,p1))  ops.py:336-343               */
-  TNN_OP_RECIP_MUL = 47   /* binary: x / y -- alias of DIV kept for log_ grad ops.py:247 */
+  TNN_OP_RECIP_MUL = 47,  /* binary: x / y -- alias of DIV kept for log_ grad ops.py:247 */
+  /* activations (core/layers.py LeakyReLU, ELU, GELU, Softplus, SiLU; new).  Unary forward
+     y = f(x), p0 = slope / alpha:
+       LEAKY_RELU  x if x >= 0 else p0 x                     f' = 1 if x >= 0 else p0
+       ELU         x if x >= 0 else p0 expm1(x)              f' = 1 if x >= 0 else p0 exp(x)
+       GELU        x Phi(x), Phi(x) = erfc(-x/sqrt2)/2       f' = Phi(x) + x phi(x),
+                                                                  phi(x) = exp(-x^2/2)/sqrt(2 pi)
+       GELU_TANH   x s, s = sigma(2u) (= (1 + tanh u)/2),    f' = s + 2x s(1-s) sqrt(2/pi)(1 + 0.134145 x^2)
+                   u = sqrt(2/pi)(x + 0.044715 x^3)
+       SOFTPLUS    max(x, 0) + log1p(exp(-|x|))              f' = sigma(x)
+       SILU        x sigma(x)                                f' = sigma(x)(1 + x(1 - sigma(x)))
+     sigma(v) = 1/(1+e^-v) for v >= 0, e^v/(1+e^v) otherwise; s(1-s) is evaluated as sigma(v) sigma(-v).
+     The kink at 0 goes to the x >= 0 branch (ReLU's convention: LeakyReLU(0) is ReLU on non-NaN x).
+     NaN gives NaN in y and in dx; +-inf give the function's limit and the derivative's limit; every
+     finite x gives a finite y and dx (terms whose weight underflowed to 0 are 0, never inf * 0).
+     Computed in the operands' dtype with libdevice's accurate functions (no fast-math); Phi is
+     libdevice's normcdf, and GELU_TANH evaluates no tanh. */
+  TNN_OP_LEAKY_RELU = 48,
+  TNN_OP_ELU = 49,
+  TNN_OP_GELU = 50,
+  TNN_OP_GELU_TANH = 51,
+  TNN_OP_SOFTPLUS = 52,
+  TNN_OP_SILU = 53,
+  /* binary backward: out = x * f'(y), x = the upstream gradient, y = the activation's input, p0 as
+     the forward's (laid out as TNN_OP_CLIP_BWD) */
+  TNN_OP_LEAKY_RELU_BWD = 60,
+  TNN_OP_ELU_BWD = 61,
+  TNN_OP_GELU_BWD = 62,
+  TNN_OP_GELU_TANH_BWD = 63,
+  TNN_OP_SOFTPLUS_BWD = 64,
+  TNN_OP_SILU_BWD = 65
 };
 
 /* ---- reduction op codes (tnn_reduce) ------------------------------------------------------ */

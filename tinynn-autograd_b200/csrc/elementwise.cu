@@ -1,6 +1,7 @@
 // Elementwise kernels with numpy broadcasting: the forward values and gradient products of
 // core/ops.py:32-249, 293-299, 333-344 of the reference (add_, mul_, div_, pow_, maximum_,
-// minimum_, exp_, log_, neg_, clip_ and the comparison operators of core/tensor.py:48-58).
+// minimum_, exp_, log_, neg_, clip_ and the comparison operators of core/tensor.py:48-58), and the
+// forward and backward passes of the LeakyReLU, ELU, GELU, Softplus and SiLU layers.
 //
 // HBM-bound.  Three launch shapes, chosen on the host after collapsing adjacent axes:
 //   flat  : every operand contiguous (or one element)  -> 128-bit vector loads, grid-stride
@@ -56,11 +57,29 @@ __device__ __forceinline__ T ew_apply(T x, T y, T z, const EwParams<T>& p) {
     if (p.flags & 1) m = m && (y >= p.p0);
     if (p.flags & 2) m = m && (y <= p.p1);
     return m ? x : x * T(0);
-  } else return x;
+  }
+  // activations (math.cuh): forward f(x); backward x = upstream gradient, y = the activation's input
+  else if constexpr (OP == TNN_OP_LEAKY_RELU) return act_leaky_relu(x, p.p0);
+  else if constexpr (OP == TNN_OP_ELU) return act_elu(x, p.p0);
+  else if constexpr (OP == TNN_OP_GELU) return act_gelu(x);
+  else if constexpr (OP == TNN_OP_GELU_TANH) return act_gelu_tanh(x);
+  else if constexpr (OP == TNN_OP_SOFTPLUS) return act_softplus(x);
+  else if constexpr (OP == TNN_OP_SILU) return act_silu(x);
+  else if constexpr (OP == TNN_OP_LEAKY_RELU_BWD) return act_leaky_relu_bwd(x, y, p.p0);
+  else if constexpr (OP == TNN_OP_ELU_BWD) return act_elu_bwd(x, y, p.p0);
+  else if constexpr (OP == TNN_OP_GELU_BWD) return act_gelu_bwd(x, y);
+  else if constexpr (OP == TNN_OP_GELU_TANH_BWD) return act_gelu_tanh_bwd(x, y);
+  else if constexpr (OP == TNN_OP_SOFTPLUS_BWD) return act_softplus_bwd(x, y);
+  else if constexpr (OP == TNN_OP_SILU_BWD) return act_silu_bwd(x, y);
+  else return x;
 }
 
+// codes below 20 and from TNN_OP_LEAKY_RELU_BWD up are binary, 20..39 ternary, 40..59 unary
+// except the two binary codes among them
 __host__ __device__ constexpr int op_arity(int op) {
-  return (op >= 20 && op < 40) ? 3 : ((op >= 40 && op != TNN_OP_CLIP_BWD && op != TNN_OP_RECIP_MUL) ? 1 : 2);
+  if (op >= 20 && op < 40) return 3;
+  if (op < 20 || op >= TNN_OP_LEAKY_RELU_BWD || op == TNN_OP_CLIP_BWD || op == TNN_OP_RECIP_MUL) return 2;
+  return 1;
 }
 
 // ---- flat ------------------------------------------------------------------------------------
@@ -387,6 +406,18 @@ static int with_op(int op, const char* name, F&& f) {
     TNN_EW_CASE(TNN_OP_SCALE)
     TNN_EW_CASE(TNN_OP_CLIP_BWD)
     TNN_EW_CASE(TNN_OP_RECIP_MUL)
+    TNN_EW_CASE(TNN_OP_LEAKY_RELU)
+    TNN_EW_CASE(TNN_OP_ELU)
+    TNN_EW_CASE(TNN_OP_GELU)
+    TNN_EW_CASE(TNN_OP_GELU_TANH)
+    TNN_EW_CASE(TNN_OP_SOFTPLUS)
+    TNN_EW_CASE(TNN_OP_SILU)
+    TNN_EW_CASE(TNN_OP_LEAKY_RELU_BWD)
+    TNN_EW_CASE(TNN_OP_ELU_BWD)
+    TNN_EW_CASE(TNN_OP_GELU_BWD)
+    TNN_EW_CASE(TNN_OP_GELU_TANH_BWD)
+    TNN_EW_CASE(TNN_OP_SOFTPLUS_BWD)
+    TNN_EW_CASE(TNN_OP_SILU_BWD)
     default:
       TNN_FAIL(std::string(name) + ": unknown op code " + std::to_string(op));
   }

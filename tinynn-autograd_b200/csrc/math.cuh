@@ -158,10 +158,96 @@ TNN_HD double m_pow(double a, double b) {
 }
 TNN_HD float m_sqrt(float x) { return sqrtf(x); }
 TNN_HD double m_sqrt(double x) { return sqrt(x); }
+// Plain libdevice functions in both precisions, for the activations (nothing there is compared
+// with `==`, so exp needs no correctly rounded f64 path).
+TNN_HD float m_exp_ld(float x) { return expf(x); }
+TNN_HD double m_exp_ld(double x) { return exp(x); }
+TNN_HD float m_expm1(float x) { return expm1f(x); }
+TNN_HD double m_expm1(double x) { return expm1(x); }
+TNN_HD float m_log1p(float x) { return log1pf(x); }
+TNN_HD double m_log1p(double x) { return log1p(x); }
 // np.maximum / np.minimum propagate NaN (fmax/fmin do not)
 template <typename T>
 TNN_HD T m_max(T a, T b) { return (a != a) ? a : ((b != b) ? b : (a > b ? a : b)); }
 template <typename T>
 TNN_HD T m_min(T a, T b) { return (a != a) ? a : ((b != b) ? b : (a < b ? a : b)); }
+
+#if defined(__CUDACC__)  // (normcdf is a CUDA math function; the host build of this header has none)
+// ---- activations (TNN_OP_LEAKY_RELU .. TNN_OP_SILU_BWD; formulas in include/tnn_b200.h) ----------
+// The kink at 0 goes to the x >= 0 branch; NaN in gives NaN out; +-inf give the limits; every finite
+// x gives a finite value and derivative.  A product x * w whose weight w has underflowed to 0 is
+// taken as 0, so no inf * 0 reaches the output (x = -inf, or x^2, x^3 overflowed).
+
+// the logistic function without overflow: s = sigma(v), sn = sigma(-v) = 1 - s (NaN for NaN v)
+template <typename T>
+struct Sigmoid2 {
+  T s, sn;
+};
+template <typename T>
+TNN_HD Sigmoid2<T> sigmoid2(T v) {
+  const T e = m_exp_ld(-fabs(v));
+  const T lo = e / (T(1) + e), hi = T(1) / (T(1) + e);
+  return v >= T(0) ? Sigmoid2<T>{hi, lo} : Sigmoid2<T>{lo, hi};
+}
+template <typename T>
+TNN_HD T mul_or_zero(T x, T w) { return w == T(0) ? T(0) : x * w; }
+
+template <typename T>
+TNN_HD T act_leaky_relu(T x, T slope) {
+  if (!(x < T(0))) return x;                      // x >= 0 or NaN
+  return mul_or_zero(x, slope);
+}
+template <typename T>
+TNN_HD T act_leaky_relu_bwd(T g, T x, T slope) {
+  if (!(x < T(0))) return x >= T(0) ? g : x;
+  return g * slope;
+}
+template <typename T>
+TNN_HD T act_elu(T x, T alpha) { return x >= T(0) ? x : alpha * m_expm1(x); }
+template <typename T>
+TNN_HD T act_elu_bwd(T g, T x, T alpha) { return x >= T(0) ? g : g * (alpha * m_exp_ld(x)); }
+
+// Phi(x) = erfc(-x / sqrt 2) / 2 as libdevice's normcdf (x / sqrt 2 is not rounded first; with erfc
+// written out, the f64 backward's flat vector kernel spills), phi(x) = exp(-x^2 / 2) / sqrt(2 pi)
+TNN_HD float m_normcdf(float x) { return normcdff(x); }
+TNN_HD double m_normcdf(double x) { return normcdf(x); }
+template <typename T>
+TNN_HD T act_gelu(T x) { return mul_or_zero(x, m_normcdf(x)); }
+template <typename T>
+TNN_HD T act_gelu_bwd(T g, T x) {
+  const T pdf = m_exp_ld(T(-0.5) * (x * x)) * T(0.39894228040143267794);
+  return g * (m_normcdf(x) + mul_or_zero(x, pdf));
+}
+
+// u = sqrt(2/pi) (x + 0.044715 x^3); y = x sigma(2u); x^3 = +-inf still gives sigma(2u) in {0, 1}
+template <typename T>
+TNN_HD Sigmoid2<T> gelu_tanh_sig(T x) {
+  return sigmoid2(T(2) * (T(0.79788456080286535588) * (x + T(0.044715) * (x * x * x))));
+}
+template <typename T>
+TNN_HD T act_gelu_tanh(T x) { return mul_or_zero(x, gelu_tanh_sig(x).s); }
+template <typename T>
+TNN_HD T act_gelu_tanh_bwd(T g, T x) {
+  const Sigmoid2<T> q = gelu_tanh_sig(x);
+  const T w = q.s * q.sn;                         // s (1 - s) without cancellation
+  // where w has underflowed, the polynomial (which overflows first at |x| ~ 2e19 in f32) is not read
+  const T t = w == T(0) ? T(0)
+                        : (T(2) * x) * w * (T(0.79788456080286535588) * (T(1) + T(0.134145) * (x * x)));
+  return g * (q.s + t);
+}
+
+template <typename T>
+TNN_HD T act_softplus(T x) { return (x > T(0) ? x : T(0)) + m_log1p(m_exp_ld(-fabs(x))); }
+template <typename T>
+TNN_HD T act_softplus_bwd(T g, T x) { return g * sigmoid2(x).s; }
+
+template <typename T>
+TNN_HD T act_silu(T x) { return mul_or_zero(x, sigmoid2(x).s); }
+template <typename T>
+TNN_HD T act_silu_bwd(T g, T x) {
+  const Sigmoid2<T> q = sigmoid2(x);
+  return g * (q.s + mul_or_zero(x, q.s * q.sn));
+}
+#endif  // __CUDACC__
 
 }  // namespace tnn
