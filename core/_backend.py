@@ -845,12 +845,18 @@ def _empty_16bit(rows, ld):
     return empty((rows, ld // 2), F32)
 
 
-def split_planes_mix(x):
-    """fp32 (R, C) -> (hi tf32 plane, bf16(x), bf16(x - hi), ld), cached for the step"""
+def _plane_cache(x):
+    """x's operand-plane cache for the current step (a fresh one when x has none from this step)"""
     cache = x.split
     if cache is None or cache.get("epoch") != _split_epoch:
         cache = {"epoch": _split_epoch}
         x.split = cache
+    return cache
+
+
+def split_planes_mix(x):
+    """fp32 (R, C) -> (hi tf32 plane, bf16(x), bf16(x - hi), ld), cached for the step"""
+    cache = _plane_cache(x)
     if "m" in cache:
         return cache["m"]
     R, C = x.shape
@@ -874,10 +880,7 @@ def split_planes_f16(x):
     """fp32 (R, C) -> (hf fp16 plane, l16 bf16 plane, ld, meta, source array, relu_mode), cached for
     the step.  A LazyReLU is split straight from its pre-activation (relu applied on load); the
     statistics come from the producer's epilogue when it left a record (cache["stat"])."""
-    cache = x.split
-    if cache is None or cache.get("epoch") != _split_epoch:
-        cache = {"epoch": _split_epoch}
-        x.split = cache
+    cache = _plane_cache(x)
     if "f" in cache:
         return cache["f"]
     R, C = x.shape
@@ -978,10 +981,7 @@ def _matmul_f16(a, b, ta, tb, bias, out, flags, act, mask_src, M, N, K):
 def split_planes(x, transposed, also_other=False):
     """fp32 (R, C) -> tf32 (hi, lo, ld) planes; transposed=True gives the (C, R) planes.
     Planes are cached on the array for the current step so forward and backward share them."""
-    cache = x.split
-    if cache is None or cache.get("epoch") != _split_epoch:
-        cache = {"epoch": _split_epoch}
-        x.split = cache
+    cache = _plane_cache(x)
     key = "t" if transposed else "p"
     if key in cache:
         return cache[key]
@@ -1032,10 +1032,11 @@ def matmul(a, b, ta=False, tb=False, bias=None, out=None, accumulate=False, relu
            reuse_a=False, reuse_b=False, act=False, mask_src=None):
     """op(a) @ op(b) (+ bias) for 2-D arrays; op = transpose when ta/tb (ops.py:150-160).
 
-    float32 products above TC_MIN_MNK run on the tcgen05 3xTF32 kernel; float64 and small or
-    odd-shaped products run on the SIMT kernel.  reuse_a/reuse_b hint that the other orientation
-    of that operand will be needed later in the step (forward -> backward), so both sets of tf32
-    planes are produced by one pass.
+    float32 products above TC_MIN_MNK run on a tcgen05 tensor-core kernel chosen by TC_SPLIT: the
+    scaled fp16 split by default (with the mixed split as its on-device fallback), the mixed
+    tf32/bf16 split, or 3xTF32; float64 and small or odd-shaped products run on the SIMT kernel.
+    reuse_a/reuse_b hint that the other orientation of that operand will be needed later in the
+    step (forward -> backward), so both sets of 3xTF32 planes are produced by one pass.
 
     act=True returns (out, relu(out)): the GEMM epilogue writes the ReLU of its result as a second
     array -- and, on the tensor-core path, that array's tf32 planes, which are attached to it so the

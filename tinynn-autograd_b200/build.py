@@ -21,6 +21,7 @@ SOURCES = ["runtime.cu", "elementwise.cu", "reduce.cu", "layout.cu", "gemm_simt.
            "gemm_tc.cu", "gemm_f16.cu", "fused.cu", "mlp_fused.cu", "comm.cu", "conv.cu",
            "batchnorm.cu", "loss.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "math.cuh"), os.path.join(CSRC, "tc_ptx.cuh"),
+           os.path.join(CSRC, "tc_gemm.cuh"),
            os.path.join(ROOT, "include", "tnn_b200.h")]
 
 # -split-compile 0: the per-kernel optimisation phase runs on all host cores (gemm_tc.cu instantiates

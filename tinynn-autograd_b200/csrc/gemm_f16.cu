@@ -36,12 +36,9 @@
 #include <cstdlib>
 
 #include "common.cuh"
-#include "tc_ptx.cuh"
+#include "tc_gemm.cuh"
 
 namespace tnn {
-namespace tc {
-extern int g_reserved_sms;   // tnn_set_gemm_reserved_sms (gemm_tc.cu)
-}
 namespace f16 {
 
 using namespace tnn::tc;
@@ -131,56 +128,6 @@ __host__ __device__ constexpr uint32_t make_idesc(int a_fmt, int b_fmt, bool a_m
          ((b_mn ? 1u : 0u) << 16) | ((uint32_t)(UMMA_N >> 3) << 17) | ((uint32_t)(TILE_M >> 4) << 24);
 }
 
-// group_m = 1: row-major.  group_m = -g: column panels of g tile columns (all tile rows of a panel,
-// row-major inside it, before the next panel), so the panel's B operand stays L2-resident.
-// group_m = g > 1: row groups (consecutive tiles walk g tile rows before the next tile column).
-__device__ __forceinline__ void tile_coords(int t, int tiles_m, int tiles_n, int group_m, int& tm, int& tn) {
-  if (group_m == 1) {
-    tm = t / tiles_n;
-    tn = t - tm * tiles_n;
-  } else if (group_m < 0) {
-    const int gn = -group_m;
-    const int per_panel = tiles_m * gn;
-    const int g = t / per_panel;
-    const int first_n = g * gn;
-    const int cols = min(gn, tiles_n - first_n);
-    const int r = t - g * per_panel;
-    tm = r / cols;
-    tn = first_n + r % cols;
-  } else {
-    const int per_group = group_m * tiles_n;
-    const int g = t / per_group;
-    const int first_m = g * group_m;
-    const int rows = min(group_m, tiles_m - first_m);
-    const int r = t - g * per_group;
-    tm = first_m + r % rows;
-    tn = r / rows;
-  }
-}
-
-// registers -> swizzled patch for the 32-column block CB of a thread's 128 sums: scale, bias
-template <int CB>
-__device__ __forceinline__ void patch_write(const float (&sum)[128], float4* patch, int lane, float f1,
-                                            float f2, const float* bias_u, int colb, int N) {
-#pragma unroll
-  for (int c4 = 0; c4 < 8; ++c4) {
-    float4 v = make_float4(sum[CB * 32 + c4 * 4] * f1 * f2, sum[CB * 32 + c4 * 4 + 1] * f1 * f2,
-                           sum[CB * 32 + c4 * 4 + 2] * f1 * f2, sum[CB * 32 + c4 * 4 + 3] * f1 * f2);
-    if (bias_u) {
-      const int c = colb + c4 * 4;
-      if (c + 3 < N) {
-        const float4 b = *reinterpret_cast<const float4*>(bias_u + c);
-        v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-      } else {
-        if (c < N) v.x += bias_u[c];
-        if (c + 1 < N) v.y += bias_u[c + 1];
-        if (c + 2 < N) v.z += bias_u[c + 2];
-      }
-    }
-    patch[lane * 8 + (c4 ^ (lane & 7))] = v;
-  }
-}
-
 // flags: 1 accumulate into D, 2 ReLU in place, 8 statistics of relu(D) instead of D
 // CL = 2: one CTA pair per tile.  CL = 4: a cluster of two pairs on adjacent tile columns (tm, 2j)
 // and (tm, 2j+1); they need the same A rows, so each CTA fetches only half of its A tile and TMA
@@ -201,14 +148,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t bar_base = smem_base + STAGES * STAGE_BYTES;
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + 2 + a); };
-  const uint32_t tmem_ptr_smem = bar_base + 8u * (2 * STAGES + 4);
-  volatile uint32_t* tmem_ptr_gen =
-      reinterpret_cast<volatile uint32_t*>(smem_gen + STAGES * STAGE_BYTES + 8 * (2 * STAGES + 4));
+  const Barriers<STAGES> bar{smem_base + STAGES * STAGE_BYTES};
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t cl_rank = cluster_ctarank();          // 0..CL-1
@@ -222,24 +162,11 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
     tma_prefetch_desc(&map_a_l);
     tma_prefetch_desc(&map_b_h);
     tma_prefetch_desc(&map_b_l);
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), CL / 2);   // one tcgen05.commit per pair that reads (or feeds) this stage
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), 16);   // one arrival per epilogue warp of both CTAs
-    }
-    fence_barrier_init();
+    // empty: one tcgen05.commit per pair that reads (or feeds) a stage; tmem_empty: one arrival per
+    // epilogue warp of both CTAs
+    bar.init(CL / 2, 16);
   }
-  if (warp == 1) {
-    tmem_alloc<2>(tmem_ptr_smem, TMEM_COLS);
-    tmem_relinquish<2>();
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_gen;
+  const uint32_t tmem_base = tmem_setup<2>(bar, smem_gen + STAGES * STAGE_BYTES, warp, TMEM_COLS);
 
   const int tiles_m = (M + TILE_M - 1) / TILE_M;
   const int tiles_n = (N + UMMA_N - 1) / UMMA_N;
@@ -248,22 +175,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
   const int num_kb = (K + BK - 1) / BK;
   const int group = blockIdx.x / CL;
   const int num_groups = gridDim.x / CL;
-  // work units: whole-K tiles [0, t_full), then the ragged last wave cut into tail_split K ranges
-  // (fixed-order read-modify-write behind a per-tile arrival counter, see gemm_tc.cu)
-  const int tail_rem = num_tiles - t_full;
-  const int num_units = t_full + tail_rem * tail_split;
-  const int kb_per_split = (num_kb + tail_split - 1) / tail_split;
-  auto decode = [&](int u, int& t, int& sp, int& kb_begin, int& kb_end) {
-    if (u < t_full) {
-      t = u; sp = 0; kb_begin = 0; kb_end = num_kb;
-    } else {
-      const int j = u - t_full;
-      t = t_full + j % tail_rem;
-      sp = j / tail_rem;
-      kb_begin = sp * kb_per_split;
-      kb_end = min(num_kb, kb_begin + kb_per_split);
-    }
-  };
+  const WorkUnits work(t_full, tail_split, num_tiles, num_kb);
 
   if (warp == 0) {
     // ================= TMA producer =================
@@ -271,26 +183,26 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int u = group; u < num_units; u += num_groups) {
+      for (int u = group; u < work.num_units; u += num_groups) {
         int t, sp, kb_begin, kb_end;
-        decode(u, t, sp, kb_begin, kb_end);
+        work.decode(u, t, sp, kb_begin, kb_end);
         int tm, tn;
         tile_coords((flags & 32) ? num_tiles - 1 - t : t, tiles_m, tiles_ns, group_m, tm, tn);
         if constexpr (CL == 4) tn = 2 * tn + (int)pair;
         const int row_a = tm * TILE_M + (int)cta_rank * ROWS;
         const int row_b = tn * UMMA_N + (int)cta_rank * ROWS;   // (beyond N for the odd pair of a ragged row: zero fill)
         for (int kb = kb_begin; kb < kb_end; ++kb) {
-          mbar_wait(empty_bar(stage), phase ^ 1u);
+          mbar_wait(bar.empty(stage), phase ^ 1u);
           const uint32_t sa_h = smem_base + stage * STAGE_BYTES;
           const uint32_t sa_l = sa_h + PLANE_BYTES;
           const uint32_t sb_h = sa_h + 2 * PLANE_BYTES;
           const uint32_t sb_l = sa_h + 3 * PLANE_BYTES;
-          if (leader) mbar_expect_tx(full_bar(stage), (uint32_t)STAGE_BYTES * 2u);
+          if (leader) mbar_expect_tx(bar.full(stage), (uint32_t)STAGE_BYTES * 2u);
           const int k0 = kb * BK;
           if (flags & 128) {
             // TIMING EXPERIMENT (TNN_EXP_FLAGS, results are wrong): no operand fetch
             if (leader)
-              asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(full_bar(stage)), "r"((uint32_t)STAGE_BYTES * 2u) : "memory");
+              asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(bar.full(stage)), "r"((uint32_t)STAGE_BYTES * 2u) : "memory");
             if (++stage == STAGES) { stage = 0; phase ^= 1u; }
             continue;
           }
@@ -328,36 +240,36 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
             const uint32_t off = pair * (uint32_t)(PLANE_BYTES / 2);
             const int ra = row_a + 64 * (int)pair;
             if constexpr (A_MN) {
-              tma_load_2d_pair_mc(sa_l + off, &map_a_l, full_bar(stage), ra, k0, mc);
-              tma_load_2d_pair_mc(sa_h + off, &map_a_h, full_bar(stage), ra, k0, mc);
+              tma_load_2d_pair_mc(sa_l + off, &map_a_l, bar.full(stage), ra, k0, mc);
+              tma_load_2d_pair_mc(sa_h + off, &map_a_h, bar.full(stage), ra, k0, mc);
             } else {
-              tma_load_2d_pair_mc(sa_l + off, &map_a_l, full_bar(stage), k0, ra, mc);
-              tma_load_2d_pair_mc(sa_h + off, &map_a_h, full_bar(stage), k0, ra, mc);
+              tma_load_2d_pair_mc(sa_l + off, &map_a_l, bar.full(stage), k0, ra, mc);
+              tma_load_2d_pair_mc(sa_h + off, &map_a_h, bar.full(stage), k0, ra, mc);
             }
           } else if constexpr (A_MN) {
 #pragma unroll
             for (int j = 0; j < ROWS / 64; ++j) {
-              tma_load_2d<2>(sa_l + j * MN_BOX_BYTES, &map_a_l, full_bar(stage), row_a + 64 * j, k0);
-              tma_load_2d<2>(sa_h + j * MN_BOX_BYTES, &map_a_h, full_bar(stage), row_a + 64 * j, k0);
+              tma_load_2d<2>(sa_l + j * MN_BOX_BYTES, &map_a_l, bar.full(stage), row_a + 64 * j, k0);
+              tma_load_2d<2>(sa_h + j * MN_BOX_BYTES, &map_a_h, bar.full(stage), row_a + 64 * j, k0);
             }
           } else {
 #pragma unroll
             for (int j = 0; j < ROWS / KBOX_ROWS; ++j) {
-              tma_load_2d<2>(sa_l + j * KBOX_ROWS * 128, &map_a_l, full_bar(stage), k0, row_a + j * KBOX_ROWS);
-              tma_load_2d<2>(sa_h + j * KBOX_ROWS * 128, &map_a_h, full_bar(stage), k0, row_a + j * KBOX_ROWS);
+              tma_load_2d<2>(sa_l + j * KBOX_ROWS * 128, &map_a_l, bar.full(stage), k0, row_a + j * KBOX_ROWS);
+              tma_load_2d<2>(sa_h + j * KBOX_ROWS * 128, &map_a_h, bar.full(stage), k0, row_a + j * KBOX_ROWS);
             }
           }
           if constexpr (B_MN) {
 #pragma unroll
             for (int j = 0; j < ROWS / 64; ++j) {
-              tma_load_2d<2>(sb_h + j * MN_BOX_BYTES, &map_b_h, full_bar(stage), row_b + 64 * j, k0);
-              tma_load_2d<2>(sb_l + j * MN_BOX_BYTES, &map_b_l, full_bar(stage), row_b + 64 * j, k0);
+              tma_load_2d<2>(sb_h + j * MN_BOX_BYTES, &map_b_h, bar.full(stage), row_b + 64 * j, k0);
+              tma_load_2d<2>(sb_l + j * MN_BOX_BYTES, &map_b_l, bar.full(stage), row_b + 64 * j, k0);
             }
           } else {
 #pragma unroll
             for (int j = 0; j < ROWS / KBOX_ROWS; ++j) {
-              tma_load_2d<2>(sb_h + j * KBOX_ROWS * 128, &map_b_h, full_bar(stage), k0, row_b + j * KBOX_ROWS);
-              tma_load_2d<2>(sb_l + j * KBOX_ROWS * 128, &map_b_l, full_bar(stage), k0, row_b + j * KBOX_ROWS);
+              tma_load_2d<2>(sb_h + j * KBOX_ROWS * 128, &map_b_h, bar.full(stage), k0, row_b + j * KBOX_ROWS);
+              tma_load_2d<2>(sb_l + j * KBOX_ROWS * 128, &map_b_l, bar.full(stage), k0, row_b + j * KBOX_ROWS);
             }
           }
           if (++stage == STAGES) {
@@ -379,14 +291,14 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
 #ifdef TNN_F16_PROBE
       long long w_full = 0, w_empty = 0, t_begin = clock64();
 #endif
-      for (int u = group; u < num_units; u += num_groups) {
+      for (int u = group; u < work.num_units; u += num_groups) {
         int t, sp, kb_begin, kb_end;
-        decode(u, t, sp, kb_begin, kb_end);
+        work.decode(u, t, sp, kb_begin, kb_end);
         for (int kb0 = kb_begin; kb0 < kb_end; kb0 += CHUNK_KB) {
 #ifdef TNN_F16_PROBE
           long long p0 = clock64();
 #endif
-          mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
+          mbar_wait(bar.tempty(acc), acc_phase ^ 1u);
 #ifdef TNN_F16_PROBE
           w_empty += clock64() - p0;
 #endif
@@ -397,7 +309,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
 #ifdef TNN_F16_PROBE
             long long p1 = clock64();
 #endif
-            mbar_wait(full_bar(stage), phase);
+            mbar_wait(bar.full(stage), phase);
 #ifdef TNN_F16_PROBE
             w_full += clock64() - p1;
 #endif
@@ -420,13 +332,13 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
               umma_bf16<2>(tmem_d, da_h, db_l, idesc, 1u);
               umma_bf16<2>(tmem_d, da_h, db_h, idesc, 1u);
             }
-            umma_commit_pair_mask(empty_bar(stage), CL == 4 ? (uint16_t)15 : (uint16_t)3);
+            umma_commit_pair_mask(bar.empty(stage), CL == 4 ? (uint16_t)15 : (uint16_t)3);
             if (++stage == STAGES) {
               stage = 0;
               phase ^= 1u;
             }
           }
-          umma_commit_pair_mask(tfull_bar(acc), pair_mask);
+          umma_commit_pair_mask(bar.tfull(acc), pair_mask);
           if (++acc == 2) {
             acc = 0;
             acc_phase ^= 1u;
@@ -458,9 +370,9 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
     long long ep_wait = 0, ep_store = 0;
     const long long ep_begin = clock64();
 #endif
-    for (int u = group; u < num_units; u += num_groups) {
+    for (int u = group; u < work.num_units; u += num_groups) {
       int t, sp, kb_begin, kb_end;
-      decode(u, t, sp, kb_begin, kb_end);
+      work.decode(u, t, sp, kb_begin, kb_end);
       const bool accumulate = (flags & 1) || sp > 0;
       const bool final_unit = (u < t_full || sp + 1 == tail_split);
       const bool emit_act = act_out != nullptr && final_unit;
@@ -479,13 +391,16 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
 #ifdef TNN_F16_PROBE
         const long long q0 = clock64();
 #endif
-        mbar_wait(tfull_bar(acc), acc_phase);
+        mbar_wait(bar.tfull(acc), acc_phase);
 #ifdef TNN_F16_PROBE
         ep_wait += clock64() - q0;
 #endif
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) +
                                (uint32_t)(acc * UMMA_N + half * 128);
+        // The chunk drain here and the split-K ordering wait below are written out in this kernel
+        // (gemm_tc.cu has its own copies) rather than taken from tc_gemm.cuh: as shared helpers they
+        // change this kernel's register allocation and spill layout, and this is the hot kernel.
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           uint32_t r[32];
@@ -494,9 +409,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
 #pragma unroll
           for (int j = 0; j < 32; ++j) sum[c * 32 + j] += __uint_as_float(r[j]);
         }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster_relaxed(tempty_bar(acc), 2 * pair);
+        tmem_hand_back<true>(bar.tempty(acc), 2 * pair, lane);
         if (++acc == 2) {
           acc = 0;
           acc_phase ^= 1u;
@@ -541,12 +454,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
         for (int cb = 0; cb < 4; ++cb) {
           const int colb = col0 + cb * 32;
           if (colb >= N) break;                                 // warp-uniform
-          switch (cb) {                                         // register indices are compile-time
-            case 0: patch_write<0>(sum, patch, lane, f1, f2, bias_u, colb, N); break;
-            case 1: patch_write<1>(sum, patch, lane, f1, f2, bias_u, colb, N); break;
-            case 2: patch_write<2>(sum, patch, lane, f1, f2, bias_u, colb, N); break;
-            default: patch_write<3>(sum, patch, lane, f1, f2, bias_u, colb, N); break;
-          }
+          patch_write<true>(cb, sum, patch, lane, f1, f2, bias_u, colb, N);
           __syncwarp();
           const int gcol = colb + c4l * 4;
           if (rows_aligned && act_aligned && colb + 32 <= N) {
@@ -664,11 +572,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
 #ifdef TNN_F16_PROBE
       ep_store += clock64() - q1;
 #endif
-      if (u >= t_full && sp + 1 < tail_split && tile_valid) {
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) atomicAdd(tile_flags + flag_idx, 1u);
-      }
+      if (u >= t_full && sp + 1 < tail_split && tile_valid) splitk_publish(tile_flags, flag_idx, lane);
     }
 #ifdef TNN_F16_PROBE
     if ((group == 0 || group == 37) && warp == 4 && lane == 0 && cta_rank == 0)
@@ -682,13 +586,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_a_h, const __grid_cons
     }
   }
 
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<2>(tmem_base, TMEM_COLS);
-  }
+  tmem_teardown<2>(warp, tmem_base, TMEM_COLS);
 }
 
 // ---- statistics + split ---------------------------------------------------------------------------
@@ -795,40 +693,16 @@ split_f16_kernel(const float* __restrict__ x, int64_t R, int64_t C, __half* __re
 }
 
 // ---- host side ---------------------------------------------------------------------------------
-static PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-
-static int get_encode_fn() {
-  if (g_encode) return 0;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  TNN_CUDA(cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &qres));
-  if (qres != cudaDriverEntryPointSuccess || !fn) TNN_FAIL("cuTensorMapEncodeTiled is not available");
-  g_encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
-  return 0;
+// 16-bit plane.  K-major [rows, K]: box {64 k, box_rows}.  MN-major [K, rows]: box {64 mn, 64 k}.
+// 128-byte swizzle both ways.
+static int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t K, int64_t ld, bool mn_major,
+                    int box_rows) {
+  return tc::make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, ptr, rows, K, ld, mn_major, mn_major ? 64 : BK,
+                      mn_major ? BK : box_rows,
+                      (mn_major || BK == 64) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                      "f16 GEMM: operand plane", "f16 GEMM: operand pitch", " (f16 planes)");
 }
 
-// 16-bit plane.  K-major [rows, K] (pitch ld): box {64 k, 128 rows}.  MN-major [K, rows] (pitch
-// ld): box {64 mn, 64 k}.  128-byte swizzle both ways.
-static int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t K, int64_t ld,
-                    bool mn_major, int box_rows = ROWS) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) TNN_FAIL("f16 GEMM: operand plane must be 16-byte aligned");
-  if (ld % 8 != 0) TNN_FAIL("f16 GEMM: operand pitch must be a multiple of 8 elements");
-  cuuint64_t dims[2] = {(cuuint64_t)(mn_major ? rows : K), (cuuint64_t)(mn_major ? K : rows)};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)(mn_major ? 64 : BK), (cuuint32_t)(mn_major ? BK : box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2,
-                        (void*)ptr, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        (mn_major || BK == 64) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) TNN_FAIL("cuTensorMapEncodeTiled (f16 planes) failed with code " + std::to_string((int)r));
-  return 0;
-}
-
-static unsigned int* g_tile_flags = nullptr;
-constexpr int MAX_FLAG_TILES = 1 << 16;
-static bool g_attr_set[2][2][2] = {};
 static int g_group_m = -8;     // tile rasterisation: panels of 8 tile columns measured 1-2 % ahead of row-major;
                                // (TNN_F16_GROUP_M), see tile_coords
 static bool g_reverse = true;  // tiles in descending order (TNN_F16_REVERSE=0: ascending): the product starts on
@@ -850,63 +724,17 @@ static int launch(float* D, int64_t ldd, const void* a_h, const void* a_l, int64
   if (make_map(&ma_l, a_l, M, K, lda, A_MN, CL == 4 ? 64 : KBOX_ROWS)) return 1;
   if (make_map(&mb_h, b_h, N, K, ldb, B_MN, KBOX_ROWS)) return 1;
   if (make_map(&mb_l, b_l, N, K, ldb, B_MN, KBOX_ROWS)) return 1;
-  auto kern = gemm_f16x3_kernel<A_MN, B_MN, CL>;
-  if (!g_attr_set[A_MN][B_MN][CL == 4]) {
-    TNN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    g_attr_set[A_MN][B_MN][CL == 4] = true;
-  }
   const int64_t tiles_m = ceil_div(M, TILE_M), tiles_n = ceil_div(N, UMMA_N);
   const int64_t tiles = tiles_m * (CL == 4 ? ceil_div(tiles_n, 2) : tiles_n);   // scheduling units
-  const int max_groups = std::max(1, (ctx().sm_count - tc::g_reserved_sms) / CL);
-  int t_full = (int)tiles, tail_split = 1;
-  if (!(flags & 2) && tiles_m * tiles_n <= MAX_FLAG_TILES) {
-    const int64_t num_kb = ceil_div(K, BK);
-    const int64_t rem = tiles % max_groups;
-    if (rem > 0) {
-      int s = 1;
-      while (s < 4 && rem * (s * 2) <= max_groups && num_kb / (s * 2) >= 512 / BK) s *= 2;
-      if (s > 1) {
-        t_full = (int)(tiles - rem);
-        tail_split = s;
-      }
-    }
-  }
-  if (tail_split > 1) {
-    if (!g_tile_flags) TNN_CUDA(cudaMalloc(&g_tile_flags, MAX_FLAG_TILES * sizeof(unsigned int)));
-    TNN_CUDA(cudaMemsetAsync(g_tile_flags, 0, (size_t)(tiles_m * tiles_n) * sizeof(unsigned int), ctx().stream));
-  }
-  const int64_t units = t_full + (tiles - t_full) * tail_split;
-  const int groups = (int)std::min<int64_t>(units, max_groups);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(groups * CL));
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = SMEM_BYTES;
-  cfg.stream = ctx().stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if constexpr (CL == 4) {
-    // a persistent grid must be co-resident: 4-CTA clusters do not tile every GPC (B200: 33 of the
-    // 37 that 148 SMs would hold), and a cluster that cannot start waits for a whole one to finish
-    static int max_clusters = 0;
-    if (!max_clusters) {
-      TNN_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
-      if (max_clusters < 1) max_clusters = 1;
-    }
-    if (groups > max_clusters) cfg.gridDim = dim3((unsigned)(max_clusters * CL));
-  }
+  const int groups = tc::max_groups(CL);
+  const tc::TailPlan plan = tc::plan_tail(flags, tiles, tiles_m * tiles_n, groups, ceil_div(K, BK), 512 / BK);
+  if (tc::clear_tile_flags(plan, tiles_m * tiles_n)) return 1;
   // rasterisation knob in scheduling units: a panel of g tile columns = g/2 units when CL = 4
   const int gm = (CL == 4 && g_group_m < 0) ? std::min(-1, g_group_m / 2) : g_group_m;
-  prof_begin(1);
-  TNN_CUDA(cudaLaunchKernelEx(&cfg, kern, ma_h, ma_l, mb_h, mb_l, D, ldd, (int)M, (int)N, (int)K, bias, flags,
-                              t_full, tail_split, g_tile_flags, act_out, mask_src, meta_a, meta_b, stat_out, gm));
-  ctx().launches++;
-  prof_end(1);
-  return 0;
+  return tc::launch_persistent<gemm_f16x3_kernel<A_MN, B_MN, CL>>(
+      CL, NUM_THREADS, SMEM_BYTES, plan.t_full + (tiles - plan.t_full) * plan.tail_split, groups, CL == 4, 1, ma_h,
+      ma_l, mb_h, mb_l, D, ldd, (int)M, (int)N, (int)K, bias, flags, plan.t_full, plan.tail_split, tc::g_tile_flags,
+      act_out, mask_src, meta_a, meta_b, stat_out, gm);
 }
 
 template <int CL>
@@ -986,14 +814,12 @@ int tnn_gemm_f16x3(float* D, int64_t ldd, const void* a_hf, const void* a_l16, i
                    const void* a_meta, const void* b_hf, const void* b_l16, int64_t ldb,
                    const void* b_meta, int64_t M, int64_t N, int64_t K, const float* bias, int flags,
                    int layout, float* act_out, const float* mask_src, void* stat_meta) {
-  TNN_REQUIRE_INIT();
-  if (M <= 0 || N <= 0) return 0;
-  if (K <= 0) TNN_FAIL("tnn_gemm_f16x3: K must be positive");
-  if (M > 2147483647LL || N > 2147483647LL || K > 2147483647LL) TNN_FAIL("tnn_gemm_f16x3: extent above int32");
+  bool empty;
+  if (tc::gemm_entry_checks("tnn_gemm_f16x3", M, N, K, empty)) return 1;
+  if (empty) return 0;
   if (!a_meta || !b_meta) TNN_FAIL("tnn_gemm_f16x3: operand meta records are required");
   if (mask_src && !act_out) TNN_FAIL("tnn_gemm_f16x3: the mask_src form needs act_out");
   if (act_out && (flags & 2)) TNN_FAIL("tnn_gemm_f16x3: act_out and the relu-in-place flag are exclusive");
-  if (f16::get_encode_fn()) return 1;
   if (getenv("TNN_EXP_FLAGS")) flags |= atoi(getenv("TNN_EXP_FLAGS")) & (128 | 256);
   static bool env_read = false;
   if (!env_read) {

@@ -42,6 +42,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "tc_gemm.cuh"
 
 namespace tnn {
 namespace tc {
@@ -71,12 +72,6 @@ struct Cfg {
   static constexpr int EPI_PATCH_BYTES = 8 * 4096;                // one 32x32 fp32 patch per epilogue warp
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/ + EPI_PATCH_BYTES;
 };
-
-}  // namespace tc
-}  // namespace tnn
-#include "tc_ptx.cuh"
-namespace tnn {
-namespace tc {
 
 // Operand tiles in shared memory (one plane of one 32-wide K block, rows = 128 M/N rows):
 //   K-major  : one TMA box {32 k, rows}: row r at r*128 B, k contiguous, 128-byte swizzle.
@@ -126,57 +121,6 @@ __host__ __device__ constexpr uint32_t make_idesc16(int m, int n, bool a_mn, boo
          ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 
-// Tile rasterisation: consecutive tile ids walk group_m tile-rows before moving to the next tile
-// column.  group_m = 1 (row-major: the ~74 concurrent CTA pairs share ~5 A row-blocks and sweep
-// all B column-blocks) measured fastest on the wide-MLP shapes; squarer patches (4/8/16) lost
-// 1-15 %, so 1 is the default and the knob stays for other shapes.
-__device__ __forceinline__ void tile_coords(int t, int tiles_m, int tiles_n, int group_m, int& tm,
-                                            int& tn) {
-  if (group_m < 0) {
-    // column panels: all tile rows of a panel of -group_m tile columns (row-major inside the panel)
-    // before the next panel, so the panel's B operand stays L2-resident across waves
-    const int gn = -group_m;
-    const int per_panel = tiles_m * gn;
-    const int g = t / per_panel;
-    const int first_n = g * gn;
-    const int cols = min(gn, tiles_n - first_n);
-    const int r = t - g * per_panel;
-    tm = r / cols;
-    tn = first_n + r % cols;
-    return;
-  }
-  const int per_group = group_m * tiles_n;
-  const int g = t / per_group;
-  const int first_m = g * group_m;
-  const int rows = min(group_m, tiles_m - first_m);
-  const int r = t - g * per_group;
-  tm = first_m + r % rows;
-  tn = r / rows;
-}
-
-// registers -> swizzled patch for the 32-column block CB of a thread's 128 sums (+ bias)
-template <int CB>
-__device__ __forceinline__ void patch_write_tc(const float (&sum)[128], float4* patch, int lane,
-                                               const float* bias_u, int colb, int N) {
-#pragma unroll
-  for (int c4 = 0; c4 < 8; ++c4) {
-    float4 v = make_float4(sum[CB * 32 + c4 * 4], sum[CB * 32 + c4 * 4 + 1], sum[CB * 32 + c4 * 4 + 2],
-                           sum[CB * 32 + c4 * 4 + 3]);
-    if (bias_u) {
-      const int c = colb + c4 * 4;
-      if (c + 3 < N) {
-        const float4 b = *reinterpret_cast<const float4*>(bias_u + c);
-        v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-      } else {
-        if (c < N) v.x += bias_u[c];
-        if (c + 1 < N) v.y += bias_u[c + 1];
-        if (c + 2 < N) v.z += bias_u[c + 2];
-      }
-    }
-    patch[lane * 8 + (c4 ^ (lane & 7))] = v;
-  }
-}
-
 // ---- the GEMM kernel ---------------------------------------------------------------------------
 // MIX = false: planes are (hi, lo) tf32, map_*_lo = the lo plane, map_*_l16 unused.
 // MIX = true : planes are (hi tf32, h16 = bf16(x), l16 = bf16(x - hi)); map_*_lo = h16.
@@ -203,15 +147,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
   // SWIZZLE_128B tiles need 1024-byte alignment
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t bar_base = smem_base + C::STAGES * C::STAGE_BYTES;
-  // barrier layout: full[STAGES], empty[STAGES], tmem_full[2], tmem_empty[2], tmem ptr
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (C::STAGES + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * C::STAGES + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * C::STAGES + 2 + a); };
-  const uint32_t tmem_ptr_smem = bar_base + 8u * (2 * C::STAGES + 4);
-  volatile uint32_t* tmem_ptr_gen =
-      reinterpret_cast<volatile uint32_t*>(smem_gen + C::STAGES * C::STAGE_BYTES + 8 * (2 * C::STAGES + 4));
+  const Barriers<C::STAGES> bar{smem_base + C::STAGES * C::STAGE_BYTES};
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t cta_rank = CG == 1 ? 0u : cluster_ctarank();
@@ -226,25 +162,9 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
       tma_prefetch_desc(&map_a_l16);
       tma_prefetch_desc(&map_b_l16);
     }
-    for (int s = 0; s < C::STAGES; ++s) {
-      mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), 8 * CG);  // one arrival per epilogue warp of every CTA in the group
-    }
-    fence_barrier_init();
+    bar.init(1, 8 * CG);   // tmem_empty: one arrival per epilogue warp of every CTA in the group
   }
-  if (warp == 1) {
-    tmem_alloc<CG>(tmem_ptr_smem, TMEM_COLS);
-    tmem_relinquish<CG>();
-  }
-  tc_fence_before();
-  if constexpr (CG == 1) __syncthreads();
-  else cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_gen;
+  const uint32_t tmem_base = tmem_setup<CG>(bar, smem_gen + C::STAGES * C::STAGE_BYTES, warp, TMEM_COLS);
 
   const int tiles_m = (M + C::TILE_M - 1) / C::TILE_M;
   const int tiles_n = (N + UMMA_N - 1) / UMMA_N;
@@ -252,26 +172,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
   const int num_kb = (K + BK - 1) / BK;
   const int group = blockIdx.x / CG;            // CTA (pair) index
   const int num_groups = gridDim.x / CG;
-  // Work units.  Tiles [0, t_full) are whole-K units.  The remaining "tail" tiles -- the ones that
-  // would form a ragged last wave (4096x4096 dW product: 256 tiles on 74 CTA pairs = 3 full waves
-  // + 34 tiles) -- are cut into tail_split K ranges each, so the last wave is short AND full:
-  // unit t_full + j covers tile t_full + j % rem, K range j / rem.  Range s > 0 adds onto what
-  // range s-1 stored, in that fixed order (a per-tile arrival counter gates the read-modify-write;
-  // never a floating-point atomic), so the result does not depend on timing.
-  const int tail_rem = num_tiles - t_full;
-  const int num_units = t_full + tail_rem * tail_split;
-  const int kb_per_split = (num_kb + tail_split - 1) / tail_split;
-  auto decode = [&](int u, int& t, int& sp, int& kb_begin, int& kb_end) {
-    if (u < t_full) {
-      t = u; sp = 0; kb_begin = 0; kb_end = num_kb;
-    } else {
-      const int j = u - t_full;
-      t = t_full + j % tail_rem;
-      sp = j / tail_rem;
-      kb_begin = sp * kb_per_split;
-      kb_end = min(num_kb, kb_begin + kb_per_split);
-    }
-  };
+  const WorkUnits work(t_full, tail_split, num_tiles, num_kb);
 
   // Register budget: the compiler is held to 168 registers per thread by the 384-thread block; the
   // epilogue warps carry 128 fp32 tile sums each, so warpgroup 0 (TMA + MMA issue, a handful of
@@ -283,15 +184,15 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int u = group; u < num_units; u += num_groups) {
+      for (int u = group; u < work.num_units; u += num_groups) {
         int t, sp, kb_begin, kb_end;
-        decode(u, t, sp, kb_begin, kb_end);
+        work.decode(u, t, sp, kb_begin, kb_end);
         int tm, tn;
         tile_coords(t, tiles_m, tiles_n, group_m, tm, tn);
         const int row_a = tm * C::TILE_M + (int)cta_rank * ROWS_A;
         const int row_b = tn * UMMA_N + (int)cta_rank * C::ROWS_B;
         for (int kb = kb_begin; kb < kb_end; ++kb) {
-          mbar_wait(empty_bar(stage), phase ^ 1u);
+          mbar_wait(bar.empty(stage), phase ^ 1u);
           const uint32_t sa_hi = smem_base + stage * C::STAGE_BYTES;
           const uint32_t sa_lo = sa_hi + C::A_BYTES;
           const uint32_t sb_hi = sa_hi + C::A_PLANES_BYTES;
@@ -303,34 +204,34 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
           const bool exp_skip_hi = MIX && (flags & 1024);   // timing experiment: 16-bit planes only
           const uint32_t tx_bytes = (uint32_t)(C::STAGE_BYTES - (exp_skip_h16 ? (C::A_BYTES + C::B_BYTES) / 2 : 0)
                                                - (exp_skip_hi ? (C::A_BYTES + C::B_BYTES) : 0)) * CG;
-          if (leader) mbar_expect_tx(full_bar(stage), tx_bytes);
+          if (leader) mbar_expect_tx(bar.full(stage), tx_bytes);
           const int k0 = kb * BK;
           if (flags & 128) {
             // timing experiment: no operand fetch at all (the MMAs run on whatever the stage holds);
             // the transaction count armed above is satisfied by hand
             if (leader)
-              asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(full_bar(stage)), "r"(tx_bytes) : "memory");
+              asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(bar.full(stage)), "r"(tx_bytes) : "memory");
           } else
           if constexpr (!MIX) {
             if constexpr (A_MN) {
 #pragma unroll
               for (int j = 0; j < ROWS_A / 32; ++j) {
-                tma_load_2d<CG>(sa_hi + j * MN_BOX_BYTES, &map_a_hi, full_bar(stage), row_a + 32 * j, k0);
-                tma_load_2d<CG>(sa_lo + j * MN_BOX_BYTES, &map_a_lo, full_bar(stage), row_a + 32 * j, k0);
+                tma_load_2d<CG>(sa_hi + j * MN_BOX_BYTES, &map_a_hi, bar.full(stage), row_a + 32 * j, k0);
+                tma_load_2d<CG>(sa_lo + j * MN_BOX_BYTES, &map_a_lo, bar.full(stage), row_a + 32 * j, k0);
               }
             } else {
-              tma_load_2d<CG>(sa_hi, &map_a_hi, full_bar(stage), k0, row_a);
-              tma_load_2d<CG>(sa_lo, &map_a_lo, full_bar(stage), k0, row_a);
+              tma_load_2d<CG>(sa_hi, &map_a_hi, bar.full(stage), k0, row_a);
+              tma_load_2d<CG>(sa_lo, &map_a_lo, bar.full(stage), k0, row_a);
             }
             if constexpr (B_MN) {
 #pragma unroll
               for (int j = 0; j < C::ROWS_B / 32; ++j) {
-                tma_load_2d<CG>(sb_hi + j * MN_BOX_BYTES, &map_b_hi, full_bar(stage), row_b + 32 * j, k0);
-                tma_load_2d<CG>(sb_lo + j * MN_BOX_BYTES, &map_b_lo, full_bar(stage), row_b + 32 * j, k0);
+                tma_load_2d<CG>(sb_hi + j * MN_BOX_BYTES, &map_b_hi, bar.full(stage), row_b + 32 * j, k0);
+                tma_load_2d<CG>(sb_lo + j * MN_BOX_BYTES, &map_b_lo, bar.full(stage), row_b + 32 * j, k0);
               }
             } else {
-              tma_load_2d<CG>(sb_hi, &map_b_hi, full_bar(stage), k0, row_b);
-              tma_load_2d<CG>(sb_lo, &map_b_lo, full_bar(stage), k0, row_b);
+              tma_load_2d<CG>(sb_hi, &map_b_hi, bar.full(stage), k0, row_b);
+              tma_load_2d<CG>(sb_lo, &map_b_lo, bar.full(stage), k0, row_b);
             }
           } else {
             // the second 32-bit plane's space holds the two bf16 planes
@@ -339,30 +240,30 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
             if constexpr (A_MN) {
 #pragma unroll
               for (int j = 0; j < ROWS_A / 32; ++j)
-                if (!exp_skip_hi) tma_load_2d<CG>(sa_hi + j * MN_BOX_BYTES, &map_a_hi, full_bar(stage), row_a + 32 * j, k0);
+                if (!exp_skip_hi) tma_load_2d<CG>(sa_hi + j * MN_BOX_BYTES, &map_a_hi, bar.full(stage), row_a + 32 * j, k0);
 #pragma unroll
               for (int j = 0; j < ROWS_A / 64; ++j) {
-                if (!exp_skip_h16) tma_load_2d<CG>(sa_h16 + j * MN_BOX_BYTES, &map_a_lo, full_bar(stage), row_a + 64 * j, k0);
-                tma_load_2d<CG>(sa_l16 + j * MN_BOX_BYTES, &map_a_l16, full_bar(stage), row_a + 64 * j, k0);
+                if (!exp_skip_h16) tma_load_2d<CG>(sa_h16 + j * MN_BOX_BYTES, &map_a_lo, bar.full(stage), row_a + 64 * j, k0);
+                tma_load_2d<CG>(sa_l16 + j * MN_BOX_BYTES, &map_a_l16, bar.full(stage), row_a + 64 * j, k0);
               }
             } else {
-              if (!exp_skip_hi) tma_load_2d<CG>(sa_hi, &map_a_hi, full_bar(stage), k0, row_a);
-              if (!exp_skip_h16) tma_load_2d<CG>(sa_h16, &map_a_lo, full_bar(stage), k0, row_a);
-              tma_load_2d<CG>(sa_l16, &map_a_l16, full_bar(stage), k0, row_a);
+              if (!exp_skip_hi) tma_load_2d<CG>(sa_hi, &map_a_hi, bar.full(stage), k0, row_a);
+              if (!exp_skip_h16) tma_load_2d<CG>(sa_h16, &map_a_lo, bar.full(stage), k0, row_a);
+              tma_load_2d<CG>(sa_l16, &map_a_l16, bar.full(stage), k0, row_a);
             }
             if constexpr (B_MN) {
 #pragma unroll
               for (int j = 0; j < C::ROWS_B / 32; ++j)
-                if (!exp_skip_hi) tma_load_2d<CG>(sb_hi + j * MN_BOX_BYTES, &map_b_hi, full_bar(stage), row_b + 32 * j, k0);
+                if (!exp_skip_hi) tma_load_2d<CG>(sb_hi + j * MN_BOX_BYTES, &map_b_hi, bar.full(stage), row_b + 32 * j, k0);
 #pragma unroll
               for (int j = 0; j < C::ROWS_B / 64; ++j) {
-                if (!exp_skip_h16) tma_load_2d<CG>(sb_h16 + j * MN_BOX_BYTES, &map_b_lo, full_bar(stage), row_b + 64 * j, k0);
-                tma_load_2d<CG>(sb_l16 + j * MN_BOX_BYTES, &map_b_l16, full_bar(stage), row_b + 64 * j, k0);
+                if (!exp_skip_h16) tma_load_2d<CG>(sb_h16 + j * MN_BOX_BYTES, &map_b_lo, bar.full(stage), row_b + 64 * j, k0);
+                tma_load_2d<CG>(sb_l16 + j * MN_BOX_BYTES, &map_b_l16, bar.full(stage), row_b + 64 * j, k0);
               }
             } else {
-              if (!exp_skip_hi) tma_load_2d<CG>(sb_hi, &map_b_hi, full_bar(stage), k0, row_b);
-              if (!exp_skip_h16) tma_load_2d<CG>(sb_h16, &map_b_lo, full_bar(stage), k0, row_b);
-              tma_load_2d<CG>(sb_l16, &map_b_l16, full_bar(stage), k0, row_b);
+              if (!exp_skip_hi) tma_load_2d<CG>(sb_hi, &map_b_hi, bar.full(stage), k0, row_b);
+              if (!exp_skip_h16) tma_load_2d<CG>(sb_h16, &map_b_lo, bar.full(stage), k0, row_b);
+              tma_load_2d<CG>(sb_l16, &map_b_l16, bar.full(stage), k0, row_b);
             }
           }
           if (++stage == C::STAGES) {
@@ -383,16 +284,16 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      for (int u = group; u < num_units; u += num_groups) {
+      for (int u = group; u < work.num_units; u += num_groups) {
         int t, sp, kb_begin, kb_end;
-        decode(u, t, sp, kb_begin, kb_end);
+        work.decode(u, t, sp, kb_begin, kb_end);
         for (int kb0 = kb_begin; kb0 < kb_end; kb0 += CHUNK_KB) {
-          mbar_wait(tempty_bar(acc), acc_phase ^ 1u);   // epilogue has drained this accumulator
+          mbar_wait(bar.tempty(acc), acc_phase ^ 1u);   // epilogue has drained this accumulator
           tc_fence_after();
           const uint32_t tmem_d = tmem_base + (uint32_t)(acc * UMMA_N);
           const int kb1 = min(kb0 + CHUNK_KB, kb_end);
           for (int kb = kb0; kb < kb1; ++kb) {
-            mbar_wait(full_bar(stage), phase);
+            mbar_wait(bar.full(stage), phase);
             tc_fence_after();
             const uint32_t sa_hi = smem_base + stage * C::STAGE_BYTES;
             const uint32_t sa_lo = sa_hi + C::A_BYTES;
@@ -442,13 +343,13 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
                               make_smem_desc<B_MN>(sb_hi + koff_b), idesc, 1u);
               }
             }
-            umma_commit<CG>(empty_bar(stage));          // frees the smem slot when the MMAs retire
+            umma_commit<CG>(bar.empty(stage));          // frees the smem slot when the MMAs retire
             if (++stage == C::STAGES) {
               stage = 0;
               phase ^= 1u;
             }
           }
-          umma_commit<CG>(tfull_bar(acc));              // chunk complete -> epilogue may drain it
+          umma_commit<CG>(bar.tfull(acc));              // chunk complete -> epilogue may drain it
           if (++acc == 2) {
             acc = 0;
             acc_phase ^= 1u;
@@ -466,9 +367,9 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
     int acc = 0;
     uint32_t acc_phase = 0;
     const bool relu = flags & 2;
-    for (int u = group; u < num_units; u += num_groups) {
+    for (int u = group; u < work.num_units; u += num_groups) {
       int t, sp, kb_begin, kb_end;
-      decode(u, t, sp, kb_begin, kb_end);
+      work.decode(u, t, sp, kb_begin, kb_end);
       const bool accumulate = (flags & 1) || sp > 0;
       // the unit that holds the complete sum also emits the fused activation outputs
       // act_out may be NULL with the planes present: the fp32 ReLU output is then never written
@@ -483,7 +384,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
 #pragma unroll
       for (int j = 0; j < 128; ++j) sum[j] = 0.f;
       for (int kb0 = kb_begin; kb0 < kb_end; kb0 += CHUNK_KB) {
-        mbar_wait(tfull_bar(acc), acc_phase);
+        mbar_wait(bar.tfull(acc), acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) +
                                (uint32_t)(acc * UMMA_N + half * 128);
@@ -497,13 +398,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
             for (int j = 0; j < 32; ++j) sum[c * 32 + j] += __uint_as_float(r[j]);
           }
         }
-        // this warp is done reading the accumulator: hand it back to the MMA issuer
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          if constexpr (CG == 1) mbar_arrive(tempty_bar(acc));
-          else mbar_arrive_cluster_relaxed(tempty_bar(acc), 0);   // publishes no memory: no MEMBAR (see gemm_f16.cu)
-        }
+        tmem_hand_back<CG != 1>(bar.tempty(acc), 0, lane);
         if (++acc == 2) {
           acc = 0;
           acc_phase ^= 1u;
@@ -548,12 +443,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
           for (int cb = 0; cb < 4; ++cb) {
             const int colb = col0 + cb * 32;
             if (colb >= N) break;                               // warp-uniform
-            switch (cb) {                                       // register indices are compile-time
-              case 0: patch_write_tc<0>(sum, patch, lane, bias_u, colb, N); break;
-              case 1: patch_write_tc<1>(sum, patch, lane, bias_u, colb, N); break;
-              case 2: patch_write_tc<2>(sum, patch, lane, bias_u, colb, N); break;
-              default: patch_write_tc<3>(sum, patch, lane, bias_u, colb, N); break;
-            }
+            patch_write<false>(cb, sum, patch, lane, 1.f, 1.f, bias_u, colb, N);
             __syncwarp();
             const int gcol = colb + c4l * 4;
 #pragma unroll 1
@@ -581,24 +471,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
         for (int cb = 0; cb < 4; ++cb) {
           const int colb = col0 + cb * 32;                      // first column of this 32-wide block
           if (colb >= N) break;                                 // warp-uniform
-          // bias is per column: add it while the thread still owns consecutive columns
-#pragma unroll
-          for (int c4 = 0; c4 < 8; ++c4) {
-            float4 v = make_float4(sum[cb * 32 + c4 * 4], sum[cb * 32 + c4 * 4 + 1],
-                                   sum[cb * 32 + c4 * 4 + 2], sum[cb * 32 + c4 * 4 + 3]);
-            if (bias_u) {
-              const int c = colb + c4 * 4;
-              if (c + 3 < N) {
-                const float4 b = *reinterpret_cast<const float4*>(bias_u + c);
-                v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-              } else {
-                if (c < N) v.x += bias_u[c];
-                if (c + 1 < N) v.y += bias_u[c + 1];
-                if (c + 2 < N) v.z += bias_u[c + 2];
-              }
-            }
-            patch[lane * 8 + (c4 ^ (lane & 7))] = v;
-          }
+          patch_write<false>(cb, sum, patch, lane, 1.f, 1.f, bias_u, colb, N);   // (cb is unrolled)
           __syncwarp();
           // whatever the store has to READ first (the previous D for accumulate, the pre-activation
           // for the ReLU mask) is fetched for all 8 row groups up front: 8-16 independent 128-bit
@@ -704,25 +577,11 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi,
           __syncwarp();
         }
       }
-      if (u >= t_full && sp + 1 < tail_split) {
-        // publish: this warp's part of the tile is in global memory
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) atomicAdd(tile_flags + t, 1u);
-      }
+      if (u >= t_full && sp + 1 < tail_split) splitk_publish(tile_flags, t, lane);
     }
   }
 
-  // teardown: everyone (both CTAs of a pair) must be done before TMEM goes away.  The single-lane
-  // roles re-converge first: the cluster barrier and tcgen05.dealloc are .aligned instructions.
-  __syncwarp();
-  tc_fence_before();
-  if constexpr (CG == 1) __syncthreads();
-  else cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<CG>(tmem_base, TMEM_COLS);
-  }
+  tmem_teardown<CG>(warp, tmem_base, TMEM_COLS);
 }
 
 // ---- fp32 -> tf32 hi/lo split (+ optional transposed copy) ----------------------------------------
@@ -861,64 +720,30 @@ split_mix_cond2_kernel(SplitArgs a, SplitArgs b, const int* __restrict__ cond_a,
 }
 
 // ---- host side ---------------------------------------------------------------------------------
-static PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-
-static int get_encode_fn() {
-  if (g_encode) return 0;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  TNN_CUDA(cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &qres));
-  if (qres != cudaDriverEntryPointSuccess || !fn) TNN_FAIL("cuTensorMapEncodeTiled is not available");
-  g_encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
-  return 0;
-}
-
-// 2-D fp32 tensor [rows, K] with row pitch ld (elements); box = [BK, box_rows], 128-byte swizzle
-// K-major plane [rows, K] (pitch ld): box {BK k, box_rows}.  MN-major plane [K, rows] (pitch ld):
-// box {32 mn, BK k}.
+// fp32 plane.  K-major [rows, K]: box {BK k, box_rows}, 128-byte swizzle.  MN-major [K, rows]: box
+// {32 mn, BK k}, 128-byte swizzle with 32-byte atoms.
 static int make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t K, int64_t ld, int box_rows,
                     bool mn_major) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) TNN_FAIL("tf32x3 GEMM: operand plane must be 16-byte aligned");
-  if (ld % 4 != 0) TNN_FAIL("tf32x3 GEMM: operand pitch must be a multiple of 4 elements");
-  cuuint64_t dims[2] = {(cuuint64_t)(mn_major ? rows : K), (cuuint64_t)(mn_major ? K : rows)};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
-  cuuint32_t box[2] = {(cuuint32_t)(mn_major ? 32 : BK), (cuuint32_t)(mn_major ? BK : box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)ptr, dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) TNN_FAIL("cuTensorMapEncodeTiled failed with code " + std::to_string((int)r));
-  return 0;
+  return tc::make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, ptr, rows, K, ld, mn_major, mn_major ? 32 : BK,
+                      mn_major ? BK : box_rows,
+                      mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
+                      "tf32x3 GEMM: operand plane", "tf32x3 GEMM: operand pitch", "");
 }
 
-// bf16 plane.  K-major [rows, K] (pitch ld): box {BK k, box_rows}, 64-byte swizzle (a row of the box
-// is 32 bf16 = 64 B).  MN-major [K, rows] (pitch ld): box {64 mn, BK k}, 128-byte swizzle.
+// bf16 plane.  K-major [rows, K]: box {BK k, box_rows}, 64-byte swizzle (a row of the box is 32 bf16 =
+// 64 B).  MN-major [K, rows]: box {64 mn, BK k}, 128-byte swizzle.
 static int make_map16(CUtensorMap* map, const void* ptr, int64_t rows, int64_t K, int64_t ld, int box_rows,
                       bool mn_major) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) TNN_FAIL("mixed GEMM: bf16 plane must be 16-byte aligned");
-  if (ld % 8 != 0) TNN_FAIL("mixed GEMM: bf16 plane pitch must be a multiple of 8 elements");
-  cuuint64_t dims[2] = {(cuuint64_t)(mn_major ? rows : K), (cuuint64_t)(mn_major ? K : rows)};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)(mn_major ? 64 : BK), (cuuint32_t)(mn_major ? BK : box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)ptr, dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        mn_major ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) TNN_FAIL("cuTensorMapEncodeTiled (bf16) failed with code " + std::to_string((int)r));
-  return 0;
+  return tc::make_map(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, ptr, rows, K, ld, mn_major, mn_major ? 64 : BK,
+                      mn_major ? BK : box_rows, mn_major ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                      "mixed GEMM: bf16 plane", "mixed GEMM: bf16 plane pitch", " (bf16)");
 }
 
 constexpr int DEFAULT_CG = 2;  // CTA pairs: measured 0.98 ms vs 1.10 ms per 8192x4096x4096 product
-static unsigned int* g_tile_flags = nullptr;   // split-K arrival counters
-constexpr int MAX_FLAG_TILES = 1 << 16;
 static int g_group_m = 1;                      // tile rasterisation group; measured on 8192x4096x4096:
                                                // 1 -> 0.95 ms, 4 -> 0.96-1.04, 8 -> 1.10, 16 -> 1.08
 static int g_force_ksplit = 0;                 // 0 = auto (tail split), 1 = off, 2/4 = every tile (TNN_GEMM_KSPLIT)
 static int g_force_cg = 0;  // 0 = default, 1 / 2 = forced (TNN_GEMM_CG or tnn_set_gemm_cta_group)
-static bool g_attr_set[3][2][2][2] = {};
-int g_reserved_sms = 0;          // SMs the persistent grids leave to other streams (NCCL); also read by gemm_f16.cu
 static int g_exp_flags = 0;  // timing experiments (TNN_EXP_*): OR-ed into the kernel's flags
 
 struct ActOut {
@@ -957,69 +782,26 @@ static int launch_gemm(float* D, int64_t ldd, const Planes& a, const Planes& b, 
     ma_l16 = ma_lo;
     mb_l16 = mb_lo;
   }
-  auto kern = gemm_tf32x3_kernel<CG, A_MN, B_MN, MIX>;
-  if (!g_attr_set[CG][A_MN][B_MN][MIX]) {
-    TNN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-    g_attr_set[CG][A_MN][B_MN][MIX] = true;
-  }
   const int64_t tiles = ceil_div(M, C::TILE_M) * ceil_div(N, UMMA_N);
-  // SMs left free on purpose (tnn_set_gemm_reserved_sms): room for an NCCL kernel running beside
-  // the backward pass (comm.cu)
-  const int usable_sms = std::max(CG, ctx().sm_count - g_reserved_sms);
-  const int max_groups = usable_sms / CG;
-  // Tail split (see the kernel): when the tile count leaves a ragged last wave, the tiles of that
-  // wave are cut along K so it runs short and full.  Measured on the 4096x4096x8192 dW product
-  // (256 tiles, 74 CTA pairs): see profiles/.  Splitting EVERY tile instead lost time (1.20 ms vs
-  // 1.03 ms, the read-modify-write epilogue of the second range costs more than the idle tail), so
-  // a forced whole-matrix split is only taken when asked for.  The ReLU epilogue needs the complete
-  // sum, so it never splits.
-  int t_full = (int)tiles, tail_split = 1;
-  if (!(flags & 2) && tiles <= MAX_FLAG_TILES && g_force_ksplit != 1) {
-    const int64_t num_kb = ceil_div(K, BK);
-    if (g_force_ksplit > 1) {
-      if (num_kb / g_force_ksplit >= 1) {
-        t_full = 0;
-        tail_split = g_force_ksplit;
-      }
-    } else {
-      const int64_t rem = tiles % max_groups;
-      if (rem > 0) {
-        int s = 1;
-        while (s < 4 && rem * (s * 2) <= max_groups && num_kb / (s * 2) >= 16) s *= 2;
-        if (s > 1) {
-          t_full = (int)(tiles - rem);
-          tail_split = s;
-        }
-      }
-    }
+  const int64_t num_kb = ceil_div(K, BK);
+  const int groups = max_groups(CG);
+  // Splitting EVERY tile instead of the tail lost time (1.20 ms vs 1.03 ms on the 4096x4096x8192 dW
+  // product: the read-modify-write epilogue of the second range costs more than the idle tail), so a
+  // forced whole-matrix split (TNN_GEMM_KSPLIT) is only taken when asked for.
+  TailPlan plan{(int)tiles, 1};
+  if (g_force_ksplit > 1) {
+    if (!(flags & 2) && tiles <= MAX_FLAG_TILES && num_kb / g_force_ksplit >= 1) plan = {0, g_force_ksplit};
+  } else if (g_force_ksplit != 1) {
+    plan = plan_tail(flags, tiles, tiles, groups, num_kb, 16);
   }
-  if (tail_split > 1) {
-    if (!g_tile_flags) TNN_CUDA(cudaMalloc(&g_tile_flags, MAX_FLAG_TILES * sizeof(unsigned int)));
-    TNN_CUDA(cudaMemsetAsync(g_tile_flags, 0, (size_t)tiles * sizeof(unsigned int), ctx().stream));
-  }
-  const int64_t units = t_full + (tiles - t_full) * tail_split;
-  int groups = (int)std::min<int64_t>(units, max_groups);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(groups * CG));
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
-  cfg.stream = ctx().stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  if (clear_tile_flags(plan, tiles)) return 1;
   // (a conditional launch is the fallback behind an f16 product: family 4, so that the per-launch
   // GEMM timing of family 1 only sees launches that do the product)
-  const int family = cond_a ? 4 : 1;
-  prof_begin(family);
-  TNN_CUDA(cudaLaunchKernelEx(&cfg, kern, ma_hi, ma_lo, ma_l16, mb_hi, mb_lo, mb_l16, D, ldd, (int)M, (int)N, (int)K, bias, flags | g_exp_flags, t_full, tail_split, g_tile_flags, g_group_m,
-                              act.out, act.hi, act.lo, (__nv_bfloat16*)act.l16, act.ld, act.mask_src, cond_a, cond_b));
-  ctx().launches++;
-  prof_end(family);
-  return 0;
+  return launch_persistent<gemm_tf32x3_kernel<CG, A_MN, B_MN, MIX>>(
+      CG, NUM_THREADS, C::SMEM_BYTES, plan.t_full + (tiles - plan.t_full) * plan.tail_split, groups, false,
+      cond_a ? 4 : 1, ma_hi, ma_lo, ma_l16, mb_hi, mb_lo, mb_l16, D, ldd, (int)M, (int)N, (int)K, bias,
+      flags | g_exp_flags, plan.t_full, plan.tail_split, g_tile_flags, g_group_m, act.out, act.hi, act.lo,
+      (__nv_bfloat16*)act.l16, act.ld, act.mask_src, cond_a, cond_b);
 }
 
 }  // namespace tc
@@ -1043,11 +825,9 @@ static int gemm_common(const char* who, bool mix, float* D, int64_t ldd, const t
                        const tnn::tc::Planes& b, int64_t M, int64_t N, int64_t K, const float* bias,
                        int flags, int layout, const tnn::tc::ActOut& act_in,
                        const int* cond_a = nullptr, const int* cond_b = nullptr) {
-  TNN_REQUIRE_INIT();
-  if (M <= 0 || N <= 0) return 0;
-  if (K <= 0) TNN_FAIL(std::string(who) + ": K must be positive");
-  if (M > 2147483647LL || N > 2147483647LL || K > 2147483647LL) TNN_FAIL(std::string(who) + ": extent above int32");
-  if (tc::get_encode_fn()) return 1;
+  bool empty;
+  if (tc::gemm_entry_checks(who, M, N, K, empty)) return 1;
+  if (empty) return 0;
   static bool env_read = false;
   if (!env_read) {
     const char* e = getenv("TNN_GEMM_CG");
