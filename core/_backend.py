@@ -29,7 +29,7 @@ NEG, EXP, LOG, COPY, CLIP, SCALE, CLIP_BWD, RECIP_MUL = range(40, 48)
 LEAKY_RELU, ELU, GELU, GELU_TANH, SOFTPLUS, SILU = range(48, 54)
 LEAKY_RELU_BWD, ELU_BWD, GELU_BWD, GELU_TANH_BWD, SOFTPLUS_BWD, SILU_BWD = range(60, 66)
 RED_SUM, RED_MAX, RED_MIN = 0, 1, 2
-OPT_SGD, OPT_ADAM, OPT_RMSPROP, OPT_MOMENTUM, OPT_ADAGRAD, OPT_ADADELTA = range(6)
+OPT_SGD, OPT_ADAM, OPT_RMSPROP, OPT_MOMENTUM, OPT_ADAGRAD, OPT_ADADELTA, OPT_ADAMW, OPT_RADAM, OPT_ADAMAX = range(9)
 
 _c_i64 = ctypes.c_int64
 _c_i32 = ctypes.c_int32

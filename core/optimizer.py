@@ -11,11 +11,17 @@ weight_decay: the reference accepts it and never applies it (the line that would
 `_step -= self.weight_decay * v`, is commented out at optimizer.py:28-29).  Same here by default;
 setting `optimizer.apply_weight_decay = True` turns exactly that line on (fused path: inside the
 optimiser kernel, hyper-parameter slot 7; compute_step path: on the per-parameter step views).
+AdamW is the exception: its decoupled decay is always on and `apply_weight_decay` has no effect on it.
+
+`optimizer.lr` is read whenever a step's coefficients are formed, so core/lr_scheduler.py can change
+it between steps, recorded steps included.
 
 The fused arena path is only taken for the built-in update rules: an optimiser whose class
 overrides `_compute_step` or `compute_step` (the reference's extension point) always goes
 through compute_step(), see core.model.Model.step.
 """
+import math
+
 import numpy as np
 
 import core._backend as be
@@ -62,7 +68,7 @@ class BaseOptimizer(object):
         if flat_step.size != total:
             raise ValueError("_compute_step returned %d elements for %d gradients" % (flat_step.size, total))
         flat_step = flat_step.view((total,))
-        wd = self._decay_coefficient()
+        wd = self._step_decay()
 
         p = 0
         steps = []
@@ -90,8 +96,12 @@ class BaseOptimizer(object):
     def _decay_coefficient(self):
         return float(self.weight_decay) if (self.apply_weight_decay and self.weight_decay) else 0.0
 
+    def _step_decay(self):
+        """c of `step -= c * v`, which compute_step applies to each parameter's step"""
+        return self._decay_coefficient()
+
     def _hyper8(self):
-        """this step's kernel coefficients: the rule's own in slots 0-5, weight decay in slot 7"""
+        """this step's kernel coefficients: the rule's own in slots 0-6, weight decay in slot 7"""
         vals = list(self._hyper())
         vals += [0.0] * (8 - len(vals))
         vals[7] = self._decay_coefficient()
@@ -235,3 +245,70 @@ class Adadelta(BaseOptimizer):
 
     def _hyper(self):
         return [self.lr, self._decay, self._eps]
+
+
+def _check_adam_args(lr, beta1, beta2, epsilon):
+    for name, v in (("lr", lr), ("epsilon", epsilon)):
+        if not (math.isfinite(v) and v >= 0.0):
+            raise ValueError("%s must be finite and non-negative, got %r" % (name, v))
+    for name, v in (("beta1", beta1), ("beta2", beta2)):
+        if not 0.0 <= v < 1.0:
+            raise ValueError("%s must lie in [0, 1), got %r" % (name, v))
+
+
+class AdamW(Adam):
+    """Adam with decoupled weight decay (torch.optim.AdamW): p = p * (1 - lr*wd) + Adam's step.
+
+    The decay is always on; `apply_weight_decay` has no effect on this rule.  On the fused path the
+    kernel scales the parameter; on the compute_step path `(lr*wd) * v` is subtracted from each
+    parameter's step."""
+    opt_code = be.OPT_ADAMW
+
+    def __init__(self, lr=0.001, beta1=0.9, beta2=0.999, epsilon=1e-8, weight_decay=0.01):
+        _check_adam_args(lr, beta1, beta2, epsilon)
+        super().__init__(lr, beta1, beta2, epsilon, weight_decay)
+
+    def _decay_coefficient(self):
+        return 0.0
+
+    def _step_decay(self):
+        return float(self.lr) * float(self.weight_decay)
+
+    def _hyper(self):
+        return super()._hyper() + [1.0 - float(self.lr) * float(self.weight_decay)]
+
+
+class RAdam(Adam):
+    """Rectified Adam (torch.optim.RAdam): with mh = m/(1-b1^t),
+    step = -lr * r_t * mh * sqrt(1-b2^t) / (sqrt(v) + eps) once the variance is tractable
+    (rho_t > 5), step = -lr * mh before.  Weight decay is opt-in, as for the reference's rules."""
+    opt_code = be.OPT_RADAM
+
+    def __init__(self, lr=0.001, beta1=0.9, beta2=0.999, epsilon=1e-8, weight_decay=0.0):
+        _check_adam_args(lr, beta1, beta2, epsilon)
+        super().__init__(lr, beta1, beta2, epsilon, weight_decay)
+
+    def _hyper(self):
+        self._t += 1
+        t, b2 = self._t, self._b2
+        bc2 = 1.0 - b2 ** t
+        rho_inf = 2.0 / (1.0 - b2) - 1.0
+        rho_t = rho_inf - 2.0 * t * b2 ** t / bc2
+        r_t = 0.0
+        if rho_t > 5.0:
+            r_t = math.sqrt((rho_t - 4.0) * (rho_t - 2.0) * rho_inf / ((rho_inf - 4.0) * (rho_inf - 2.0) * rho_t))
+        return [self.lr, self._b1, b2, self._eps, 1.0 - self._b1 ** t, math.sqrt(bc2), r_t]
+
+
+class Adamax(Adam):
+    """Adam's infinity-norm variant (torch.optim.Adamax): u = max(b2*u, |g| + eps);
+    step = -(lr/(1-b1^t)) * m / u.  Weight decay is opt-in, as for the reference's rules."""
+    opt_code = be.OPT_ADAMAX
+
+    def __init__(self, lr=0.002, beta1=0.9, beta2=0.999, epsilon=1e-8, weight_decay=0.0):
+        _check_adam_args(lr, beta1, beta2, epsilon)
+        super().__init__(lr, beta1, beta2, epsilon, weight_decay)
+
+    def _hyper(self):
+        self._t += 1
+        return [self.lr, self._b1, self._b2, self._eps, self.lr / (1.0 - self._b1 ** self._t)]

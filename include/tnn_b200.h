@@ -105,7 +105,10 @@ enum {
   TNN_OPT_RMSPROP = 2,  /* optimizer.py:107 */
   TNN_OPT_MOMENTUM = 3, /* optimizer.py:126 */
   TNN_OPT_ADAGRAD = 4,  /* optimizer.py:143 */
-  TNN_OPT_ADADELTA = 5  /* optimizer.py:158 */
+  TNN_OPT_ADADELTA = 5, /* optimizer.py:158 */
+  TNN_OPT_ADAMW = 6,    /* decoupled weight decay (Loshchilov & Hutter) */
+  TNN_OPT_RADAM = 7,    /* rectified Adam (Liu et al.) */
+  TNN_OPT_ADAMAX = 8    /* Adam's infinity-norm variant (Kingma & Ba, section 7) */
 };
 
 /* ---- lifecycle / errors ------------------------------------------------------------------- */
@@ -477,8 +480,14 @@ int tnn_mlp_tail_step(int n_layers, const int64_t* in_dims, const int64_t* out_d
  * hyper-parameters:
  *   SGD [lr]; ADAM [lr, b1, b2, eps, 1-b1^t, 1-b2^t]; RMSPROP [lr, decay, momentum, eps];
  *   MOMENTUM [lr, momentum]; ADAGRAD [lr, eps]; ADADELTA [lr, decay, eps];
+ *   ADAMW [lr, b1, b2, eps, 1-b1^t, 1-b2^t, 1-lr*wd]: Adam's step, then param = param*h[6] + step
+ *     (with param NULL, step_out receives Adam's step alone and the caller adds the decay);
+ *   RADAM [lr, b1, b2, eps, 1-b1^t, sqrt(1-b2^t), r_t]: mh = m/h[4]; step = -lr*r_t*mh*h[5]/(sqrt(v)+eps)
+ *     if r_t > 0, else -lr*mh.  r_t is the rectification term, 0 while rho_t <= 5; the kernel reads it
+ *     at run time, so a recorded step switches branch when the uploaded r_t becomes positive;
+ *   ADAMAX [lr, b1, b2, eps, lr/(1-b1^t)]: u = max(b2*u, |g|+eps) (NaN propagates); step = -h[4]*m/u.
  *   every rule: h[7] = weight-decay coefficient, 0 = off (optimizer.py:28-29 `_step -= wd * v`,
- *   commented out upstream and therefore opt-in here; needs param != NULL).
+ *   commented out upstream and therefore opt-in here; needs param != NULL).  AdamW passes 0 there.
  * param (updated in place: param += step) and step_out (receives step) may each be NULL. */
 int tnn_opt_step(int opt, int dtype, void* param, void* step_out, const void* grad, void* s0,
                  void* s1, int64_t n, const double* h, int n_h);

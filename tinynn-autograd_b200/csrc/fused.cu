@@ -5,6 +5,7 @@
 //                                                        losses.py:24-32
 //  * SGD / Adam / RMSProp / Momentum / Adagrad / Adadelta on the flat parameter arena
 //                                                        optimizer.py:41-164, model.py:45-61
+//  * AdamW / RAdam / Adamax, which share Adam's per-element code and 128-bit kernel
 // All HBM-bound streaming kernels: 128-bit accesses, grid-stride, grids in multiples of the SM
 // count.  Reductions inside the loss are two-stage and deterministic (see reduce.cu).
 #include <algorithm>
@@ -468,6 +469,51 @@ struct OptH {
   double h[8];
 };
 
+template <int OPT>
+constexpr bool adam_family = OPT == TNN_OPT_ADAM || OPT == TNN_OPT_ADAMW || OPT == TNN_OPT_RADAM ||
+                             OPT == TNN_OPT_ADAMAX;
+
+// The Adam family's per-element update, shared by opt_kernel and adam_vec_kernel so that the scalar
+// and the 128-bit path give the same bits.  The coefficients are narrowed once from the host's doubles
+// (include/tnn_b200.h lists each rule's h[] layout).
+template <int OPT, typename T>
+struct AdamRule {
+  T lr, omb1, b2, eps, c4, c5, c6, wd;
+  __device__ __forceinline__ explicit AdamRule(const OptH& hh)
+      // 1-b1 and 1-b2 are formed in double like the reference's Python floats, then narrowed
+      : lr((T)hh.h[0]), omb1((T)(1.0 - hh.h[1])), b2(OPT == TNN_OPT_ADAMAX ? (T)hh.h[2] : (T)(1.0 - hh.h[2])),
+        eps((T)hh.h[3]), c4((T)hh.h[4]), c5((T)hh.h[5]), c6((T)hh.h[6]), wd((T)hh.h[7]) {}
+
+  // moments m (state 0) and v (state 1; Adamax: the infinity norm u) updated in place; returns the
+  // step before any weight decay
+  __device__ __forceinline__ T step(T g, T& m, T& v) const {
+    m += omb1 * (g - m);
+    if constexpr (OPT == TNN_OPT_ADAMAX) {
+      v = m_max(b2 * v, fabs(g) + eps);   // NaN in either operand propagates
+      return -c4 * m / v;
+    } else {
+      v += b2 * (g * g - v);              // b2 holds 1-b2 here
+      if constexpr (OPT == TNN_OPT_RADAM) {
+        // r_t (c6) is read here rather than chosen on the host: a recorded step reads it from
+        // device memory at every replay and switches to the rectified form when t reaches it
+        const T mh = m / c4;
+        if (c6 > T(0)) return -lr * c6 * mh * c5 / (m_sqrt(v) + eps);
+        return -lr * mh;
+      } else {
+        T mh = m / c4, vh = v / c5;
+        return -lr * mh / (m_sqrt(vh) + eps);
+      }
+    }
+  }
+
+  // the new parameter; `step` takes the opt-in weight decay (h[7], optimizer.py:28-29)
+  __device__ __forceinline__ T apply(T p, T& step) const {
+    if (wd != T(0)) step -= wd * p;
+    if constexpr (OPT == TNN_OPT_ADAMW) return p * c6 + step;   // decoupled decay: p * (1 - lr*wd)
+    return p + step;
+  }
+};
+
 template <int OPT, typename T>
 __global__ void __launch_bounds__(256)
 opt_kernel(T* param, T* step_out, const T* grad, T* s0, T* s1, int64_t n, OptH hh,
@@ -478,71 +524,67 @@ opt_kernel(T* param, T* step_out, const T* grad, T* s0, T* s1, int64_t n, OptH h
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     const T g = grad[i];
     T step;
-    if constexpr (OPT == TNN_OPT_SGD) {
-      step = -(T)hh.h[0] * g;
-    } else if constexpr (OPT == TNN_OPT_ADAM) {
-      // 1-b1 and 1-b2 are formed in double like the reference's Python floats, then narrowed
-      const T lr = (T)hh.h[0], omb1 = (T)(1.0 - hh.h[1]), omb2 = (T)(1.0 - hh.h[2]), eps = (T)hh.h[3];
-      const T bc1 = (T)hh.h[4], bc2 = (T)hh.h[5];
+    if constexpr (adam_family<OPT>) {
+      const AdamRule<OPT, T> rule(hh);
       T m = s0[i], v = s1[i];
-      m += omb1 * (g - m);
-      v += omb2 * (g * g - v);
+      step = rule.step(g, m, v);
       s0[i] = m;
       s1[i] = v;
-      T mh = m / bc1, vh = v / bc2;
-      step = -lr * mh / (m_sqrt(vh) + eps);
-    } else if constexpr (OPT == TNN_OPT_RMSPROP) {
-      const T lr = (T)hh.h[0], omd = (T)(1.0 - hh.h[1]), mom_c = (T)hh.h[2], eps = (T)hh.h[3];
-      T ms = s0[i], mom = s1[i];
-      ms += omd * (g * g - ms);
-      mom = mom_c * mom + lr * g / m_sqrt(ms + eps);
-      s0[i] = ms;
-      s1[i] = mom;
-      step = -mom;
-    } else if constexpr (OPT == TNN_OPT_MOMENTUM) {
-      const T lr = (T)hh.h[0], mom_c = (T)hh.h[1];
-      T acc = mom_c * s0[i] + g;
-      s0[i] = acc;
-      step = -lr * acc;
-    } else if constexpr (OPT == TNN_OPT_ADAGRAD) {
-      const T lr = (T)hh.h[0], eps = (T)hh.h[1];
-      T G = s0[i] + g * g;
-      s0[i] = G;
-      step = -(lr / m_sqrt(G + eps)) * g;
-    } else {  // ADADELTA
-      const T lr = (T)hh.h[0], omd = (T)(1.0 - hh.h[1]), eps = (T)hh.h[2];
-      T Eg = s0[i], delta = s1[i];
-      Eg += omd * (g * g - Eg);
-      T sd = m_sqrt(delta + eps);
-      T d = g * (sd / m_sqrt(Eg + eps));
-      step = -lr * d;
-      delta += omd * (d * d - delta);
-      s0[i] = Eg;
-      s1[i] = delta;
-    }
-    if (param) {
-      // optimizer.py:28-29 (`_step -= self.weight_decay * v`, commented out upstream): applied only
-      // when the host passes a non-zero coefficient in h[7] (BaseOptimizer.apply_weight_decay)
-      const T wd = (T)hh.h[7];
-      const T p = param[i];
-      if (wd != T(0)) step -= wd * p;
-      param[i] = p + step;
+      if (param) param[i] = rule.apply(param[i], step);
+    } else {
+      if constexpr (OPT == TNN_OPT_SGD) {
+        step = -(T)hh.h[0] * g;
+      } else if constexpr (OPT == TNN_OPT_RMSPROP) {
+        const T lr = (T)hh.h[0], omd = (T)(1.0 - hh.h[1]), mom_c = (T)hh.h[2], eps = (T)hh.h[3];
+        T ms = s0[i], mom = s1[i];
+        ms += omd * (g * g - ms);
+        mom = mom_c * mom + lr * g / m_sqrt(ms + eps);
+        s0[i] = ms;
+        s1[i] = mom;
+        step = -mom;
+      } else if constexpr (OPT == TNN_OPT_MOMENTUM) {
+        const T lr = (T)hh.h[0], mom_c = (T)hh.h[1];
+        T acc = mom_c * s0[i] + g;
+        s0[i] = acc;
+        step = -lr * acc;
+      } else if constexpr (OPT == TNN_OPT_ADAGRAD) {
+        const T lr = (T)hh.h[0], eps = (T)hh.h[1];
+        T G = s0[i] + g * g;
+        s0[i] = G;
+        step = -(lr / m_sqrt(G + eps)) * g;
+      } else {  // ADADELTA
+        const T lr = (T)hh.h[0], omd = (T)(1.0 - hh.h[1]), eps = (T)hh.h[2];
+        T Eg = s0[i], delta = s1[i];
+        Eg += omd * (g * g - Eg);
+        T sd = m_sqrt(delta + eps);
+        T d = g * (sd / m_sqrt(Eg + eps));
+        step = -lr * d;
+        delta += omd * (d * d - delta);
+        s0[i] = Eg;
+        s1[i] = delta;
+      }
+      if (param) {
+        // optimizer.py:28-29 (`_step -= self.weight_decay * v`, commented out upstream): applied only
+        // when the host passes a non-zero coefficient in h[7] (BaseOptimizer.apply_weight_decay)
+        const T wd = (T)hh.h[7];
+        const T p = param[i];
+        if (wd != T(0)) step -= wd * p;
+        param[i] = p + step;
+      }
     }
     if (step_out) step_out[i] = step;
   }
 }
 
-// Adam is the hot one (28 B/param): 128-bit variant
-template <typename T>
+// The Adam family is the hot one (28 B/param): 128-bit variant
+template <int OPT, typename T>
 __global__ void __launch_bounds__(256)
 adam_vec_kernel(T* param, const T* grad, T* s0, T* s1, int64_t nv, OptH hh, const OptH* hdev) {
   pdl_sync();
   if (hdev) hh = *hdev;
   constexpr int W = 16 / sizeof(T);
   using V = Pack<T, W>;
-  const T lr = (T)hh.h[0], omb1 = (T)(1.0 - hh.h[1]), omb2 = (T)(1.0 - hh.h[2]), eps = (T)hh.h[3];
-  const T bc1 = (T)hh.h[4], bc2 = (T)hh.h[5];
-  const T wd = (T)hh.h[7];   // weight decay, 0 = off (optimizer.py:28-29)
+  const AdamRule<OPT, T> rule(hh);
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride) {
     const V g = reinterpret_cast<const V*>(grad)[i];
@@ -551,17 +593,30 @@ adam_vec_kernel(T* param, const T* grad, T* s0, T* s1, int64_t nv, OptH hh, cons
     V p = reinterpret_cast<const V*>(param)[i];
 #pragma unroll
     for (int k = 0; k < W; ++k) {
-      m.v[k] += omb1 * (g.v[k] - m.v[k]);
-      v.v[k] += omb2 * (g.v[k] * g.v[k] - v.v[k]);
-      T mh = m.v[k] / bc1, vh = v.v[k] / bc2;
-      T step = -lr * mh / (m_sqrt(vh) + eps);
-      if (wd != T(0)) step -= wd * p.v[k];
-      p.v[k] += step;
+      T step = rule.step(g.v[k], m.v[k], v.v[k]);
+      p.v[k] = rule.apply(p.v[k], step);
     }
     reinterpret_cast<V*>(s0)[i] = m;
     reinterpret_cast<V*>(s1)[i] = v;
     reinterpret_cast<V*>(param)[i] = p;
   }
+}
+
+// calls f(std::integral_constant<int, OPT>) for a known optimizer code
+template <typename F>
+static int with_opt(int opt, F&& f) {
+  switch (opt) {
+    case TNN_OPT_SGD: return f(std::integral_constant<int, TNN_OPT_SGD>{});
+    case TNN_OPT_ADAM: return f(std::integral_constant<int, TNN_OPT_ADAM>{});
+    case TNN_OPT_RMSPROP: return f(std::integral_constant<int, TNN_OPT_RMSPROP>{});
+    case TNN_OPT_MOMENTUM: return f(std::integral_constant<int, TNN_OPT_MOMENTUM>{});
+    case TNN_OPT_ADAGRAD: return f(std::integral_constant<int, TNN_OPT_ADAGRAD>{});
+    case TNN_OPT_ADADELTA: return f(std::integral_constant<int, TNN_OPT_ADADELTA>{});
+    case TNN_OPT_ADAMW: return f(std::integral_constant<int, TNN_OPT_ADAMW>{});
+    case TNN_OPT_RADAM: return f(std::integral_constant<int, TNN_OPT_RADAM>{});
+    case TNN_OPT_ADAMAX: return f(std::integral_constant<int, TNN_OPT_ADAMAX>{});
+  }
+  TNN_FAIL("tnn_opt_step: unknown optimizer code");
 }
 
 template <typename T>
@@ -572,31 +627,26 @@ static int opt_dispatch(int opt, T* param, T* step_out, const T* grad, T* s0, T*
   // a small arena is the tail of a launch-bound chain (the MNIST-sized step): programmatic dependency
   const bool pdl = grid <= 2 * ctx().sm_count;
   constexpr int W = 16 / sizeof(T);
-  if (opt == TNN_OPT_ADAM && param && !step_out && aligned16(param) && aligned16(grad) && aligned16(s0) &&
-      aligned16(s1) && n >= W) {
-    const int64_t nv = n / W, done = nv * W;
-    TNN_CUDA(launch_small(adam_vec_kernel<T>, dim3(ew_grid(nv, 256)), dim3(256), st, pdl, 1u, param, grad, s0, s1, nv, hh, hdev));
-    ctx().launches++;
-    if (done == n) return 0;
-    TNN_CUDA(launch_small(opt_kernel<TNN_OPT_ADAM, T>, dim3(1), dim3(256), st, pdl, 1u, param + done, (T*)nullptr,
-                          grad + done, s0 + done, s1 + done, n - done, hh, hdev));
-    TNN_POST_LAUNCH();
-    return 0;
-  }
-  auto run = [&](auto OPT) {
+  const bool vec = param && !step_out && aligned16(param) && aligned16(grad) && aligned16(s0) &&
+                   aligned16(s1) && n >= W;
+  return with_opt(opt, [&](auto OPT) {
+    if constexpr (adam_family<OPT>) {
+      if (vec) {
+        const int64_t nv = n / W, done = nv * W;
+        TNN_CUDA(launch_small(adam_vec_kernel<OPT, T>, dim3(ew_grid(nv, 256)), dim3(256), st, pdl, 1u, param, grad,
+                              s0, s1, nv, hh, hdev));
+        ctx().launches++;
+        if (done == n) return 0;
+        TNN_CUDA(launch_small(opt_kernel<OPT, T>, dim3(1), dim3(256), st, pdl, 1u, param + done, (T*)nullptr,
+                              grad + done, s0 + done, s1 + done, n - done, hh, hdev));
+        TNN_POST_LAUNCH();
+        return 0;
+      }
+    }
     TNN_CUDA(launch_small(opt_kernel<OPT, T>, dim3(grid), dim3(256), st, pdl, 1u, param, step_out, grad, s0, s1, n, hh, hdev));
     TNN_POST_LAUNCH();
     return 0;
-  };
-  switch (opt) {
-    case TNN_OPT_SGD: return run(std::integral_constant<int, TNN_OPT_SGD>{});
-    case TNN_OPT_ADAM: return run(std::integral_constant<int, TNN_OPT_ADAM>{});
-    case TNN_OPT_RMSPROP: return run(std::integral_constant<int, TNN_OPT_RMSPROP>{});
-    case TNN_OPT_MOMENTUM: return run(std::integral_constant<int, TNN_OPT_MOMENTUM>{});
-    case TNN_OPT_ADAGRAD: return run(std::integral_constant<int, TNN_OPT_ADAGRAD>{});
-    case TNN_OPT_ADADELTA: return run(std::integral_constant<int, TNN_OPT_ADADELTA>{});
-  }
-  TNN_FAIL("tnn_opt_step: unknown optimizer code");
+  });
 }
 
 // ---- CE host drivers ---------------------------------------------------------------------------
